@@ -73,6 +73,10 @@ def parse_args():
     ap.add_argument('--no-extras', action='store_true', help='skip the legs outside the headline (cold / fresh start / per-step API / '
                                                              'published protocol / K2+K4 roofline / cpu baseline)')
     ap.add_argument('--cpu-seconds', type=float, default=15., help='budget of the cpu_baseline sample')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed bench step returned (ClosedLoop.run logs cost / u0 / n_solves / status and '
+                         'the final states x) to DIR/<name>.npy as float64, to compare two builds output for output; '
+                         'steps without a solution (status != 0, cost inf) are written as cost 0 and u0 0')
     a = ap.parse_args()
     w = WORKLOADS[a.workload]
     for k in ('instances', 'window', 'max_solves', 'max_roots', 'steps', 'warmup'):
@@ -116,6 +120,27 @@ def initial_states(workload, model, lo, hi):
 def noise(model, n_steps, n_inst, sigma, seed):
     rng = np.random.default_rng(seed)
     return sigma * rng.standard_normal((n_steps, n_inst, model['A'].shape[0])) * model['x_max']
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, suffix=''):
+    """Writes {name: array [..., n_inst, ...] with the instance axis given per array} as out_dir/<name><suffix>.npy in
+    float64.  Above DUMP_LIMIT bytes in all, a fixed seeded sample of the instances is written instead, and its indices
+    as instances<suffix>.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (np.asarray(v, dtype=np.float64), axis) for k, (v, axis) in arrays.items()}
+    v0, axis0 = next(iter(arrays.values()))
+    n_inst = v0.shape[axis0]
+    total = sum(v.nbytes for v, _ in arrays.values())
+    if total > DUMP_LIMIT:
+        keep = max(1, n_inst * DUMP_LIMIT // total)
+        idx = np.sort(np.random.default_rng(0).choice(n_inst, keep, replace=False))
+        arrays = {k: (np.take(v, idx, axis=axis), axis) for k, (v, axis) in arrays.items()}
+        np.save(os.path.join(out_dir, 'instances%s.npy' % suffix), idx.astype(np.float64))
+    for k, (v, _) in arrays.items():
+        np.save(os.path.join(out_dir, '%s%s.npy' % (k, suffix)), v)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -425,6 +450,15 @@ def run_b200(args):
         ev.append((a, b))
     l0 = loop.launches
     ms, qps, iters, my_qps = timed_loop(torch, dist, loop, args.steps, world, dev_step)
+    if args.dump_outputs:            # the legs below reuse `logs` and the loop: copy the last timed step's results now
+        out = {k: logs[k].cpu().numpy() for k in ('cost', 'u0', 'n_solves', 'status')}
+        # a step without a solution (status != 0 and no incumbent: the instance has left the loop) comes back as cost inf and
+        # u0 NaN; it is written as 0 and `status` tells which entries those are
+        none = (out['status'] != 0) & ~np.isfinite(out['cost'])
+        out['cost'] = np.where(none, 0., out['cost'])
+        out['u0'] = np.where(none[..., None], 0., out['u0'])
+        dump_outputs(args.dump_outputs, {k: (v, 1) for k, v in out.items()} | {'x': (loop.x.cpu().numpy(), 0)},
+                     '_rank%d' % rank if world > 1 else '')
     cnt = timed_loop.last.astype(float)
     launches = loop.launches - l0
     clocks = sampler.stop()
@@ -649,6 +683,8 @@ def run_b200(args):
 if __name__ == '__main__':
     a = parse_args()
     if a.impl == 'reference':
+        if a.dump_outputs:
+            sys.exit('bench.py: --dump-outputs is implemented for --impl b200')
         run_reference(a)
     else:
         run_b200(a)

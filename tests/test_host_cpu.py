@@ -272,6 +272,34 @@ def test_product_control_flow_equals_reference_on_the_golden_run():
     assert n_p < 40
 
 
+def test_product_control_flow_reproduces_the_golden_noisy_loop():
+    """The product's host control flow (device_search = False) with the QP answers the golden fixtures were made with
+    (oracle core variant 0, every node solved from the empty working set) on the reference's golden noisy CP20 loop
+    (cp20_closed_loop.npz): every step the warm-started search reaches the reference's optimum and mode sequence with
+    as many QPs, and hands on a warm start of the same size.  The oracle's answers carry the last bits of the host's
+    BLAS (tests/test_oracle_cpu.py): costs to 1e-9, and QP counts within 2 where near-ties in best-first order flip."""
+    from tests.util import oracle_launch
+    model = load_model('cp20')
+    ctl = make_controller(model)
+    ctl.device_search = False
+    ctl.qp.setParam('Method', -1)                    # no active-set hand-over
+    launch = oracle_launch(model, ctl.problem, variant=0)
+    # the golden run solved every node from the empty working set
+    ctl.qp._launch = lambda x0, lb, ub, y0, yc0: launch(x0, lb, ub, None, None)
+    g = np.load(os.path.join(GOLDEN, 'cp20_closed_loop.npz'))
+    x, ws = model['x0_nominal'].copy(), None
+    for t in range(len(g['noisy_cost'])):
+        assert np.allclose(x, g['noisy_x'][t], rtol=0, atol=1e-9)
+        sol, leaves, n, _ = ctl.feedforward(x, warm_start=ws, printing_period=None)
+        assert abs(n - g['noisy_n_warm'][t]) <= 2
+        assert abs(sol.objective - g['noisy_cost_warm'][t]) <= 1e-9 * abs(g['noisy_cost_warm'][t])
+        assert np.array_equal(np.array(sol.variables['ub']), g['noisy_ub'][t])
+        e = g['noisy_e'][t]
+        ws, _, _ = ctl.construct_warm_start(leaves, sol.variables['x'][0], sol.variables['uc'][0], sol.variables['ub'][0], e)
+        assert len(ws) == g['noisy_cover'][t]
+        x = sol.variables['x'][1] + e
+
+
 def test_miqp_comparator_finds_the_same_optimum():
     """SURVEY.md 8f-1: the Gurobi-free stand-in of `feedforward_gurobi` (controller.py:723-776) -- a conventional MIQP
     branch and bound through the QP seam that ignores the time structure -- must return the optimum the structured
@@ -388,3 +416,29 @@ def test_bench_arguments_follow_the_driver_contract(monkeypatch):
         monkeypatch.setattr(sys, 'argv', ['bench.py', '--workload', w, '--impl', 'reference'])
         r = bench.parse_args()
         assert bench.workload_config(b, 1) == bench.workload_config(r, 1)
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs DIR: float64 .npy files of what the last timed step returned; above the size limit the same
+    seeded sample of instances in every array, its indices written beside them."""
+    import sys
+    import bench
+    monkeypatch.setattr(sys, 'argv', ['bench.py', '--dump-outputs', str(tmp_path)])
+    assert bench.parse_args().dump_outputs == str(tmp_path)
+    S, N = 3, 40
+    rng = np.random.default_rng(1)
+    arrays = {'cost': (rng.standard_normal((S, N)), 1), 'u0': (rng.standard_normal((S, N, 7)), 1),
+              'n_solves': (rng.integers(0, 99, (S, N)).astype(np.int32), 1), 'x': (rng.standard_normal((N, 4)), 0)}
+    bench.dump_outputs(str(tmp_path / 'all'), arrays)
+    for k, (v, _) in arrays.items():
+        got = np.load(tmp_path / 'all' / ('%s.npy' % k))
+        assert got.dtype == np.float64 and np.array_equal(got, v)
+    assert not (tmp_path / 'all' / 'instances.npy').exists()
+    monkeypatch.setattr(bench, 'DUMP_LIMIT', 2000)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    idx = np.load(tmp_path / 'a' / 'instances.npy').astype(int)
+    assert 0 < len(idx) < N and np.array_equal(idx, np.load(tmp_path / 'b' / 'instances.npy'))
+    assert sum(os.path.getsize(tmp_path / 'a' / ('%s.npy' % k)) for k in arrays) <= 2000 + 4 * 128   # + .npy headers
+    for k, (v, axis) in arrays.items():
+        assert np.array_equal(np.load(tmp_path / 'a' / ('%s.npy' % k)), np.take(v, idx, axis=axis))

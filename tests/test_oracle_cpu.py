@@ -69,14 +69,17 @@ def test_c_core_certificates_on_golden_nodes(cp20):
         r = cert.certify(model, cond, g['x0'], g['lb'][i], g['ub'][i], out)
         assert r['dual_neg'] >= 0.
         if out['status'] == 2:
-            assert out['cost'] == g['cost'][i]
+            # the fixture holds the bits of one host: the oracle's precompute goes through numpy's BLAS, whose kernels (and
+            # last bits) depend on the CPU
+            assert abs(out['cost'] - g['cost'][i]) <= 1e-9 * abs(g['cost'][i])
             assert r['prim_eq'] <= 1e-9 and r['prim_viol'] <= 2e-4 and r['dual_stat'] <= 1e-7
             assert abs(r['gap']) <= 1e-6
         else:
             fam = cert.families(model, cond, g['x0'], 3, None, out['y'])
             scale = np.sum(np.concatenate(fam['mu']) * arow[:cond.mc]) + np.sum(np.concatenate(fam['nu_lb'] + fam['nu_ub']))
             assert r['dual_stat'] <= 1e-9 * scale and r['ray_cost'] > 1e-9 * scale
-            assert abs(out['farkas'] - g['farkas'][i]) <= 1e-9 * abs(g['farkas'][i])
+            # the value of a (non-unique) infeasibility proof amplifies the host-BLAS bits above: 4e-9 seen between hosts
+            assert abs(out['farkas'] - g['farkas'][i]) <= 1e-6 * abs(g['farkas'][i])
 
 
 def test_c_core_vs_numpy_referee(cp20):
@@ -113,7 +116,7 @@ def test_restatement_reproduces_golden_closed_loop(cp20):
     ctl = OracleController(model, core, hot_start=False)
     log = closed_loop(ctl, model['x0_nominal'], 3, warm=True)
     for t, s in enumerate(log):
-        assert s['cost'] == g['nom_cost_warm'][t]
+        assert abs(s['cost'] - g['nom_cost_warm'][t]) <= 1e-9 * g['nom_cost_warm'][t]      # host BLAS: see above
         assert s['solves'] == g['nom_n_warm'][t]
         assert s['cover'] == g['nom_cover'][t]
         assert np.array_equal(s['ub'], g['nom_ub'][t])

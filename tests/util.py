@@ -68,14 +68,15 @@ def leaves_from_golden(pd, g):
     return out
 
 
-def oracle_launch(model, pd):
+def oracle_launch(model, pd, variant=1):
     """A stand-in for BoundedQP._launch (the device call) backed by the CPU oracle core: lets the CPU suite drive the
     product's and the reference's control flow through the product's BoundedQP front end without a GPU.  Same
-    contract: (x0, lb, ub, y0, yc0) -> dict(status, cost, dobj, iters, primal, dual, yc, runtime)."""
+    contract: (x0, lb, ub, y0, yc0) -> dict(status, cost, dobj, iters, primal, dual, yc, runtime).  variant: of
+    oracle/qp_core.c (1 = the CUDA kernel's thin factor, 0 = the full factor the golden fixtures were made with)."""
     from oracle.qp_c import CoreC
     from oracle.condense import Condensed
     from oracle import certify as cert
-    core = CoreC(model, variant=1)
+    core = CoreC(model, variant=variant)
     cond = Condensed(model)
     L = pd.layout
 
