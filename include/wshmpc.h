@@ -84,6 +84,21 @@ int wshmpc_set_search_rule(wshmpc_handle *h, int rule);
  * representable; only the leading run of assigned binaries is eliminated from the node's QP.  Sticky per handle. */
 int wshmpc_set_branch_order(wshmpc_handle *h, const int *order);
 
+/* node rule of the device-side branch and bound (wshmpc_bnb_solve, wshmpc_closed_loop).  Sticky per handle.
+ *   0  the structured search (default): branch on the first unassigned binary of the branching order, a node is an incumbent
+ *      iff every binary is pinned, a child's bound = parent cost + the multiplier of the bound that moves (controller.py:395-429).
+ *   1  the conventional MIQP branch and bound of feedforward_miqp (controller.py:530-582), the paper's "Gurobi fair" comparator
+ *      (feedforward_gurobi, controller.py:723-776) without Gurobi: after a node's solve, branch on the unassigned binary
+ *      j = t*nub+i whose relaxed value u is the most fractional (|u - rint(u)| largest, ties to the smaller j; the branching
+ *      order is ignored); the node is an incumbent when that fractionality is <= 1e-9; children [value 0, value 1] both get
+ *      bound = the parent's relaxation cost and start from the parent's record.  Candidate selection (wshmpc_set_search_rule)
+ *      is unchanged.  A MIP start is a tree from wshmpc_tree_init_guess.
+ *   2  rule 1, and in wshmpc_closed_loop a MIP start at every step of an instance whose previous step left an incumbent: the
+ *      previous incumbent's binaries shifted by one step, zero at the end (shift_binary_solution, controller.py:586-588); no
+ *      guess on step 0 of a `fresh` launch.
+ * Rules 1 and 2 run cold trees only: wshmpc_closed_loop with warm = 1 fails under them. */
+int wshmpc_set_node_rule(wshmpc_handle *h, int rule);
+
 /* K1 -- batched node QP relaxation.
  * Replaces, per node: controller._solve_subproblem (controller.py:229-271) = _set_bound_binaries
  * (:273-298) + BoundedQP.optimize (bounded_qp.py:200-228) + SubproblemSolution.from_controller
@@ -169,6 +184,14 @@ int wshmpc_bnb_solve(wshmpc_handle *h, int n_inst, const double *d_x0, const int
 
 /* cold start: every instance gets the single root node Node({}) with lb = -inf (branch_and_bound.py:432) */
 int wshmpc_tree_init_root(wshmpc_handle *h, int n_inst, const wshmpc_tree *tree);
+
+/* MIP start (the ub_guess of feedforward_miqp, controller.py:552-556): instance k gets node 0 = the guess (every binary pinned,
+ * lb = -inf, no record: solved first under best_first, from the empty working set) and node 1 = the root, or the root alone
+ * where d_has[k] == 0.  The guess's solve counts in n_solves; after it the node is never a candidate again (its lb is the
+ * incumbent's cost or +inf).
+ *   d_guess [n_inst][nb] binary values j = t*nub+i, rounded with rint (to 0 or 1)
+ *   d_has   [n_inst] or NULL (every instance has a guess) */
+int wshmpc_tree_init_guess(wshmpc_handle *h, int n_inst, const wshmpc_tree *tree, const double *d_guess, const int *d_has);
 
 /* K2 + K4 -- warm start for the next time step, one CTA per instance, one warp per leaf.
  * Replaces construct_warm_start (controller.py:431-564) = _retain_leaf (:615-633) + identifier shift

@@ -42,8 +42,8 @@ def load_library():
     return _lib
 
 
-EXPORTS = ('wshmpc_last_error', 'wshmpc_ctas_per_sm', 'wshmpc_set_search_rule', 'wshmpc_set_branch_order', 'wshmpc_create', 'wshmpc_destroy', 'wshmpc_get_layout', 'wshmpc_solve_nodes',
-           'wshmpc_tree_init_root', 'wshmpc_bnb_solve', 'wshmpc_shift_tree', 'wshmpc_closed_loop', 'wshmpc_mailbox_create', 'wshmpc_mailbox_destroy', 'wshmpc_lp_batch')
+EXPORTS = ('wshmpc_last_error', 'wshmpc_ctas_per_sm', 'wshmpc_set_search_rule', 'wshmpc_set_branch_order', 'wshmpc_set_node_rule', 'wshmpc_create', 'wshmpc_destroy', 'wshmpc_get_layout', 'wshmpc_solve_nodes',
+           'wshmpc_tree_init_root', 'wshmpc_tree_init_guess', 'wshmpc_bnb_solve', 'wshmpc_shift_tree', 'wshmpc_closed_loop', 'wshmpc_mailbox_create', 'wshmpc_mailbox_destroy', 'wshmpc_lp_batch')
 
 
 class _Mailbox(C.Structure):
@@ -165,6 +165,11 @@ class Handle(object):
         """0 best_first, 1 depth_first, 2 breadth_first (branch_and_bound.py:501-563) for the device-side B&B."""
         _check(self.lib.wshmpc_set_search_rule(self._h, int(rule)))
 
+    def set_node_rule(self, rule):
+        """0 the structured search (default), 1 the conventional MIQP branch and bound of feedforward_miqp (most fractional
+        binary, controller.py:530-582), 2 rule 1 with a MIP start at every step of the fused closed loop (wshmpc_set_node_rule)."""
+        _check(self.lib.wshmpc_set_node_rule(self._h, int(rule)))
+
     def set_branch_order(self, order):
         """Static branching order of the device-side B&B: permutation of the binaries j = t * nub + i, or None for the
         chronological order of branch_in_time (wshmpc_set_branch_order)."""
@@ -223,6 +228,17 @@ class Handle(object):
 
     def tree_init_root(self, tree):
         _check(self.lib.wshmpc_tree_init_root(self._h, tree.n_inst, C.byref(tree.c)))
+
+    def tree_init_guess(self, tree, guess, has=None):
+        """MIP start (wshmpc_tree_init_guess): instance k gets [guess, root], or the root alone where has[k] == 0.
+        guess [n_inst, nb] CUDA fp64 tensor of binary values (rounded on the device); has [n_inst] CUDA int32 tensor or None."""
+        import torch
+        N = tree.n_inst
+        assert guess.is_cuda and guess.dtype == torch.float64 and guess.is_contiguous() and tuple(guess.shape) == (N, self.pd.nb)
+        if has is not None:
+            assert has.is_cuda and has.dtype == torch.int32 and has.is_contiguous() and tuple(has.shape) == (N,)
+        P = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
+        _check(self.lib.wshmpc_tree_init_guess(self._h, N, C.byref(tree.c), P(guess), P(has)))
 
     def bnb_solve(self, x0, tree, tol=0., max_solves=1024, active=None, out=None, trace=False, totals=None):
         """K3: branch and bound of every instance of `tree` at states x0 [n_inst, nx] (CUDA fp64 tensor).

@@ -19,8 +19,19 @@ def shard(n_total, rank, world):
 
 class ClosedLoop(object):
 
-    def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=512, n_slots=None):
+    def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
+                 mip_start=True):
+        """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
+        paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
+        incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
+        tree holds (default 512; 2 for the comparator, whose trees hold a guess and a root)."""
         import torch
+        if comparator and warm:
+            raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
+        if max_roots is None:
+            max_roots = 2 if comparator else 512
+        self.comparator, self.mip_start = comparator, mip_start
+        self.node_rule = (2 if mip_start else 1) if comparator else 0
         self.ctl, self.n_inst, self.warm, self.tol = controller, n_inst, warm, tol
         self.max_solves, self.max_roots = max_solves, max_roots
         slots = n_slots if n_slots is not None else min(n_inst, controller.default_slots())
@@ -68,6 +79,47 @@ class ClosedLoop(object):
         from .rebalance import rebalance
         return rebalance(self.trees[self.cur], self.x, self.active, self.gid, group, min_gap)
 
+    def _init_tree(self, tree):
+        """Root node of a cold step; in comparator mode with mip_start, [MIP start, root] for every instance whose previous
+        step left an incumbent (what the fused loop builds on the device, wshmpc_set_node_rule 2)."""
+        import torch
+        h = self.h
+        if self.node_rule == 2 and not self.fresh:
+            T, nx, nu, nub = self.ctl.T, self.ctl.mld.nx, self.ctl.mld.nu, self.ctl.mld.nub
+            ub = self.out['primal'][:, (T + 1) * nx:].reshape(self.n_inst, T, nu)[:, :, nu - nub:]
+            guess = torch.zeros((self.n_inst, T, nub), dtype=torch.float64, device=ub.device)
+            guess[:, :T - 1] = torch.round(ub[:, 1:])                    # shift_binary_solution (controller.py:586-588)
+            has = ((self.active != 0) & torch.isfinite(self.out['cost'])).to(torch.int32)
+            h.tree_init_guess(tree, guess.reshape(self.n_inst, T * nub), has)
+        else:
+            h.tree_init_root(tree)
+        self.launches += 1
+        self.fresh = False
+
+    def _bnb(self, tree):
+        h = self.h
+        if self.node_rule:
+            h.set_node_rule(self.node_rule)
+        try:
+            h.bnb_solve(self.x, tree, tol=self.tol, max_solves=self.max_solves, active=self.active, out=self.out,
+                        totals=self.totals)
+        finally:
+            if self.node_rule:
+                h.set_node_rule(0)
+        self.launches += 1
+
+    def _closed_loop(self, n_steps, par, e, logs, mailbox=None):
+        h = self.h
+        fresh = self.fresh if (self.warm or self.comparator) else True
+        if self.node_rule:
+            h.set_node_rule(self.node_rule)
+        try:
+            return h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, e, self.active, self.trees, self.out,
+                                 tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mailbox)
+        finally:
+            if self.node_rule:
+                h.set_node_rule(0)
+
     def step(self, e=None, x=None):
         """One receding-horizon step of every instance.  `x` (optional, [n_inst, nx] CUDA tensor)
         overrides the state (measured state fed back from the host); `e` is the model error e_t."""
@@ -76,15 +128,12 @@ class ClosedLoop(object):
             self.x.copy_(x)
         tree = self.trees[self.cur]
         if self.fresh or not self.warm:
-            h.tree_init_root(tree); self.launches += 1
-            self.fresh = False
+            self._init_tree(tree)
         if self.events is not None:
             import torch
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             ev[0].record()
-        h.bnb_solve(self.x, tree, tol=self.tol, max_solves=self.max_solves, active=self.active, out=self.out,
-                    totals=self.totals)
-        self.launches += 1
+        self._bnb(tree)
         if self.events is not None:
             ev[1].record()
         # K2 + K4 (in cold mode only its plant update matters: the next step re-initialises the root)
@@ -109,10 +158,8 @@ class ClosedLoop(object):
         h = self.h
         tree = self.trees[self.cur]
         if self.fresh or not self.warm:
-            h.tree_init_root(tree); self.launches += 1
-            self.fresh = False
-        h.bnb_solve(self.x, tree, tol=self.tol, max_solves=self.max_solves, active=self.active, out=self.out, totals=self.totals)
-        self.launches += 1
+            self._init_tree(tree)
+        self._bnb(tree)
         nx, nu, T = self.ctl.mld.nx, self.ctl.mld.nu, self.ctl.T
         prim = self.out['primal'].cpu().numpy()
         x_now = self.x.cpu().numpy()
@@ -141,16 +188,11 @@ class ClosedLoop(object):
         form of calling step() n_steps times, without a barrier between the steps of different instances.
         e: [n_steps, n_inst, nx] CUDA tensor of model errors or None.  Returns per-step logs
         (cost, u0, n_solves, status), each [n_steps, n_inst, ...]; self.x holds the final states."""
-        h = self.h
-        if self.warm:
-            par, fresh = self.cur, self.fresh
-        else:
-            par, fresh = self.cur, True
+        par = self.cur
         # states and trees flip together: make the state parity equal to the tree parity
         if self.xpar != par:
             self.xbuf[par].copy_(self.xbuf[self.xpar]); self.xpar = par
-        logs = h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, e, self.active, self.trees, self.out,
-                             tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs)
+        logs = self._closed_loop(n_steps, par, e, logs)
         self.launches += 2
         self.fresh = False
         self.cur = (self.cur + n_steps) & 1
@@ -175,17 +217,13 @@ class ClosedLoop(object):
             self._mailbox = Mailbox(h, N)
         mb = self._mailbox
         mb.clear()
-        if self.warm:
-            par, fresh = self.cur, self.fresh
-        else:
-            par, fresh = self.cur, True
+        par = self.cur
         if self.xpar != par:
             self.xbuf[par].copy_(self.xbuf[self.xpar]); self.xpar = par
         nx, nu = self.ctl.mld.nx, self.ctl.mld.nu
         host = dict(u0=np.full((n_steps, N, nu), np.nan), x1=np.zeros((n_steps, N, nx)), cost=np.full((n_steps, N), np.inf),
                     status=np.zeros((n_steps, N), dtype=np.int32))
-        logs = h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, None, self.active, self.trees, self.out,
-                             tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mb)
+        logs = self._closed_loop(n_steps, par, None, logs, mailbox=mb)
         self.launches += 2
         seen = np.zeros(N, dtype=np.int32)
         t_end = time.time() + timeout_s

@@ -583,6 +583,66 @@ class HybridModelPredictiveController(object):
 
     feedforward_gurobi = feedforward_miqp       # the reference's name for the comparator leg (there is no Gurobi underneath)
 
+    def feedforward_miqp_batch(self, x0, ub_guess=None, tol=0., max_solves=None, n_slots=None, active=None, trace=False):
+        """`feedforward_miqp` for many independent initial states in ONE launch of the device-side branch and bound under the
+        conventional node rule (wshmpc_set_node_rule 1): most fractional binary, integral relaxations are incumbents, bounds
+        are relaxation values only; candidate selection is the handle's search rule (best_first by default).
+        x0 [N, nx]; ub_guess: MIP start [N, T, nub], or [T, nub] for every instance, or None.
+        Returns (result dict of CUDA tensors, tree) like feedforward_batch; nothing is synchronised.  With trace=True,
+        res['trace'][k, 2 s] is the node solved s-th; the tree keeps each solved node's identifier and relaxation cost (lb)."""
+        self._require_gpu()
+        ms = self.max_solves if max_solves is None else max_solves
+        N = x0.shape[0]
+        T, nub = self.T, self.mld.nub
+        h = self.handle(n_slots if n_slots is not None else max(self._n_slots, min(N, self.default_slots())))
+        x0 = self._as_device(x0, (N, self.mld.nx))
+        tree = self.new_tree(N, 2, ms)
+        if ub_guess is None:
+            h.tree_init_root(tree)
+        else:
+            g = np.asarray(ub_guess, dtype=float) if not hasattr(ub_guess, 'is_cuda') else ub_guess
+            g = self._as_device(g, tuple(g.shape))
+            if g.dim() == 2:
+                g = g[None].expand(N, T, nub)
+            if tuple(g.shape) != (N, T, nub):
+                raise ValueError('ub_guess must be [N, T, nub] or [T, nub]')
+            h.tree_init_guess(tree, g.reshape(N, T * nub).contiguous())
+        h.set_node_rule(1)
+        try:
+            res = h.bnb_solve(x0, tree, tol=tol, max_solves=ms, active=active, trace=trace)
+        finally:
+            h.set_node_rule(0)              # launch parameters are copied at the launch: the rule can go back at once
+        res['x0'] = x0
+        return res, tree
+
+    def feedforward_miqp_device(self, x0, gurobi_params={}, ub_guess=None, tol=0.):
+        """`feedforward_miqp` (same arguments, same result: variables {'x', 'uc', 'ub'} stacked over time with 'ub' rounded,
+        objective, nodes, solver seconds) as one instance of `feedforward_miqp_batch`: the whole search in one launch, no host
+        round trip per node.  It visits the same nodes in the same order as the host loop.  Children start from their
+        parent's record, which is what `Method` = 1 (the default) means; any other `Method` solves every node from the empty
+        working set, and that runs the host loop."""
+        import torch
+        self._set_gurobi_params(gurobi_params)
+        if self.qp.Params.Method != 1:
+            return self.feedforward_miqp(x0, gurobi_params, ub_guess=ub_guess, tol=tol)
+        start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        start.record()
+        guess = None if ub_guess is None else np.asarray(ub_guess, dtype=float)[None]
+        res, _ = self.feedforward_miqp_batch(np.asarray(x0, dtype=float)[None], ub_guess=guess, tol=tol, n_slots=1)
+        end.record()
+        end.synchronize()
+        status, nodes = int(res['status'][0]), int(res['n_solves'][0])
+        if status >= 2:
+            raise RuntimeError('device branch and bound failed with status %d (2 = capacity, 3 = QP iteration limit)' % status)
+        seconds = start.elapsed_time(end) * 1e-3
+        if status == 1:
+            return None, np.inf, nodes, seconds
+        T, nx, nu, nuc = self.T, self.mld.nx, self.mld.nu, self.problem.nuc
+        rec = res['primal'][0].cpu().numpy()
+        U = rec[(T + 1) * nx:].reshape(T, nu)
+        variables = {'x': rec[:(T + 1) * nx].reshape(T + 1, nx).copy(), 'uc': U[:, :nuc].copy(), 'ub': np.round(U[:, nuc:])}
+        return variables, float(res['cost'][0]), nodes, seconds
+
     def shift_binary_solution(self, ub):
         """controller.py:811-812."""
         return np.vstack((ub[1:], np.zeros(self.mld.nub)))

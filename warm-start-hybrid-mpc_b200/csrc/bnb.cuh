@@ -21,6 +21,13 @@ struct TreeView {
 #define BNB_CAPACITY 2
 #define BNB_QP_LIMIT 3
 
+// node rules of K3 (wshmpc_set_node_rule): 0 the structured search (branch on the first unassigned binary of the branching
+// order, a node is an incumbent iff every binary is pinned, children inherit dual bounds); 1 the conventional MIQP branch and
+// bound of feedforward_miqp (controller.py:530-582); 2 = 1 with a MIP start at every step of the fused closed loop
+#define BNB_RULE_MIQP 1
+#define BNB_RULE_MIQP_START 2
+#define BNB_INTEGRAL_TOL 1e-9     // largest |u - rint(u)| of an integral relaxation (feedforward_miqp)
+
 // per-slot scratch of the B&B kernel (doubles): lb | ub | primal record | cost | dobj
 __host__ __device__ __forceinline__ size_t bnb_scratch_doubles(int nb, int n_primal) { return 2 * (size_t)nb + n_primal + 4; }
 
@@ -40,6 +47,9 @@ __global__ void init_root_kernel(int n_inst, TreeView tr)
 // K3
 // ---------------------------------------------------------------------------------------------
 // branch and bound of ONE instance by the calling CTA (all threads).  Returns the status.
+// RULE: 0 the structured search, 1 the conventional MIQP rule (BNB_RULE_MIQP; the branching binary is chosen AFTER the
+// node's solve, from its relaxation) -- a template parameter, so that the default kernels carry none of the rule-1 code.
+template <int RULE>
 __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, const SlotPtrs &sp, double *y, double *sc, int *iters_s,
                                    int inst, const double *xi, const TreeView &tr, double tol, int max_solves,
                                    double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *trace,
@@ -95,7 +105,7 @@ __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, 
         block_argmin(first_free, ff, SMV(red), SMI(ired));
         const int d_elim = ff < 0 ? nb : ff;
         int jb = d_elim;
-        if (P.border) {
+        if (RULE == 0 && P.border) {
             for (int p = WS_TID; p < nb; p += WS_NT) {
                 const int j = P.border[p];
                 if (!((mw[j >> 5] >> (j & 31)) & 1u) && fo < 0) { fo = p; first_in_order = (double)p; }
@@ -154,16 +164,33 @@ __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, 
         const int myrec = nr;
         iters += *iters_s; ksum += k; kmx = max(kmx, iters_s[1]); dsum += min(d_elim, P.n_elim); k0sum += iters_s[2] & 0xffff;
         ++nr; ++solves;
+        bool integral = d == nb;
+        if (RULE != 0 && cost < cutoff) {
+            // conventional MIQP rule (controller.py:567-576): the unassigned binary j = t nub + i whose relaxed value u is the
+            // most fractional, |u - rint(u)| largest, ties to the smaller j (np.argmax); pinned binaries count as 0.  The
+            // node is integral (an incumbent) when that largest fractionality is <= BNB_INTEGRAL_TOL.
+            const double *ubp = prim + (size_t)(P.T + 1) * P.nx + P.nuc;
+            double fr = 0.; int fj = -1;
+            for (int j = WS_TID; j < nb; j += WS_NT) {
+                if ((mw[j >> 5] >> (j & 31)) & 1u) continue;
+                const double u = ubp[(j / P.nub) * P.nu + j % P.nub], f = fabs(u - rint(u));
+                if (fj < 0 || f > fr) { fr = f; fj = j; }
+            }
+            block_argmax(fr, fj, SMV(red), SMI(ired));
+            integral = fj < 0 || fr <= BNB_INTEGRAL_TOL;
+            jb = fj;
+        }
         // ---- prune / incumbent / branch (branch_and_bound.py:476-489)
         if (cost >= cutoff) {
             // pruned: the node stays a leaf with its new bound
-        } else if (d == nb) {
+        } else if (integral) {
             inc = bi; ub = cost;
             double *ip = inc_primal + (size_t)inst * P.n_primal;
             for (int j = WS_TID; j < P.n_primal; j += WS_NT) ip[j] = prim[j];
         } else {
-            // children [value 0, value 1] of binary jb = (t, i); bound += multiplier of the bound that moves
-            const double l0 = cost + dual[P.off_nuub + jb], l1 = cost + dual[P.off_nulb + jb];
+            // children [value 0, value 1] of binary jb = (t, i); bound += multiplier of the bound that moves (rule 0) or
+            // = the parent's relaxation cost (conventional rule: no dual-bound inheritance)
+            const double l0 = RULE == 0 ? cost + dual[P.off_nuub + jb] : cost, l1 = RULE == 0 ? cost + dual[P.off_nulb + jb] : cost;
             unsigned int *c0 = bits + (size_t)nn * tr.words, *c1 = c0 + tr.words;
             unsigned int *m0 = mask + (size_t)nn * tr.words, *m1 = m0 + tr.words;
             for (int w = WS_TID; w < tr.words; w += WS_NT) {
@@ -195,7 +222,7 @@ __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, 
     return st;
 }
 
-template <int LANES>
+template <int LANES, int RULE>
 __device__ __forceinline__ void
 bnb_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double *scratch, int *work_counter, int n_slots,
            int n_inst, const double *__restrict__ x0, const int *__restrict__ active, const TreeView &tr,
@@ -224,7 +251,7 @@ bnb_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double 
             if (WS_TID == 0) { inc_cost[inst] = INFINITY; inc_node[inst] = -1; n_solves[inst] = 0; status_out[inst] = BNB_INFEASIBLE; }
             continue;
         }
-        const int st = bnb_instance(P, cx, sp, y, sc, iters_s, inst, x0 + (size_t)inst * P.nx, tr, tol, max_solves,
+        const int st = bnb_instance<RULE>(P, cx, sp, y, sc, iters_s, inst, x0 + (size_t)inst * P.nx, tr, tol, max_solves,
                                     inc_cost, inc_node, inc_primal, n_solves, trace, totals);
         if (WS_TID == 0) status_out[inst] = st;
     }
@@ -239,14 +266,27 @@ bnb_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double 
 // one lane per CTA: 255 registers per thread (launches that cannot fill two lanes per SM: latency mode, large systems)
 __global__ void __launch_bounds__(WS_NT, 1) bnb_kernel_1(WS_BNB_ARGS)
 #if WS_TU_HAS(3)
-{ bnb_body<1>(WS_BNB_PASS); }
+{ bnb_body<1, 0>(WS_BNB_PASS); }
 #else
 ;
 #endif
 // WS_MAXL lanes per CTA: 65536 / (WS_MAXL WS_NT) registers per thread (throughput mode)
 __global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) bnb_kernel_m(WS_BNB_ARGS)
 #if WS_TU_HAS(4)
-{ bnb_body<WS_MAXL>(WS_BNB_PASS); }
+{ bnb_body<WS_MAXL, 0>(WS_BNB_PASS); }
+#else
+;
+#endif
+// the same two builds under the conventional MIQP node rule (wshmpc_set_node_rule 1 or 2)
+__global__ void __launch_bounds__(WS_NT, 1) bnb_miqp_kernel_1(WS_BNB_ARGS)
+#if WS_TU_HAS(7)
+{ bnb_body<1, BNB_RULE_MIQP>(WS_BNB_PASS); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) bnb_miqp_kernel_m(WS_BNB_ARGS)
+#if WS_TU_HAS(8)
+{ bnb_body<WS_MAXL, BNB_RULE_MIQP>(WS_BNB_PASS); }
 #else
 ;
 #endif
@@ -623,7 +663,42 @@ __device__ __forceinline__ void init_root(const TreeView &tr, int k)
     for (int w = 0; w < tr.words; ++w) { tr.bits[o * tr.words + w] = 0u; tr.mask[o * tr.words + w] = 0u; }
 }
 
-template <int LANES>
+// MIP start (feedforward_miqp's ub_guess, controller.py:552-556): node 0 = the guess, every binary j pinned to rint(g(j))
+// (a value of 0 or 1), lb = -inf and no record (solved from the empty working set, first under best-first); node 1 = the
+// root.  Threads tid = 0 .. nt - 1 of the caller share the work; the caller provides the barrier.
+template <class Guess>
+__device__ __forceinline__ void init_guess(const TreeView &tr, int k, int nb, Guess g, int tid, int nt)
+{
+    const size_t o = (size_t)k * tr.cap_nodes;
+    for (int w = tid; w < tr.words; w += nt) {
+        unsigned int b = 0u, m = 0u;
+        for (int q = 0; q < 32 && 32 * w + q < nb; ++q) {
+            m |= 1u << q;
+            if (rint(g(32 * w + q)) != 0.) b |= 1u << q;
+        }
+        tr.bits[o * tr.words + w] = b; tr.mask[o * tr.words + w] = m;
+        tr.bits[(o + 1) * tr.words + w] = 0u; tr.mask[(o + 1) * tr.words + w] = 0u;
+    }
+    if (tid == 0) {
+        tr.n_nodes[k] = 2; tr.n_recs[k] = 0;
+        tr.depth[o] = nb; tr.alive[o] = 1; tr.rec[o] = -1; tr.lb[o] = -INFINITY;
+        tr.depth[o + 1] = 0; tr.alive[o + 1] = 1; tr.rec[o + 1] = -1; tr.lb[o + 1] = -INFINITY;
+    }
+}
+
+#if WS_TU_HAS(0)
+// wshmpc_tree_init_guess: [guess, root] for every instance with has[k] != 0 (has = null: all), the root alone otherwise
+__global__ void init_guess_kernel(int n_inst, int nb, TreeView tr, const double *__restrict__ guess, const int *__restrict__ has)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_inst) return;
+    if (has && !has[k]) { init_root(tr, k); return; }
+    const double *gk = guess + (size_t)k * nb;
+    init_guess(tr, k, nb, [&](int j) { return gk[j]; }, 0, 1);
+}
+#endif
+
+template <int LANES, int RULE>
 __device__ __forceinline__ void
 closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double *scratch, const LoopView &L, int n_slots, int n_inst,
                    const TreeView &t0, const TreeView &t1, double tol, int max_solves,
@@ -739,7 +814,16 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
             const double *xc = L.x + (size_t)par * xs;
             double *xn = L.x + (size_t)(par ^ 1) * xs;
             if (!L.warm || (t == 0 && L.fresh)) {
-                if (WS_TID == 0) init_root(cur, inst);
+                if (RULE != 0 && P.node_rule == BNB_RULE_MIQP_START && !(t == 0 && L.fresh) && L.active[inst] && inc_cost[inst] < INFINITY) {
+                    // MIP start: the previous step's incumbent binaries shifted by one step, zero at the end
+                    // (shift_binary_solution, controller.py:586-588)
+                    const double *ub1 = inc_primal + (size_t)inst * P.n_primal + (size_t)(P.T + 1) * P.nx + P.nu + P.nuc;
+                    const int T = P.T, nub = P.nub, nu = P.nu;
+                    init_guess(cur, inst, P.nb, [&](int j) { const int tt = j / nub; return tt < T - 1 ? ub1[tt * nu + j % nub] : 0.; },
+                               WS_TID, WS_NT);
+                } else if (WS_TID == 0) {
+                    init_root(cur, inst);
+                }
                 WS_SYNC();
             }
             int st;
@@ -748,7 +832,7 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                 st = BNB_INFEASIBLE;
                 WS_SYNC();
             } else {
-                st = bnb_instance(P, cx, sp, y, sc, iters_s, inst, xc + (size_t)inst * P.nx, cur, tol, max_solves,
+                st = bnb_instance<RULE>(P, cx, sp, y, sc, iters_s, inst, xc + (size_t)inst * P.nx, cur, tol, max_solves,
                                   inc_cost, inc_node, inc_primal, n_solves, nullptr, totals);
             }
             if (WS_TID == 0) {
@@ -793,13 +877,26 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
     n_solves, status_out, totals
 __global__ void __launch_bounds__(WS_NT, 1) closed_loop_kernel_1(WS_LOOP_ARGS)
 #if WS_TU_HAS(5)
-{ closed_loop_body<1>(WS_LOOP_PASS); }
+{ closed_loop_body<1, 0>(WS_LOOP_PASS); }
 #else
 ;
 #endif
 __global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_kernel_m(WS_LOOP_ARGS)
 #if WS_TU_HAS(6)
-{ closed_loop_body<WS_MAXL>(WS_LOOP_PASS); }
+{ closed_loop_body<WS_MAXL, 0>(WS_LOOP_PASS); }
+#else
+;
+#endif
+// the fused loop of the conventional MIQP comparator (node rule 1 or 2; cold trees only)
+__global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_kernel_1(WS_LOOP_ARGS)
+#if WS_TU_HAS(9)
+{ closed_loop_body<1, BNB_RULE_MIQP>(WS_LOOP_PASS); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_kernel_m(WS_LOOP_ARGS)
+#if WS_TU_HAS(10)
+{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP>(WS_LOOP_PASS); }
 #else
 ;
 #endif

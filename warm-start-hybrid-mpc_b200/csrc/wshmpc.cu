@@ -305,6 +305,10 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     WS_CUDA(cudaFuncSetAttribute(bnb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(bnb_miqp_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(bnb_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * bnb_scratch_doubles(p->nb, L.primal) * sizeof(double))); h->allocs.push_back(d); h->scratch = (double *)d;
     WS_CUDA(cudaMalloc(&d, 64)); h->allocs.push_back(d); h->work_counter = (int *)d;
     h->shift_smem = shift_smem_bytes(P, optin, &h->shift_stage);
@@ -346,6 +350,14 @@ extern "C" int wshmpc_set_search_rule(wshmpc_handle *h, int rule)
     if (!h) WS_FAIL(-1, "null handle");
     if (rule < 0 || rule > 2) WS_FAIL(-1, "search rule %d: 0 best_first, 1 depth_first, 2 breadth_first", rule);
     h->P.search_rule = rule; h->P1.search_rule = rule;
+    return 0;
+}
+
+extern "C" int wshmpc_set_node_rule(wshmpc_handle *h, int rule)
+{
+    if (!h) WS_FAIL(-1, "null handle");
+    if (rule < 0 || rule > 2) WS_FAIL(-1, "node rule %d: 0 structured, 1 conventional MIQP, 2 conventional MIQP with a MIP start", rule);
+    h->P.node_rule = rule; h->P1.node_rule = rule;
     return 0;
 }
 
@@ -421,6 +433,18 @@ extern "C" int wshmpc_tree_init_root(wshmpc_handle *h, int n_inst, const wshmpc_
     return 0;
 }
 
+extern "C" int wshmpc_tree_init_guess(wshmpc_handle *h, int n_inst, const wshmpc_tree *tree, const double *d_guess, const int *d_has)
+{
+    if (!h) WS_FAIL(-1, "null handle");
+    if (n_inst <= 0) return 0;
+    if (!d_guess) WS_FAIL(-1, "null guess");
+    TreeView tv; int rc = tree_view(h, tree, &tv); if (rc) return rc;
+    WS_CUDA(cudaSetDevice(h->device));
+    init_guess_kernel<<<(n_inst + 127) / 128, 128, 0, h->stream>>>(n_inst, h->P.nb, tv, d_guess, d_has);
+    WS_CUDA(cudaGetLastError());
+    return 0;
+}
+
 extern "C" int wshmpc_bnb_solve(wshmpc_handle *h, int n_inst, const double *d_x0, const int *d_active,
                                 const wshmpc_tree *tree, double tol, int max_solves,
                                 double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
@@ -434,12 +458,16 @@ extern "C" int wshmpc_bnb_solve(wshmpc_handle *h, int n_inst, const double *d_x0
     WS_CUDA(cudaSetDevice(h->device));
     WS_CUDA(cudaMemsetAsync(h->work_counter, 0, sizeof(int), h->stream));
     const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
-    if (slots <= h->n_sm || h->P.lanes == 1)
-        bnb_kernel_1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
+    const bool one = slots <= h->n_sm || h->P.lanes == 1, miqp = h->P.node_rule != 0;
+    // the node rule picks the kernel: the structured search's kernels carry no code of the conventional rule
+    auto *k1 = miqp ? bnb_miqp_kernel_1 : bnb_kernel_1;
+    auto *km = miqp ? bnb_miqp_kernel_m : bnb_kernel_m;
+    if (one)
+        k1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
             h->P1, h->slot_d, h->slot_i, h->ybuf, h->scratch, h->work_counter, slots, n_inst, d_x0, d_active, tv, tol, max_solves,
             d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_trace, d_totals);
     else
-    bnb_kernel_m<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
+    km<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
         h->P, h->slot_d, h->slot_i, h->ybuf, h->scratch, h->work_counter, slots, n_inst, d_x0, d_active, tv, tol, max_solves,
         d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_trace, d_totals);
     WS_CUDA(cudaGetLastError());
@@ -479,6 +507,7 @@ extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loo
         WS_FAIL(-1, "null argument");
     if (h->P.T < 2) WS_FAIL(-1, "tree shifting needs T >= 2");
     if (h->P.nub > 32) WS_FAIL(-1, "tree shifting supports nub <= 32");
+    if (loop->warm && h->P.node_rule != 0) WS_FAIL(-1, "node rule %d: the conventional MIQP search runs cold trees only (warm = 0)", h->P.node_rule);
     if ((size_t)h->P.so.pool_sz < shift_smem_doubles(h->P, WS_NT)) WS_FAIL(-4, "shared memory too small for the fused warm start");
     if ((long long)n_inst * (loop->n_steps + 1) > 0x7fffffffLL) WS_FAIL(-1, "too many tasks");
     TreeView v0, v1; int rc = tree_view(h, tree0, &v0); if (rc) return rc;
@@ -509,12 +538,15 @@ extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loo
     loop_init_kernel<<<(n_items + 255) / 256, 256, 0, h->stream>>>(n_inst, n_items, L);
     WS_CUDA(cudaGetLastError());
     const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
+    const bool miqp = h->P.node_rule != 0;
+    auto *k1 = miqp ? closed_loop_miqp_kernel_1 : closed_loop_kernel_1;
+    auto *km = miqp ? closed_loop_miqp_kernel_m : closed_loop_kernel_m;
     if (slots <= h->n_sm || h->P.lanes == 1)
-        closed_loop_kernel_1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
+        k1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
             h->P1, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
             d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals);
     else
-    closed_loop_kernel_m<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
+    km<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
         h->P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
         d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals);
     WS_CUDA(cudaGetLastError());
