@@ -274,6 +274,35 @@ int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop,
                        double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
                        int *d_status, unsigned long long *d_totals);
 
+/* The nonlinear benchmark plant on the device: the cart-pole between two soft walls (plants.CartPoleWithWalls), integrated
+ * by explicit Euler with n_sub sub-steps of dt / n_sub and the cart force held constant over dt -- the rule of
+ * CartPoleWithWalls.simulate.  The state is x = (qc, qp, qc', qp') (nx = 4); the cart force is input component fc_index. */
+#define WSHMPC_PLANT_CARTPOLE_NPARAM 7      /* mc, mp, l, d, stiffness, damping, g */
+typedef struct {
+    int kind;              /* 1: cart-pole between two soft walls (plants.CartPoleWithWalls); other values are errors */
+    int n_sets;            /* 1: every instance uses set 0;  n_inst (or n for wshmpc_plant_step): set k for instance k */
+    const double *d_params;/* [n_sets][WSHMPC_PLANT_CARTPOLE_NPARAM], device */
+    double dt;             /* sample time of the controller's model */
+    int n_sub;             /* Euler sub-steps per sample */
+    int fc_index;          /* input component applied as the cart force */
+    double *d_log_x;       /* [n_steps][n_inst][nx] state after every step, or NULL (closed loop only) */
+} wshmpc_plant;
+
+/* d_x_out[i] = the plant's state after dt from d_x[i] under the input d_u[i] (one thread per state; asynchronous).
+ *   d_x, d_x_out [n][nx] (may not overlap), d_u [n][nu] */
+int wshmpc_plant_step(wshmpc_handle *h, const wshmpc_plant *pl, int n, const double *d_x, const double *d_u, double *d_x_out);
+
+/* wshmpc_closed_loop against the nonlinear plant, advanced on the device.  For every step t of a live instance i with an
+ * incumbent:  u0 = the incumbent's first input,  x_meas = Phi(x_t, u0[fc_index]; set i) + d_e[t][i] (loop->d_e optional:
+ * an additive disturbance on the plant output),  the warm start is corrected with e = x_meas - x_1|t (construct_warm_start's
+ * e0), and x_{t+1} = x_meas.  An instance without an incumbent keeps its state and is switched off.  Results equal calling
+ * wshmpc_bnb_solve, wshmpc_plant_step and wshmpc_shift_tree (with e0 = e) once per step.  A mailbox is an error (the host is
+ * the plant there). */
+int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                             const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
+                             double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                             int *d_status, unsigned long long *d_totals);
+
 /* Batched small LPs in standard form (SURVEY.md 8f-2):   min c'y  s.t.  E y = r,  y >= 0   for n_lp problems at once,
  * one CTA per LP (two-phase tableau simplex in shared memory).  Replaces the host LP loops the reference runs through
  * BoundedQP / Gurobi while a controller is built: `_update_mu` (controller.py:186-227: h_Tm1.size LPs sharing [F G]' and h,

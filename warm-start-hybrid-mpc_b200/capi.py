@@ -43,7 +43,8 @@ def load_library():
 
 
 EXPORTS = ('wshmpc_last_error', 'wshmpc_ctas_per_sm', 'wshmpc_set_search_rule', 'wshmpc_set_branch_order', 'wshmpc_set_node_rule', 'wshmpc_create', 'wshmpc_destroy', 'wshmpc_get_layout', 'wshmpc_solve_nodes',
-           'wshmpc_tree_init_root', 'wshmpc_tree_init_guess', 'wshmpc_bnb_solve', 'wshmpc_shift_tree', 'wshmpc_closed_loop', 'wshmpc_mailbox_create', 'wshmpc_mailbox_destroy', 'wshmpc_lp_batch')
+           'wshmpc_tree_init_root', 'wshmpc_tree_init_guess', 'wshmpc_bnb_solve', 'wshmpc_shift_tree', 'wshmpc_closed_loop', 'wshmpc_mailbox_create', 'wshmpc_mailbox_destroy', 'wshmpc_lp_batch',
+           'wshmpc_plant_step', 'wshmpc_closed_loop_plant')
 
 
 class _Mailbox(C.Structure):
@@ -88,6 +89,20 @@ class _Loop(C.Structure):
     _fields_ = ([(k, C.c_int) for k in ('n_steps', 'warm', 'fresh', 'par')]
                 + [(k, C.c_void_p) for k in ('d_queue', 'd_step_of', 'd_x', 'd_e', 'd_active', 'd_log_cost', 'd_log_u0',
                                              'd_log_solves', 'd_log_status', 'mailbox')])
+
+
+class _Plant(C.Structure):
+    _fields_ = [('kind', C.c_int), ('n_sets', C.c_int), ('d_params', C.c_void_p), ('dt', C.c_double), ('n_sub', C.c_int),
+                ('fc_index', C.c_int), ('d_log_x', C.c_void_p)]
+
+
+def _plant_struct(plant, log_x=None):
+    """wshmpc_plant of a plants.DevicePlant (the cart-pole between soft walls, kind 1)"""
+    c = _Plant()
+    c.kind, c.n_sets, c.d_params = 1, plant.n_sets, plant.params.data_ptr()
+    c.dt, c.n_sub, c.fc_index = plant.dt, plant.n_sub, plant.fc_index
+    c.d_log_x = log_x.data_ptr() if log_x is not None else None
+    return c
 
 
 class _Tree(C.Structure):
@@ -267,11 +282,28 @@ class Handle(object):
         _check(self.lib.wshmpc_shift_tree(self._h, old_tree.n_inst, P(x0), P(e0), C.byref(old_tree.c), P(inc_cost),
                                           P(inc_primal), P(active), C.byref(new_tree.c), P(x_next), P(u0)))
 
+    def plant_step(self, plant, x, u, out=None):
+        """wshmpc_plant_step: the states after one sample of the device plant `plant` (plants.DevicePlant) from x [n, nx]
+        under inputs u [n, nu] (CUDA fp64 tensors).  Returns out [n, nx].  Asynchronous."""
+        import torch
+        n = x.shape[0]
+        for a, w in ((x, self.pd.nx), (u, self.pd.nu)):
+            assert a.is_cuda and a.dtype == torch.float64 and tuple(a.shape) == (n, w)
+        x, u = x.contiguous(), u.contiguous()
+        if out is None:
+            out = torch.empty_like(x)
+        c = _plant_struct(plant)
+        _check(self.lib.wshmpc_plant_step(self._h, C.byref(c), n, C.c_void_p(x.data_ptr()), C.c_void_p(u.data_ptr()),
+                                          C.c_void_p(out.data_ptr())))
+        return out
+
     def closed_loop(self, n_steps, warm, fresh, par, xbuf, e, active, trees, out, tol=0., max_solves=1024, totals=None, logs=None,
-                    mailbox=None):
+                    mailbox=None, plant=None):
         """Fused closed loop (wshmpc_closed_loop): `n_steps` receding-horizon steps of every instance in one
         launch.  xbuf [2, n_inst, nx]; e [n_steps, n_inst, nx] or None; trees = (tree0, tree1).  Asynchronous.
         mailbox: a Mailbox -- the host is in the loop every step (the caller must answer it while the kernel runs).
+        plant: a plants.DevicePlant -- the nonlinear plant advances the state on the device (wshmpc_closed_loop_plant), e is
+        an additive disturbance on its output, and the logs gain 'x' [n_steps, n_inst, nx], the state after every step.
         Returns the dict of per-step logs (CUDA tensors)."""
         import torch
         dev = self.torch_device
@@ -297,9 +329,16 @@ class Handle(object):
         L.d_log_cost, L.d_log_u0, L.d_log_solves, L.d_log_status = P(logs['cost']), P(logs['u0']), P(logs['n_solves']), P(logs['status'])
         L.mailbox = C.addressof(mailbox.c) if mailbox is not None else None
         V = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
-        _check(self.lib.wshmpc_closed_loop(self._h, N, C.byref(L), C.byref(trees[0].c), C.byref(trees[1].c), C.c_double(tol),
-                                           int(max_solves), V(out['cost']), V(out['node']), V(out['primal']), V(out['n_solves']),
-                                           V(out['status']), V(totals)))
+        tail = (C.byref(trees[0].c), C.byref(trees[1].c), C.c_double(tol), int(max_solves), V(out['cost']), V(out['node']),
+                V(out['primal']), V(out['n_solves']), V(out['status']), V(totals))
+        if plant is None:
+            _check(self.lib.wshmpc_closed_loop(self._h, N, C.byref(L), *tail))
+        else:
+            if 'x' not in logs:
+                logs['x'] = torch.empty((n_steps, N, nx), dtype=torch.float64, device=dev)
+            assert logs['x'].is_contiguous() and tuple(logs['x'].shape) == (n_steps, N, nx)
+            c = _plant_struct(plant, logs['x'])
+            _check(self.lib.wshmpc_closed_loop_plant(self._h, N, C.byref(L), C.byref(c), *tail))
         return logs
 
 

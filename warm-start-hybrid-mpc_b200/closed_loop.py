@@ -20,14 +20,20 @@ def shard(n_total, rank, world):
 class ClosedLoop(object):
 
     def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
-                 mip_start=True):
+                 mip_start=True, plant=None):
         """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
         paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
         incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
-        tree holds (default 512; 2 for the comparator, whose trees hold a guess and a root)."""
+        tree holds (default 512; 2 for the comparator, whose trees hold a guess and a root).
+        plant: a plants.DevicePlant -- step() and run() advance the state through the nonlinear plant on the device instead
+        of x <- x_1|t + e: x_{t+1} = Phi(x_t, u0) + e_t (e an optional disturbance), and the warm start is corrected with
+        the measured model error x_{t+1} - x_1|t.  It has one parameter set, or one per instance."""
         import torch
         if comparator and warm:
             raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
+        if plant is not None and plant.n_sets not in (1, n_inst):
+            raise ValueError('the plant has %d parameter sets: 1, or one per instance (%d)' % (plant.n_sets, n_inst))
+        self.plant = plant
         if max_roots is None:
             max_roots = 2 if comparator else 512
         self.comparator, self.mip_start = comparator, mip_start
@@ -76,6 +82,8 @@ class ClosedLoop(object):
         """Periodic load balancing between the ranks of a torch.distributed job (rebalance.py): live instances move from
         the busiest ranks into the slots of dead instances of the idlest ones, with their warm-start trees.  Call it
         between steps / windows.  Returns (sent, received, plan)."""
+        if self.plant is not None and self.plant.n_sets > 1:
+            raise ValueError('rebalance does not move per-instance plant parameter sets with their instances')
         from .rebalance import rebalance
         return rebalance(self.trees[self.cur], self.x, self.active, self.gid, group, min_gap)
 
@@ -115,14 +123,17 @@ class ClosedLoop(object):
             h.set_node_rule(self.node_rule)
         try:
             return h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, e, self.active, self.trees, self.out,
-                                 tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mailbox)
+                                 tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mailbox,
+                                 plant=self.plant)
         finally:
             if self.node_rule:
                 h.set_node_rule(0)
 
     def step(self, e=None, x=None):
         """One receding-horizon step of every instance.  `x` (optional, [n_inst, nx] CUDA tensor)
-        overrides the state (measured state fed back from the host); `e` is the model error e_t."""
+        overrides the state (measured state fed back from the host); `e` is the model error e_t.
+        With a device plant: branch and bound (K3), the plant from the live instances' states and inputs (plus e, a
+        disturbance), the model error x_meas - x_1|t, K2 + K4, and the next state x_meas -- all on the device."""
         h = self.h
         if x is not None:
             self.x.copy_(x)
@@ -138,8 +149,13 @@ class ClosedLoop(object):
             ev[1].record()
         # K2 + K4 (in cold mode only its plant update matters: the next step re-initialises the root)
         new = self.trees[1 - self.cur]
+        x_meas = None
+        if self.plant is not None:
+            x_meas, e = self._device_plant(e)
         h.shift_tree(self.x, e, tree, self.out['cost'], self.out['primal'], new, active=self.active,
                      x_next=self.xbuf[1 - self.xpar], u0=self.u0)
+        if x_meas is not None:
+            self.xbuf[1 - self.xpar].copy_(x_meas)
         self.cur = 1 - self.cur
         self.launches += 1
         if self.events is not None:
@@ -147,6 +163,19 @@ class ClosedLoop(object):
             self.events.append(tuple(ev))
         self.xpar = 1 - self.xpar
         return self.out
+
+    def _device_plant(self, d):
+        """(x_meas, e) of step(): x_meas = Phi(x, u0) + d where the step has an incumbent, else x; e = x_meas - x_1|t there,
+        else 0 (what the fused loop computes in the lane)"""
+        import torch
+        nx, nu, T = self.ctl.mld.nx, self.ctl.mld.nu, self.ctl.T
+        prim = self.out['primal']
+        live = ((self.active != 0) & torch.isfinite(self.out['cost']))[:, None]
+        x_meas = self.plant.step(self.h, self.x, prim[:, (T + 1) * nx:(T + 1) * nx + nu])
+        if d is not None:
+            x_meas = x_meas + d
+        x_meas = torch.where(live, x_meas, self.x)
+        return x_meas, torch.where(live, x_meas - prim[:, nx:2 * nx], torch.zeros_like(x_meas))
 
     def step_with_plant(self, plant):
         """One receding-horizon step against a TRUE plant instead of the linear model + noise: branch and bound (K3), the
@@ -186,8 +215,9 @@ class ClosedLoop(object):
     def run(self, n_steps, e=None, logs=None):
         """`n_steps` receding-horizon steps of every instance in ONE launch (wshmpc_closed_loop): the fused
         form of calling step() n_steps times, without a barrier between the steps of different instances.
-        e: [n_steps, n_inst, nx] CUDA tensor of model errors or None.  Returns per-step logs
-        (cost, u0, n_solves, status), each [n_steps, n_inst, ...]; self.x holds the final states."""
+        e: [n_steps, n_inst, nx] CUDA tensor of model errors or None (with a device plant: of disturbances on the plant's
+        output).  Returns per-step logs (cost, u0, n_solves, status), each [n_steps, n_inst, ...], and with a device plant
+        also x, the state after every step; self.x holds the final states."""
         par = self.cur
         # states and trees flip together: make the state parity equal to the tree parity
         if self.xpar != par:
@@ -212,6 +242,8 @@ class ClosedLoop(object):
         import time
         import torch
         from .capi import Mailbox
+        if self.plant is not None:
+            raise ValueError('run_mailbox: the host is the plant there; this loop has a device plant (use run or step)')
         h, N = self.h, self.n_inst
         if getattr(self, '_mailbox', None) is None:
             self._mailbox = Mailbox(h, N)

@@ -7,6 +7,7 @@
 #pragma once
 #include "qp_device.cuh"
 #include "records.cuh"
+#include "plant.cuh"
 
 struct TreeView {
     int cap_nodes, cap_recs, words;
@@ -698,12 +699,14 @@ __global__ void init_guess_kernel(int n_inst, int nb, TreeView tr, const double 
 }
 #endif
 
-template <int LANES, int RULE>
+// PLANT: the state advances through the nonlinear plant on the device (wshmpc_closed_loop_plant, `pv`) instead of the linear
+// model plus an additive error; the kernels without it carry no code of the plant and never read `pv`.
+template <int LANES, int RULE, bool PLANT>
 __device__ __forceinline__ void
 closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double *scratch, const LoopView &L, int n_slots, int n_inst,
                    const TreeView &t0, const TreeView &t1, double tol, int max_solves,
                    double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *status_out,
-                   unsigned long long *totals)
+                   unsigned long long *totals, const PlantView &pv)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_inst_[WS_MAXL];
@@ -841,7 +844,32 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                 L.log_cost[lo] = inc_cost[inst]; L.log_solves[lo] = n_solves[inst]; L.log_status[lo] = st;
             }
             WS_SYNC();
-            if (!mbx) {
+            if (PLANT && !mbx) {
+                // x_meas = Phi(x_t, u0[fc_index]) (+ d_e[t]) is the next state; e = x_meas - x_1|t corrects the warm start,
+                // handed over through pv.stage like the mailbox's answer.  Without an incumbent the state is kept.
+                if (WS_TID == 0) {
+                    const double *xi = xc + (size_t)inst * 4;
+                    double *xo = xn + (size_t)inst * 4, *ei = pv.stage + (size_t)inst * 4;
+                    if (L.active[inst] != 0 && inc_cost[inst] < INFINITY) {
+                        const double *ip = inc_primal + (size_t)inst * P.n_primal;
+                        double x[4] = {xi[0], xi[1], xi[2], xi[3]};
+                        cartpole_walls_step(pv.prm + (pv.n_sets == 1 ? 0 : (size_t)inst * WS_PLANT_NPARAM), x,
+                                            ip[(size_t)(P.T + 1) * P.nx + pv.fc_index], pv.h, pv.n_sub);
+                        const double *de = L.e ? L.e + (size_t)t * xs + (size_t)inst * 4 : nullptr;
+                        for (int j = 0; j < 4; ++j) {
+                            const double xm = de ? __dadd_rn(x[j], de[j]) : x[j];
+                            xo[j] = xm; ei[j] = __dsub_rn(xm, ip[4 + j]);
+                        }
+                    } else {
+                        for (int j = 0; j < 4; ++j) { xo[j] = xi[j]; ei[j] = 0.; }
+                    }
+                    if (pv.log_x) for (int j = 0; j < 4; ++j) pv.log_x[(size_t)t * xs + (size_t)inst * 4 + j] = xo[j];
+                }
+                const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, pv.stage,
+                                                      cur, inc_cost, inc_primal, L.active, nxt, nullptr, L.log_u0 + (size_t)t * n_inst * P.nu);
+                if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
+                prof_mark(19);
+            } else if (!mbx) {
                 const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, L.e ? L.e + (size_t)t * xs : nullptr,
                                                       cur, inc_cost, inc_primal, L.active, nxt, xn, L.log_u0 + (size_t)t * n_inst * P.nu);
                 if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
@@ -877,26 +905,64 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
     n_solves, status_out, totals
 __global__ void __launch_bounds__(WS_NT, 1) closed_loop_kernel_1(WS_LOOP_ARGS)
 #if WS_TU_HAS(5)
-{ closed_loop_body<1, 0>(WS_LOOP_PASS); }
+{ closed_loop_body<1, 0, false>(WS_LOOP_PASS, PlantView()); }
 #else
 ;
 #endif
 __global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_kernel_m(WS_LOOP_ARGS)
 #if WS_TU_HAS(6)
-{ closed_loop_body<WS_MAXL, 0>(WS_LOOP_PASS); }
+{ closed_loop_body<WS_MAXL, 0, false>(WS_LOOP_PASS, PlantView()); }
 #else
 ;
 #endif
 // the fused loop of the conventional MIQP comparator (node rule 1 or 2; cold trees only)
 __global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_kernel_1(WS_LOOP_ARGS)
 #if WS_TU_HAS(9)
-{ closed_loop_body<1, BNB_RULE_MIQP>(WS_LOOP_PASS); }
+{ closed_loop_body<1, BNB_RULE_MIQP, false>(WS_LOOP_PASS, PlantView()); }
 #else
 ;
 #endif
 __global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_kernel_m(WS_LOOP_ARGS)
 #if WS_TU_HAS(10)
-{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP>(WS_LOOP_PASS); }
+{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP, false>(WS_LOOP_PASS, PlantView()); }
 #else
 ;
+#endif
+// the fused loop against the nonlinear plant (wshmpc_closed_loop_plant): node rule 0 (warm or cold) and the comparator
+__global__ void __launch_bounds__(WS_NT, 1) closed_loop_plant_kernel_1(WS_LOOP_ARGS, PlantView pv)
+#if WS_TU_HAS(11)
+{ closed_loop_body<1, 0, true>(WS_LOOP_PASS, pv); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_plant_kernel_m(WS_LOOP_ARGS, PlantView pv)
+#if WS_TU_HAS(12)
+{ closed_loop_body<WS_MAXL, 0, true>(WS_LOOP_PASS, pv); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_plant_kernel_1(WS_LOOP_ARGS, PlantView pv)
+#if WS_TU_HAS(13)
+{ closed_loop_body<1, BNB_RULE_MIQP, true>(WS_LOOP_PASS, pv); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_plant_kernel_m(WS_LOOP_ARGS, PlantView pv)
+#if WS_TU_HAS(14)
+{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP, true>(WS_LOOP_PASS, pv); }
+#else
+;
+#endif
+
+#if WS_TU_HAS(0)
+// wshmpc_plant_step: one thread per state, x_out[i] = Phi(x[i], u[i][fc_index]; parameter set i or 0)
+__global__ void plant_step_kernel(PlantView pv, int n, int nu, const double *__restrict__ x, const double *__restrict__ u,
+                                  double *__restrict__ x_out)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double xi[4] = {x[(size_t)i * 4], x[(size_t)i * 4 + 1], x[(size_t)i * 4 + 2], x[(size_t)i * 4 + 3]};
+    cartpole_walls_step(pv.prm + (pv.n_sets == 1 ? 0 : (size_t)i * WS_PLANT_NPARAM), xi, u[(size_t)i * nu + pv.fc_index], pv.h, pv.n_sub);
+    for (int j = 0; j < 4; ++j) x_out[(size_t)i * 4 + j] = xi[j];
+}
 #endif

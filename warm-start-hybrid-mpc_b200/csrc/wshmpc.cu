@@ -35,6 +35,7 @@ struct wshmpc_handle {
     size_t shift_smem; int shift_stage;      // dynamic shared memory of shift_tree_kernel, of which staging buffers (doubles)
     size_t smem;
     wshmpc_layout layout;
+    double *plant_stage; int plant_stage_n;              // wshmpc_closed_loop_plant: [n][nx] model errors (allocated on first use)
 };
 
 extern "C" const char *wshmpc_last_error(void) { return g_err.c_str(); }
@@ -309,6 +310,10 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     WS_CUDA(cudaFuncSetAttribute(bnb_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * bnb_scratch_doubles(p->nb, L.primal) * sizeof(double))); h->allocs.push_back(d); h->scratch = (double *)d;
     WS_CUDA(cudaMalloc(&d, 64)); h->allocs.push_back(d); h->work_counter = (int *)d;
     h->shift_smem = shift_smem_bytes(P, optin, &h->shift_stage);
@@ -341,6 +346,7 @@ extern "C" int wshmpc_destroy(wshmpc_handle *h)
     if (!h) return 0;
     cudaSetDevice(h->device);
     for (void *p : h->allocs) cudaFree(p);
+    if (h->plant_stage) cudaFree(h->plant_stage);
     delete h;
     return 0;
 }
@@ -494,10 +500,38 @@ extern "C" int wshmpc_shift_tree(wshmpc_handle *h, int n_inst, const double *d_x
     return 0;
 }
 
-extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop,
-                                  const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
-                                  double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
-                                  int *d_status, unsigned long long *d_totals)
+// a wshmpc_plant checked against the handle's problem; n = the states it is applied to
+static int plant_view(const wshmpc_handle *h, const wshmpc_plant *pl, int n, PlantView *v)
+{
+    if (!pl) WS_FAIL(-1, "null plant");
+    if (pl->kind != 1) WS_FAIL(-1, "plant kind %d: 1 is the cart-pole between two soft walls, the only kind", pl->kind);
+    if (h->P.nx != 4) WS_FAIL(-1, "the cart-pole plant has 4 states, the problem has nx = %d", h->P.nx);
+    if (pl->fc_index < 0 || pl->fc_index >= h->P.nu) WS_FAIL(-1, "plant fc_index = %d out of range (nu = %d)", pl->fc_index, h->P.nu);
+    if (!(pl->dt > 0.) || pl->n_sub <= 0) WS_FAIL(-1, "plant needs dt > 0 and n_sub > 0 (dt = %g, n_sub = %d)", pl->dt, pl->n_sub);
+    if (pl->n_sets != 1 && pl->n_sets != n) WS_FAIL(-1, "plant n_sets = %d: 1 or one per instance (%d)", pl->n_sets, n);
+    if (!pl->d_params) WS_FAIL(-1, "null plant parameters");
+    v->prm = pl->d_params; v->n_sets = pl->n_sets; v->n_sub = pl->n_sub; v->h = pl->dt / pl->n_sub; v->fc_index = pl->fc_index;
+    v->log_x = pl->d_log_x; v->stage = nullptr;
+    return 0;
+}
+
+extern "C" int wshmpc_plant_step(wshmpc_handle *h, const wshmpc_plant *pl, int n, const double *d_x, const double *d_u, double *d_x_out)
+{
+    if (!h) WS_FAIL(-1, "null handle");
+    if (n <= 0) return 0;
+    if (!d_x || !d_u || !d_x_out) WS_FAIL(-1, "null argument");
+    PlantView v; int rc = plant_view(h, pl, n, &v); if (rc) return rc;
+    WS_CUDA(cudaSetDevice(h->device));
+    plant_step_kernel<<<(n + 127) / 128, 128, 0, h->stream>>>(v, n, h->P.nu, d_x, d_u, d_x_out);
+    WS_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// wshmpc_closed_loop (plant = null: x <- x_1|t + e_t) and wshmpc_closed_loop_plant
+static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                              const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
+                              double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                              int *d_status, unsigned long long *d_totals)
 {
     if (!h || !loop) WS_FAIL(-1, "null argument");
     if (n_inst <= 0 || loop->n_steps <= 0) return 0;
@@ -513,6 +547,19 @@ extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loo
     TreeView v0, v1; int rc = tree_view(h, tree0, &v0); if (rc) return rc;
     rc = tree_view(h, tree1, &v1); if (rc) return rc;
     if (v0.rec_dual == v1.rec_dual || v0.lb == v1.lb) WS_FAIL(-1, "the two trees must be distinct buffers");
+    PlantView pv;
+    memset(&pv, 0, sizeof(pv));
+    if (plant) {
+        if (loop->mailbox) WS_FAIL(-1, "a plant and a mailbox: with a mailbox the host is the plant");
+        rc = plant_view(h, plant, n_inst, &pv); if (rc) return rc;
+        WS_CUDA(cudaSetDevice(h->device));
+        if (h->plant_stage_n < n_inst) {
+            if (h->plant_stage) { WS_CUDA(cudaFree(h->plant_stage)); h->plant_stage = nullptr; h->plant_stage_n = 0; }
+            WS_CUDA(cudaMalloc((void **)&h->plant_stage, (size_t)n_inst * 4 * sizeof(double)));
+            h->plant_stage_n = n_inst;
+        }
+        pv.stage = h->plant_stage;
+    }
     LoopView L;
     L.n_steps = loop->n_steps; L.warm = loop->warm; L.fresh = loop->fresh; L.par = loop->par & 1;
     L.q = loop->d_queue; L.step_of = loop->d_step_of; L.x = loop->d_x; L.e = loop->d_e; L.active = loop->d_active;
@@ -538,19 +585,42 @@ extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loo
     loop_init_kernel<<<(n_items + 255) / 256, 256, 0, h->stream>>>(n_inst, n_items, L);
     WS_CUDA(cudaGetLastError());
     const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
-    const bool miqp = h->P.node_rule != 0;
-    auto *k1 = miqp ? closed_loop_miqp_kernel_1 : closed_loop_kernel_1;
-    auto *km = miqp ? closed_loop_miqp_kernel_m : closed_loop_kernel_m;
-    if (slots <= h->n_sm || h->P.lanes == 1)
-        k1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
-            h->P1, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
+    const bool miqp = h->P.node_rule != 0, one = slots <= h->n_sm || h->P.lanes == 1;
+    const DevProblem &P = one ? h->P1 : h->P;
+    const dim3 grid(one ? slots : (slots + h->P.lanes - 1) / h->P.lanes), block(one ? WS_NT : h->P.lanes * WS_NT);
+    if (plant) {
+        auto *k = one ? (miqp ? closed_loop_miqp_plant_kernel_1 : closed_loop_plant_kernel_1)
+                      : (miqp ? closed_loop_miqp_plant_kernel_m : closed_loop_plant_kernel_m);
+        k<<<grid, block, P.so.total_bytes, h->stream>>>(
+            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
+            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, pv);
+    } else {
+        auto *k = one ? (miqp ? closed_loop_miqp_kernel_1 : closed_loop_kernel_1) : (miqp ? closed_loop_miqp_kernel_m : closed_loop_kernel_m);
+        k<<<grid, block, P.so.total_bytes, h->stream>>>(
+            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
             d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals);
-    else
-    km<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
-        h->P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
-        d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals);
+    }
     WS_CUDA(cudaGetLastError());
     return 0;
+}
+
+extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop,
+                                  const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
+                                  double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                                  int *d_status, unsigned long long *d_totals)
+{
+    return closed_loop_launch(h, n_inst, loop, nullptr, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
+                              d_n_solves, d_status, d_totals);
+}
+
+extern "C" int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                                        const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
+                                        double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                                        int *d_status, unsigned long long *d_totals)
+{
+    if (!plant) WS_FAIL(-1, "null plant");
+    return closed_loop_launch(h, n_inst, loop, plant, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
+                              d_n_solves, d_status, d_totals);
 }
 
 // host mailbox: pinned, mapped host memory the running kernel and the host both see

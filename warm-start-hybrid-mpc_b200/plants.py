@@ -15,10 +15,19 @@ when it pushes:  f = max(0, -stiffness * gap -/+ damping * tip velocity)  if gap
 import numpy as np
 
 
+def n_substeps(dt, h_des):
+    """Euler sub-steps per sample of CartPoleWithWalls.simulate"""
+    return max(1, int(round(dt / h_des)))
+
+
 class CartPoleWithWalls(object):
 
     def __init__(self, mc=1., mp=1., l=1., d=.5, stiffness=100., damping=10., g=10.):
         self.mc, self.mp, self.l, self.d, self.k, self.c, self.g = mc, mp, l, d, stiffness, damping, g
+
+    def params(self):
+        """(mc, mp, l, d, stiffness, damping, g): the parameter set of the device plant (WSHMPC_PLANT_CARTPOLE_NPARAM)"""
+        return np.array([self.mc, self.mp, self.l, self.d, self.k, self.c, self.g], dtype=float)
 
     def gaps(self, x):
         """distance of the pole tip from the left / right wall (negative in penetration)"""
@@ -51,7 +60,7 @@ class CartPoleWithWalls(object):
     def simulate(self, x, dt, fc=0., h_des=.001):
         """explicit Euler with sub-steps of about h_des (nonlinear_dynamics.py:112-118); returns the state after dt.
         x [..., 4], fc [...] (held constant over dt)."""
-        n = max(1, int(round(dt / h_des)))
+        n = n_substeps(dt, h_des)
         h = dt / n
         x = np.array(x, dtype=float)
         fc = np.asarray(fc, dtype=float)
@@ -68,3 +77,34 @@ class CartPoleWithWalls(object):
         B = np.zeros((4, 3))
         B[2:, 0] = Minv.dot([1., 0.]); B[2:, 1] = Minv.dot([1., -l]); B[2:, 2] = Minv.dot([-1., l])
         return A, B
+
+
+class DevicePlant(object):
+    """The cart-pole between soft walls integrated on the device (wshmpc_plant in include/wshmpc.h): what
+    CartPoleWithWalls.simulate(x, dt, u[:, fc_index], h_des) computes, for a batch of states, in the closed loop
+    (ClosedLoop(..., plant=DevicePlant(...))) or standalone (step).
+
+    plants: one CartPoleWithWalls for every instance, or a list of them, one per instance (a robustness sweep over
+    plant parameters).  The Euler sub-step count follows simulate: n_sub = max(1, round(dt / h_des))."""
+
+    def __init__(self, plants, dt, h_des=1e-3, fc_index=0, device='cuda'):
+        import torch
+        ps = [plants] if isinstance(plants, CartPoleWithWalls) else list(plants)
+        if not ps or not all(isinstance(p, CartPoleWithWalls) for p in ps):
+            raise ValueError('plants: a CartPoleWithWalls or a non-empty list of them')
+        if not dt > 0. or not h_des > 0.:
+            raise ValueError('dt and h_des must be positive (dt = %r, h_des = %r)' % (dt, h_des))
+        if int(fc_index) != fc_index or fc_index < 0:
+            raise ValueError('fc_index must be a non-negative input index, got %r' % (fc_index,))
+        self.dt, self.fc_index = float(dt), int(fc_index)
+        self.n_sub = n_substeps(dt, h_des)
+        self.params = torch.as_tensor(np.stack([p.params() for p in ps]), dtype=torch.float64, device=device).contiguous()
+
+    @property
+    def n_sets(self):
+        return self.params.shape[0]
+
+    def step(self, handle, x, u):
+        """States after dt from x [n, 4] under inputs u [n, nu] (CUDA fp64 tensors); parameter set k for state k when
+        there is one set per state (wshmpc_plant_step).  Asynchronous on the handle's stream."""
+        return handle.plant_step(self, x, u)
