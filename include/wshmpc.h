@@ -217,7 +217,8 @@ int wshmpc_shift_tree(wshmpc_handle *h, int n_inst, const double *d_x0, const do
  * global memory feeds the CTAs).  Replaces the experiment loop of
  * notebooks/cart_pole_with_walls/statistical_analysis.py:93-196 (cold or warm-started feedforward,
  * construct_warm_start, x <- x_1|t + e_t on the linear plant) for the whole batch; results are identical to
- * calling wshmpc_bnb_solve + wshmpc_shift_tree once per step.
+ * calling wshmpc_bnb_solve + wshmpc_shift_tree once per step.  An instance without an incumbent leaves the loop, unless a
+ * fallback is configured (wshmpc_closed_loop_fallback).
  */
 /* Host mailbox of the fused closed loop: the host is in the loop EVERY receding-horizon step of every instance (a true
  * plant, measured states) and there is still no barrier between instances -- what a per-step call of
@@ -295,13 +296,57 @@ int wshmpc_plant_step(wshmpc_handle *h, const wshmpc_plant *pl, int n, const dou
 /* wshmpc_closed_loop against the nonlinear plant, advanced on the device.  For every step t of a live instance i with an
  * incumbent:  u0 = the incumbent's first input,  x_meas = Phi(x_t, u0[fc_index]; set i) + d_e[t][i] (loop->d_e optional:
  * an additive disturbance on the plant output),  the warm start is corrected with e = x_meas - x_1|t (construct_warm_start's
- * e0), and x_{t+1} = x_meas.  An instance without an incumbent keeps its state and is switched off.  Results equal calling
+ * e0), and x_{t+1} = x_meas.  An instance without an incumbent keeps its state and is switched off, unless a fallback is
+ * configured (wshmpc_closed_loop_fallback).  Results equal calling
  * wshmpc_bnb_solve, wshmpc_plant_step and wshmpc_shift_tree (with e0 = e) once per step.  A mailbox is an error (the host is
  * the plant there). */
 int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
                              const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
                              double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
                              int *d_status, unsigned long long *d_totals);
+
+/* Fallback through infeasible MIQPs: an instance whose step has no incumbent applies the next input of its last plan and
+ * solves again at the next sample, instead of leaving the loop.  The plan is the primal record of the last step with an
+ * incumbent and `age` counts the steps since then (-1: no plan).  At step t of a live instance, after its branch and bound:
+ *   incumbent                                 plan <- incumbent, age <- 0; the applied pair is the incumbent;       hold 0
+ *   status 1 (infeasible), age + 1 <= max_hold  age <- age + 1; applied u_0 = u_age of the plan,
+ *                                             x_1|t = A x_t + B u_0; the instance stays live;                      hold age
+ *   otherwise (no plan, plan used up, status 2 or 3, instance off)   the instance is switched off as without a fallback; hold -1
+ * A status-1 step ran its search to the end: its leaves are a complete cover (Farkas proofs and bounds) and K2 + K4 shift them
+ * with the applied input like a solved tree.  The logs of a fallback step keep cost +inf and status 1; u0 is the applied
+ * input.  All buffers are device memory owned by the caller, so plans survive launches.
+ *   d_plan       [n_inst][layout.primal]
+ *   d_age        [n_inst] in/out (fill with -1 to start without plans)
+ *   d_app_cost   [n_inst] applied pair, what K2 + K4 and the plant read in place of the incumbent: the incumbent's cost, 0 on a
+ *                fallback step, +inf where the instance leaves the loop
+ *   d_app_primal [n_inst][layout.primal] the incumbent's record; on a fallback step only x_0, x_1 and u_0 are defined.
+ *                Must not overlap d_plan.
+ *   d_hold       [n_steps][n_inst] (wshmpc_closed_loop_fallback) or [n_inst] (wshmpc_fallback_step): 0 the incumbent,
+ *                a > 0 input u_a of the plan, -1 the instance left the loop (or was off)
+ * max_hold = 0 is the behaviour without a fallback, bit for bit. */
+typedef struct {
+    int max_hold;          /* H, 0 <= H <= T - 1 */
+    double *d_plan;
+    int *d_age;
+    double *d_app_cost;
+    double *d_app_primal;
+    int *d_hold;
+} wshmpc_fallback;
+
+/* wshmpc_closed_loop (plant = NULL: the linear plant x <- x_1|t + e_t) or wshmpc_closed_loop_plant under the fallback policy:
+ * the plant and the warm start of every step use the applied pair.  Fails under node rules 1 and 2 (the comparator), with a
+ * mailbox, for max_hold outside 0 .. T - 1, null buffers, or d_plan overlapping d_app_primal. */
+int wshmpc_closed_loop_fallback(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                                const wshmpc_fallback *fb, const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol,
+                                int max_solves, double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                                int *d_status, unsigned long long *d_totals);
+
+/* Lock-step form of the policy, between wshmpc_bnb_solve and wshmpc_shift_tree / wshmpc_plant_step (one thread per instance,
+ * asynchronous): writes d_app_cost, d_app_primal, d_age, d_plan and d_hold [n_inst] from the step's d_status / d_inc_cost /
+ * d_inc_primal at states d_x; d_active (NULL: every instance) marks the live instances.  The caller then passes d_app_cost and
+ * d_app_primal to wshmpc_shift_tree as the incumbent (and u_0 of d_app_primal to the plant).  Same failures as above. */
+int wshmpc_fallback_step(wshmpc_handle *h, int n_inst, const wshmpc_fallback *fb, const double *d_x, const int *d_active,
+                         const int *d_status, const double *d_inc_cost, const double *d_inc_primal);
 
 /* Batched small LPs in standard form (SURVEY.md 8f-2):   min c'y  s.t.  E y = r,  y >= 0   for n_lp problems at once,
  * one CTA per LP (two-phase tableau simplex in shared memory).  Replaces the host LP loops the reference runs through

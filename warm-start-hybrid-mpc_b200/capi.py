@@ -44,7 +44,7 @@ def load_library():
 
 EXPORTS = ('wshmpc_last_error', 'wshmpc_ctas_per_sm', 'wshmpc_set_search_rule', 'wshmpc_set_branch_order', 'wshmpc_set_node_rule', 'wshmpc_create', 'wshmpc_destroy', 'wshmpc_get_layout', 'wshmpc_solve_nodes',
            'wshmpc_tree_init_root', 'wshmpc_tree_init_guess', 'wshmpc_bnb_solve', 'wshmpc_shift_tree', 'wshmpc_closed_loop', 'wshmpc_mailbox_create', 'wshmpc_mailbox_destroy', 'wshmpc_lp_batch',
-           'wshmpc_plant_step', 'wshmpc_closed_loop_plant')
+           'wshmpc_plant_step', 'wshmpc_closed_loop_plant', 'wshmpc_closed_loop_fallback', 'wshmpc_fallback_step')
 
 
 class _Mailbox(C.Structure):
@@ -102,6 +102,21 @@ def _plant_struct(plant, log_x=None):
     c.kind, c.n_sets, c.d_params = 1, plant.n_sets, plant.params.data_ptr()
     c.dt, c.n_sub, c.fc_index = plant.dt, plant.n_sub, plant.fc_index
     c.d_log_x = log_x.data_ptr() if log_x is not None else None
+    return c
+
+
+class _Fallback(C.Structure):
+    _fields_ = [('max_hold', C.c_int), ('d_plan', C.c_void_p), ('d_age', C.c_void_p), ('d_app_cost', C.c_void_p),
+                ('d_app_primal', C.c_void_p), ('d_hold', C.c_void_p)]
+
+
+def _fallback_struct(fb, hold):
+    """wshmpc_fallback of a dict(max_hold, plan, age, app_cost, app_primal) of CUDA tensors, with the hold log `hold`"""
+    c = _Fallback()
+    c.max_hold = int(fb['max_hold'])
+    for k in ('plan', 'age', 'app_cost', 'app_primal'):
+        setattr(c, 'd_' + k, fb[k].data_ptr() if fb[k] is not None else None)
+    c.d_hold = hold.data_ptr() if hold is not None else None
     return c
 
 
@@ -297,13 +312,35 @@ class Handle(object):
                                           C.c_void_p(out.data_ptr())))
         return out
 
+    def new_fallback(self, n_inst, max_hold):
+        """Caller-owned buffers of the fallback policy (wshmpc_fallback) for n_inst instances, without plans (age -1):
+        dict(max_hold, plan, age, app_cost, app_primal, hold [n_inst]) of CUDA tensors."""
+        import torch
+        f64 = dict(dtype=torch.float64, device=self.torch_device)
+        i32 = dict(dtype=torch.int32, device=self.torch_device)
+        P = self.layout.primal
+        return dict(max_hold=int(max_hold), plan=torch.zeros((n_inst, P), **f64), age=torch.full((n_inst,), -1, **i32),
+                    app_cost=torch.zeros(n_inst, **f64), app_primal=torch.zeros((n_inst, P), **f64),
+                    hold=torch.zeros(n_inst, **i32))
+
+    def fallback_step(self, fb, x, active, out):
+        """wshmpc_fallback_step: the fallback policy after a lock-step branch and bound (`out` of bnb_solve) at states
+        x [n_inst, nx]; writes fb['app_cost'], fb['app_primal'], fb['age'], fb['plan'] and fb['hold'].  Asynchronous."""
+        N = x.shape[0]
+        c = _fallback_struct(fb, fb['hold'])
+        V = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
+        _check(self.lib.wshmpc_fallback_step(self._h, N, C.byref(c), V(x), V(active), V(out['status']), V(out['cost']),
+                                             V(out['primal'])))
+
     def closed_loop(self, n_steps, warm, fresh, par, xbuf, e, active, trees, out, tol=0., max_solves=1024, totals=None, logs=None,
-                    mailbox=None, plant=None):
+                    mailbox=None, plant=None, fallback=None):
         """Fused closed loop (wshmpc_closed_loop): `n_steps` receding-horizon steps of every instance in one
         launch.  xbuf [2, n_inst, nx]; e [n_steps, n_inst, nx] or None; trees = (tree0, tree1).  Asynchronous.
         mailbox: a Mailbox -- the host is in the loop every step (the caller must answer it while the kernel runs).
         plant: a plants.DevicePlant -- the nonlinear plant advances the state on the device (wshmpc_closed_loop_plant), e is
         an additive disturbance on its output, and the logs gain 'x' [n_steps, n_inst, nx], the state after every step.
+        fallback: buffers of new_fallback -- the loop runs under the fallback policy (wshmpc_closed_loop_fallback, also with
+        max_hold = 0) and the logs gain 'hold' [n_steps, n_inst].
         Returns the dict of per-step logs (CUDA tensors)."""
         import torch
         dev = self.torch_device
@@ -331,13 +368,22 @@ class Handle(object):
         V = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
         tail = (C.byref(trees[0].c), C.byref(trees[1].c), C.c_double(tol), int(max_solves), V(out['cost']), V(out['node']),
                 V(out['primal']), V(out['n_solves']), V(out['status']), V(totals))
-        if plant is None:
-            _check(self.lib.wshmpc_closed_loop(self._h, N, C.byref(L), *tail))
-        else:
+        c = None
+        if plant is not None:
             if 'x' not in logs:
                 logs['x'] = torch.empty((n_steps, N, nx), dtype=torch.float64, device=dev)
             assert logs['x'].is_contiguous() and tuple(logs['x'].shape) == (n_steps, N, nx)
             c = _plant_struct(plant, logs['x'])
+        if fallback is not None:
+            if 'hold' not in logs:
+                logs['hold'] = torch.empty((n_steps, N), dtype=torch.int32, device=dev)
+            assert logs['hold'].is_contiguous() and tuple(logs['hold'].shape) == (n_steps, N)
+            f = _fallback_struct(fallback, logs['hold'])
+            _check(self.lib.wshmpc_closed_loop_fallback(self._h, N, C.byref(L), C.byref(c) if c is not None else None,
+                                                        C.byref(f), *tail))
+        elif plant is None:
+            _check(self.lib.wshmpc_closed_loop(self._h, N, C.byref(L), *tail))
+        else:
             _check(self.lib.wshmpc_closed_loop_plant(self._h, N, C.byref(L), C.byref(c), *tail))
         return logs
 

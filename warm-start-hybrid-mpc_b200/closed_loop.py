@@ -20,19 +20,27 @@ def shard(n_total, rank, world):
 class ClosedLoop(object):
 
     def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
-                 mip_start=True, plant=None):
+                 mip_start=True, plant=None, fallback=0):
         """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
         paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
         incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
         tree holds (default 512; 2 for the comparator, whose trees hold a guess and a root).
         plant: a plants.DevicePlant -- step() and run() advance the state through the nonlinear plant on the device instead
         of x <- x_1|t + e: x_{t+1} = Phi(x_t, u0) + e_t (e an optional disturbance), and the warm start is corrected with
-        the measured model error x_{t+1} - x_1|t.  It has one parameter set, or one per instance."""
+        the measured model error x_{t+1} - x_1|t.  It has one parameter set, or one per instance.
+        fallback: H, 0 <= H <= T - 1.  With H > 0 an instance whose MIQP is infeasible applies the next input of its last plan
+        for up to H steps in a row instead of leaving the loop, and the shifted tree of the infeasible step warm-starts the
+        next one (wshmpc_fallback in include/wshmpc.h); out['hold'] and the logs' 'hold' say where each applied input came
+        from (0 the incumbent, a > 0 input u_a of the plan, -1 none).  Not with the comparator."""
         import torch
         if comparator and warm:
             raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
         if plant is not None and plant.n_sets not in (1, n_inst):
             raise ValueError('the plant has %d parameter sets: 1, or one per instance (%d)' % (plant.n_sets, n_inst))
+        if int(fallback) != fallback or not 0 <= fallback <= controller.T - 1:
+            raise ValueError('fallback = %r: the steps an instance may hold its plan, 0 .. T - 1 = %d' % (fallback, controller.T - 1))
+        if fallback and comparator:
+            raise ValueError('the fallback policy runs under the structured search only, not with the MIQP comparator')
         self.plant = plant
         if max_roots is None:
             max_roots = 2 if comparator else 512
@@ -61,6 +69,9 @@ class ClosedLoop(object):
         self.fresh = True
         self.launches = 0
         self.events = None          # list -> (start, after K3, after K2+K4) CUDA events of every step
+        self.fb = h.new_fallback(n_inst, fallback) if fallback else None     # plans, ages, applied pairs (wshmpc_fallback)
+        if self.fb is not None:
+            self.out['hold'] = self.fb['hold']
 
     @property
     def x(self):
@@ -75,6 +86,8 @@ class ClosedLoop(object):
         import torch
         self.x.copy_(torch.as_tensor(np.asarray(x0, dtype=float) if not torch.is_tensor(x0) else x0))
         self.active.fill_(1)
+        if self.fb is not None:
+            self.fb['age'].fill_(-1)
         self.totals.zero_()
         self.fresh = True
 
@@ -84,6 +97,8 @@ class ClosedLoop(object):
         between steps / windows.  Returns (sent, received, plan)."""
         if self.plant is not None and self.plant.n_sets > 1:
             raise ValueError('rebalance does not move per-instance plant parameter sets with their instances')
+        if self.fb is not None:
+            raise ValueError('rebalance does not move the fallback plans with their instances')
         from .rebalance import rebalance
         return rebalance(self.trees[self.cur], self.x, self.active, self.gid, group, min_gap)
 
@@ -124,16 +139,25 @@ class ClosedLoop(object):
         try:
             return h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, e, self.active, self.trees, self.out,
                                  tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mailbox,
-                                 plant=self.plant)
+                                 plant=self.plant, fallback=self.fb)
         finally:
             if self.node_rule:
                 h.set_node_rule(0)
+
+    def _applied(self):
+        """(cost, primal) of the pair the plant and K2 + K4 apply: the incumbent, or with a fallback the policy's choice
+        (wshmpc_fallback_step, run right after the branch and bound)"""
+        if self.fb is None:
+            return self.out['cost'], self.out['primal']
+        self.h.fallback_step(self.fb, self.x, self.active, self.out)
+        return self.fb['app_cost'], self.fb['app_primal']
 
     def step(self, e=None, x=None):
         """One receding-horizon step of every instance.  `x` (optional, [n_inst, nx] CUDA tensor)
         overrides the state (measured state fed back from the host); `e` is the model error e_t.
         With a device plant: branch and bound (K3), the plant from the live instances' states and inputs (plus e, a
-        disturbance), the model error x_meas - x_1|t, K2 + K4, and the next state x_meas -- all on the device."""
+        disturbance), the model error x_meas - x_1|t, K2 + K4, and the next state x_meas -- all on the device.
+        With a fallback, the plant and K2 + K4 apply the policy's input (out['hold'])."""
         h = self.h
         if x is not None:
             self.x.copy_(x)
@@ -147,12 +171,13 @@ class ClosedLoop(object):
         self._bnb(tree)
         if self.events is not None:
             ev[1].record()
+        cost, prim = self._applied()
         # K2 + K4 (in cold mode only its plant update matters: the next step re-initialises the root)
         new = self.trees[1 - self.cur]
         x_meas = None
         if self.plant is not None:
-            x_meas, e = self._device_plant(e)
-        h.shift_tree(self.x, e, tree, self.out['cost'], self.out['primal'], new, active=self.active,
+            x_meas, e = self._device_plant(e, cost, prim)
+        h.shift_tree(self.x, e, tree, cost, prim, new, active=self.active,
                      x_next=self.xbuf[1 - self.xpar], u0=self.u0)
         if x_meas is not None:
             self.xbuf[1 - self.xpar].copy_(x_meas)
@@ -164,13 +189,12 @@ class ClosedLoop(object):
         self.xpar = 1 - self.xpar
         return self.out
 
-    def _device_plant(self, d):
-        """(x_meas, e) of step(): x_meas = Phi(x, u0) + d where the step has an incumbent, else x; e = x_meas - x_1|t there,
-        else 0 (what the fused loop computes in the lane)"""
+    def _device_plant(self, d, cost, prim):
+        """(x_meas, e) of step(): x_meas = Phi(x, u0) + d where the step has an applied pair (cost, prim), else x;
+        e = x_meas - x_1|t there, else 0 (what the fused loop computes in the lane)"""
         import torch
         nx, nu, T = self.ctl.mld.nx, self.ctl.mld.nu, self.ctl.T
-        prim = self.out['primal']
-        live = ((self.active != 0) & torch.isfinite(self.out['cost']))[:, None]
+        live = ((self.active != 0) & torch.isfinite(cost))[:, None]
         x_meas = self.plant.step(self.h, self.x, prim[:, (T + 1) * nx:(T + 1) * nx + nu])
         if d is not None:
             x_meas = x_meas + d
@@ -181,7 +205,8 @@ class ClosedLoop(object):
         """One receding-horizon step against a TRUE plant instead of the linear model + noise: branch and bound (K3), the
         applied input goes to `plant(x [n, nx], u0 [n, nu]) -> next measured state [n, nx]` (host numpy, e.g.
         plants.CartPoleWithWalls.simulate), the model error e_t = x_measured - x_1|t is what the warm start of the next
-        step is corrected with (construct_warm_start's e0, controller.py:503-564), then K2 + K4.
+        step is corrected with (construct_warm_start's e0, controller.py:503-564), then K2 + K4.  With a fallback the plant
+        gets the policy's input and x_1|t is that of the applied pair (out['hold']).
         Returns (out, u0 [n, nu] numpy, e [n, nx] numpy)."""
         import torch
         h = self.h
@@ -189,19 +214,20 @@ class ClosedLoop(object):
         if self.fresh or not self.warm:
             self._init_tree(tree)
         self._bnb(tree)
+        cost_d, prim_d = self._applied()
         nx, nu, T = self.ctl.mld.nx, self.ctl.mld.nu, self.ctl.T
-        prim = self.out['primal'].cpu().numpy()
+        prim = prim_d.cpu().numpy()
         x_now = self.x.cpu().numpy()
         u0 = prim[:, (T + 1) * nx:(T + 1) * nx + nu]
         x_pred = prim[:, nx:2 * nx]
-        live = (self.active.cpu().numpy() != 0) & np.isfinite(self.out['cost'].cpu().numpy())
+        live = (self.active.cpu().numpy() != 0) & np.isfinite(cost_d.cpu().numpy())
         x_meas = np.array(x_now)
         if live.any():
             x_meas[live] = plant(x_now[live], u0[live])
         e = np.where(live[:, None], x_meas - x_pred, 0.)
         ed = torch.as_tensor(e, device=self.x.device)
         new = self.trees[1 - self.cur]
-        h.shift_tree(self.x, ed, tree, self.out['cost'], self.out['primal'], new, active=self.active,
+        h.shift_tree(self.x, ed, tree, cost_d, prim_d, new, active=self.active,
                      x_next=self.xbuf[1 - self.xpar], u0=self.u0)
         if live.any():
             # the next step starts from the MEASURED state itself (x_1|t + (x_measured - x_1|t) is one rounding away from it)
@@ -216,8 +242,8 @@ class ClosedLoop(object):
         """`n_steps` receding-horizon steps of every instance in ONE launch (wshmpc_closed_loop): the fused
         form of calling step() n_steps times, without a barrier between the steps of different instances.
         e: [n_steps, n_inst, nx] CUDA tensor of model errors or None (with a device plant: of disturbances on the plant's
-        output).  Returns per-step logs (cost, u0, n_solves, status), each [n_steps, n_inst, ...], and with a device plant
-        also x, the state after every step; self.x holds the final states."""
+        output).  Returns per-step logs (cost, u0, n_solves, status), each [n_steps, n_inst, ...], with a device plant
+        also x, the state after every step, and with a fallback also hold; self.x holds the final states."""
         par = self.cur
         # states and trees flip together: make the state parity equal to the tree parity
         if self.xpar != par:
@@ -244,6 +270,8 @@ class ClosedLoop(object):
         from .capi import Mailbox
         if self.plant is not None:
             raise ValueError('run_mailbox: the host is the plant there; this loop has a device plant (use run or step)')
+        if self.fb is not None:
+            raise ValueError('run_mailbox has no fallback policy: use run, step or step_with_plant')
         h, N = self.h, self.n_inst
         if getattr(self, '_mailbox', None) is None:
             self._mailbox = Mailbox(h, N)

@@ -699,14 +699,73 @@ __global__ void init_guess_kernel(int n_inst, int nb, TreeView tr, const double 
 }
 #endif
 
+// Fallback through infeasible MIQPs (wshmpc_fallback): caller-owned buffers, so that plans survive launches and windows.
+struct FallbackView {
+    int max_hold;            // H: steps an instance may run on its last plan, 0 <= H <= T - 1
+    double *plan;            // [n_inst][n_primal] primal record of the last step with an incumbent
+    int *age;                // [n_inst] steps since that step, -1 = no plan
+    double *app_cost;        // [n_inst] applied pair: +inf = the instance leaves the loop, finite otherwise
+    double *app_primal;      // [n_inst][n_primal] (a fallback step defines x_0, x_1 and u_0 only)
+    int *hold;               // [n_inst] of the step: 0 the incumbent, a > 0 input u_a of the plan, -1 none
+};
+
+// The fallback policy for instance `inst` after its branch and bound (status st; the fused loop and wshmpc_fallback_step):
+//   incumbent                            plan <- incumbent, age 0, applied pair = incumbent, hold 0;
+//   status 1, a plan with age + 1 <= H   age += 1, applied u_0 = u_age of the plan, x_1 = A x + B u_0 (fused multiply-adds
+//                                        in a fixed order, so that every caller gets the same bits), hold = age;
+//   otherwise                            applied cost +inf (K2 + K4 switch the instance off), hold -1.
+// Threads tid = 0 .. nt - 1 share the copies; `sync` is the callers' barrier (age is read by all before thread 0 writes it).
+template <class Sync>
+__device__ __forceinline__ void fallback_apply(const DevProblem &P, const FallbackView &fb, int inst, bool live, int st,
+                                               const double *__restrict__ x, const double *__restrict__ inc_cost,
+                                               const double *__restrict__ inc_primal, int *hold, int tid, int nt, Sync sync)
+{
+    const int nx = P.nx, nu = P.nu, np_ = P.n_primal;
+    const size_t o = (size_t)inst * np_;
+    const int a = fb.age[inst];
+    const int mode = !live ? 2 : inc_cost[inst] < INFINITY ? 0 : (st == BNB_INFEASIBLE && a >= 0 && a + 1 <= fb.max_hold) ? 1 : 2;
+    if (mode == 0) {
+        for (int j = tid; j < np_; j += nt) { const double v = inc_primal[o + j]; fb.plan[o + j] = v; fb.app_primal[o + j] = v; }
+    } else if (mode == 1) {
+        const double *u = fb.plan + o + (size_t)(P.T + 1) * nx + (size_t)(a + 1) * nu;
+        double *ap = fb.app_primal + o;
+        for (int j = tid; j < nx; j += nt) {
+            double s = 0.;
+            for (int c = 0; c < nx; ++c) s = __fma_rn(P.A[j * nx + c], x[c], s);
+            for (int c = 0; c < nu; ++c) s = __fma_rn(P.B[j * nu + c], u[c], s);
+            ap[j] = x[j]; ap[nx + j] = s;
+        }
+        for (int j = tid; j < nu; j += nt) ap[(size_t)(P.T + 1) * nx + j] = u[j];
+    }
+    sync();
+    if (tid == 0) {
+        if (mode == 0) { fb.age[inst] = 0; fb.app_cost[inst] = inc_cost[inst]; hold[inst] = 0; }
+        else if (mode == 1) { fb.age[inst] = a + 1; fb.app_cost[inst] = 0.; hold[inst] = a + 1; }
+        else { fb.app_cost[inst] = INFINITY; hold[inst] = -1; }
+    }
+}
+
+#if WS_TU_HAS(0)
+// wshmpc_fallback_step: one thread per instance
+__global__ void fallback_step_kernel(DevProblem P, int n_inst, FallbackView fb, const double *__restrict__ x, const int *__restrict__ active,
+                                     const int *__restrict__ status, const double *__restrict__ inc_cost, const double *__restrict__ inc_primal)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_inst) return;
+    fallback_apply(P, fb, i, !active || active[i] != 0, status[i], x + (size_t)i * P.nx, inc_cost, inc_primal, fb.hold, 0, 1, [] {});
+}
+#endif
+
 // PLANT: the state advances through the nonlinear plant on the device (wshmpc_closed_loop_plant, `pv`) instead of the linear
 // model plus an additive error; the kernels without it carry no code of the plant and never read `pv`.
-template <int LANES, int RULE, bool PLANT>
+// FB: the fallback policy (wshmpc_closed_loop_fallback, `fv`): after K3 the plant and K2 + K4 read the applied pair
+// fv.app_cost / fv.app_primal instead of the incumbent; the kernels without it never read `fv`.
+template <int LANES, int RULE, bool PLANT, bool FB = false>
 __device__ __forceinline__ void
 closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double *scratch, const LoopView &L, int n_slots, int n_inst,
                    const TreeView &t0, const TreeView &t1, double tol, int max_solves,
                    double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *status_out,
-                   unsigned long long *totals, const PlantView &pv)
+                   unsigned long long *totals, const PlantView &pv, const FallbackView &fv = FallbackView())
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_inst_[WS_MAXL];
@@ -844,14 +903,22 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                 L.log_cost[lo] = inc_cost[inst]; L.log_solves[lo] = n_solves[inst]; L.log_status[lo] = st;
             }
             WS_SYNC();
+            // the pair the plant and K2 + K4 apply: the incumbent, or under FB the policy's choice
+            const double *a_cost = inc_cost, *a_primal = inc_primal;
+            if (FB) {
+                fallback_apply(P, fv, inst, L.active[inst] != 0, st, xc + (size_t)inst * P.nx, inc_cost, inc_primal,
+                               fv.hold + (size_t)t * n_inst, WS_TID, WS_NT, [] { WS_SYNC(); });
+                WS_SYNC();
+                a_cost = fv.app_cost; a_primal = fv.app_primal;
+            }
             if (PLANT && !mbx) {
                 // x_meas = Phi(x_t, u0[fc_index]) (+ d_e[t]) is the next state; e = x_meas - x_1|t corrects the warm start,
                 // handed over through pv.stage like the mailbox's answer.  Without an incumbent the state is kept.
                 if (WS_TID == 0) {
                     const double *xi = xc + (size_t)inst * 4;
                     double *xo = xn + (size_t)inst * 4, *ei = pv.stage + (size_t)inst * 4;
-                    if (L.active[inst] != 0 && inc_cost[inst] < INFINITY) {
-                        const double *ip = inc_primal + (size_t)inst * P.n_primal;
+                    if (L.active[inst] != 0 && a_cost[inst] < INFINITY) {
+                        const double *ip = a_primal + (size_t)inst * P.n_primal;
                         double x[4] = {xi[0], xi[1], xi[2], xi[3]};
                         cartpole_walls_step(pv.prm + (pv.n_sets == 1 ? 0 : (size_t)inst * WS_PLANT_NPARAM), x,
                                             ip[(size_t)(P.T + 1) * P.nx + pv.fc_index], pv.h, pv.n_sub);
@@ -866,12 +933,12 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                     if (pv.log_x) for (int j = 0; j < 4; ++j) pv.log_x[(size_t)t * xs + (size_t)inst * 4 + j] = xo[j];
                 }
                 const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, pv.stage,
-                                                      cur, inc_cost, inc_primal, L.active, nxt, nullptr, L.log_u0 + (size_t)t * n_inst * P.nu);
+                                                      cur, a_cost, a_primal, L.active, nxt, nullptr, L.log_u0 + (size_t)t * n_inst * P.nu);
                 if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
                 prof_mark(19);
             } else if (!mbx) {
                 const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, L.e ? L.e + (size_t)t * xs : nullptr,
-                                                      cur, inc_cost, inc_primal, L.active, nxt, xn, L.log_u0 + (size_t)t * n_inst * P.nu);
+                                                      cur, a_cost, a_primal, L.active, nxt, xn, L.log_u0 + (size_t)t * n_inst * P.nu);
                 if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
                 prof_mark(19);
             } else {
@@ -950,6 +1017,32 @@ __global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_plant_kernel_1(WS_L
 __global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_plant_kernel_m(WS_LOOP_ARGS, PlantView pv)
 #if WS_TU_HAS(14)
 { closed_loop_body<WS_MAXL, BNB_RULE_MIQP, true>(WS_LOOP_PASS, pv); }
+#else
+;
+#endif
+// the fused loop under the fallback policy (wshmpc_closed_loop_fallback; node rule 0, warm or cold): linear plant ...
+__global__ void __launch_bounds__(WS_NT, 1) closed_loop_fb_kernel_1(WS_LOOP_ARGS, FallbackView fv)
+#if WS_TU_HAS(15)
+{ closed_loop_body<1, 0, false, true>(WS_LOOP_PASS, PlantView(), fv); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_fb_kernel_m(WS_LOOP_ARGS, FallbackView fv)
+#if WS_TU_HAS(16)
+{ closed_loop_body<WS_MAXL, 0, false, true>(WS_LOOP_PASS, PlantView(), fv); }
+#else
+;
+#endif
+// ... and the nonlinear plant on the device
+__global__ void __launch_bounds__(WS_NT, 1) closed_loop_plant_fb_kernel_1(WS_LOOP_ARGS, PlantView pv, FallbackView fv)
+#if WS_TU_HAS(17)
+{ closed_loop_body<1, 0, true, true>(WS_LOOP_PASS, pv, fv); }
+#else
+;
+#endif
+__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_plant_fb_kernel_m(WS_LOOP_ARGS, PlantView pv, FallbackView fv)
+#if WS_TU_HAS(18)
+{ closed_loop_body<WS_MAXL, 0, true, true>(WS_LOOP_PASS, pv, fv); }
 #else
 ;
 #endif

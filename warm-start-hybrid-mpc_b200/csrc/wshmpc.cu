@@ -314,6 +314,10 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_fb_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_fb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_fb_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_fb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * bnb_scratch_doubles(p->nb, L.primal) * sizeof(double))); h->allocs.push_back(d); h->scratch = (double *)d;
     WS_CUDA(cudaMalloc(&d, 64)); h->allocs.push_back(d); h->work_counter = (int *)d;
     h->shift_smem = shift_smem_bytes(P, optin, &h->shift_stage);
@@ -527,8 +531,37 @@ extern "C" int wshmpc_plant_step(wshmpc_handle *h, const wshmpc_plant *pl, int n
     return 0;
 }
 
-// wshmpc_closed_loop (plant = null: x <- x_1|t + e_t) and wshmpc_closed_loop_plant
+// a wshmpc_fallback checked against the handle's problem; n = the instances it serves
+static int fallback_view(const wshmpc_handle *h, const wshmpc_fallback *fb, int n, FallbackView *v)
+{
+    if (!fb) WS_FAIL(-1, "null fallback");
+    if (h->P.node_rule != 0) WS_FAIL(-1, "node rule %d: the fallback policy runs under the structured search (node rule 0) only", h->P.node_rule);
+    if (fb->max_hold < 0 || fb->max_hold > h->P.T - 1) WS_FAIL(-1, "fallback max_hold = %d out of range 0 .. T - 1 = %d", fb->max_hold, h->P.T - 1);
+    if (!fb->d_plan || !fb->d_age || !fb->d_app_cost || !fb->d_app_primal || !fb->d_hold) WS_FAIL(-1, "null fallback buffer");
+    const size_t bytes = (size_t)n * h->P.n_primal * sizeof(double);
+    const char *p = (const char *)fb->d_plan, *a = (const char *)fb->d_app_primal;
+    if (p < a + bytes && a < p + bytes) WS_FAIL(-1, "fallback d_plan and d_app_primal overlap");
+    v->max_hold = fb->max_hold; v->plan = fb->d_plan; v->age = fb->d_age; v->app_cost = fb->d_app_cost;
+    v->app_primal = fb->d_app_primal; v->hold = fb->d_hold;
+    return 0;
+}
+
+extern "C" int wshmpc_fallback_step(wshmpc_handle *h, int n_inst, const wshmpc_fallback *fb, const double *d_x, const int *d_active,
+                                    const int *d_status, const double *d_inc_cost, const double *d_inc_primal)
+{
+    if (!h) WS_FAIL(-1, "null handle");
+    if (n_inst <= 0) return 0;
+    if (!d_x || !d_status || !d_inc_cost || !d_inc_primal) WS_FAIL(-1, "null argument");
+    FallbackView v; int rc = fallback_view(h, fb, n_inst, &v); if (rc) return rc;
+    WS_CUDA(cudaSetDevice(h->device));
+    fallback_step_kernel<<<(n_inst + 127) / 128, 128, 0, h->stream>>>(h->P, n_inst, v, d_x, d_active, d_status, d_inc_cost, d_inc_primal);
+    WS_CUDA(cudaGetLastError());
+    return 0;
+}
+
+// wshmpc_closed_loop (plant = null: x <- x_1|t + e_t), wshmpc_closed_loop_plant and wshmpc_closed_loop_fallback (fb != null)
 static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                              const wshmpc_fallback *fb,
                               const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol, int max_solves,
                               double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
                               int *d_status, unsigned long long *d_totals)
@@ -560,6 +593,12 @@ static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *l
         }
         pv.stage = h->plant_stage;
     }
+    FallbackView fv;
+    memset(&fv, 0, sizeof(fv));
+    if (fb) {
+        if (loop->mailbox) WS_FAIL(-1, "a fallback and a mailbox: the mailbox loop has no fallback policy");
+        rc = fallback_view(h, fb, n_inst, &fv); if (rc) return rc;
+    }
     LoopView L;
     L.n_steps = loop->n_steps; L.warm = loop->warm; L.fresh = loop->fresh; L.par = loop->par & 1;
     L.q = loop->d_queue; L.step_of = loop->d_step_of; L.x = loop->d_x; L.e = loop->d_e; L.active = loop->d_active;
@@ -588,7 +627,17 @@ static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *l
     const bool miqp = h->P.node_rule != 0, one = slots <= h->n_sm || h->P.lanes == 1;
     const DevProblem &P = one ? h->P1 : h->P;
     const dim3 grid(one ? slots : (slots + h->P.lanes - 1) / h->P.lanes), block(one ? WS_NT : h->P.lanes * WS_NT);
-    if (plant) {
+    if (fb && plant) {
+        auto *k = one ? closed_loop_plant_fb_kernel_1 : closed_loop_plant_fb_kernel_m;
+        k<<<grid, block, P.so.total_bytes, h->stream>>>(
+            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
+            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, pv, fv);
+    } else if (fb) {
+        auto *k = one ? closed_loop_fb_kernel_1 : closed_loop_fb_kernel_m;
+        k<<<grid, block, P.so.total_bytes, h->stream>>>(
+            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
+            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, fv);
+    } else if (plant) {
         auto *k = one ? (miqp ? closed_loop_miqp_plant_kernel_1 : closed_loop_plant_kernel_1)
                       : (miqp ? closed_loop_miqp_plant_kernel_m : closed_loop_plant_kernel_m);
         k<<<grid, block, P.so.total_bytes, h->stream>>>(
@@ -609,7 +658,7 @@ extern "C" int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loo
                                   double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
                                   int *d_status, unsigned long long *d_totals)
 {
-    return closed_loop_launch(h, n_inst, loop, nullptr, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
+    return closed_loop_launch(h, n_inst, loop, nullptr, nullptr, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
                               d_n_solves, d_status, d_totals);
 }
 
@@ -619,7 +668,17 @@ extern "C" int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshm
                                         int *d_status, unsigned long long *d_totals)
 {
     if (!plant) WS_FAIL(-1, "null plant");
-    return closed_loop_launch(h, n_inst, loop, plant, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
+    return closed_loop_launch(h, n_inst, loop, plant, nullptr, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
+                              d_n_solves, d_status, d_totals);
+}
+
+extern "C" int wshmpc_closed_loop_fallback(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
+                                           const wshmpc_fallback *fb, const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol,
+                                           int max_solves, double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,
+                                           int *d_status, unsigned long long *d_totals)
+{
+    if (!fb) WS_FAIL(-1, "null fallback");
+    return closed_loop_launch(h, n_inst, loop, plant, fb, tree0, tree1, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal,
                               d_n_solves, d_status, d_totals);
 }
 
