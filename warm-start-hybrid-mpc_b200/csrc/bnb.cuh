@@ -264,33 +264,7 @@ bnb_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double 
     double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *status_out, int *trace, unsigned long long *totals
 #define WS_BNB_PASS P, slot_d, slot_i, ybuf, scratch, work_counter, n_slots, n_inst, x0, active, tr, tol, max_solves, \
     inc_cost, inc_node, inc_primal, n_solves, status_out, trace, totals
-// one lane per CTA: 255 registers per thread (launches that cannot fill two lanes per SM: latency mode, large systems)
-__global__ void __launch_bounds__(WS_NT, 1) bnb_kernel_1(WS_BNB_ARGS)
-#if WS_TU_HAS(3)
-{ bnb_body<1, 0>(WS_BNB_PASS); }
-#else
-;
-#endif
-// WS_MAXL lanes per CTA: 65536 / (WS_MAXL WS_NT) registers per thread (throughput mode)
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) bnb_kernel_m(WS_BNB_ARGS)
-#if WS_TU_HAS(4)
-{ bnb_body<WS_MAXL, 0>(WS_BNB_PASS); }
-#else
-;
-#endif
-// the same two builds under the conventional MIQP node rule (wshmpc_set_node_rule 1 or 2)
-__global__ void __launch_bounds__(WS_NT, 1) bnb_miqp_kernel_1(WS_BNB_ARGS)
-#if WS_TU_HAS(7)
-{ bnb_body<1, BNB_RULE_MIQP>(WS_BNB_PASS); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) bnb_miqp_kernel_m(WS_BNB_ARGS)
-#if WS_TU_HAS(8)
-{ bnb_body<WS_MAXL, BNB_RULE_MIQP>(WS_BNB_PASS); }
-#else
-;
-#endif
+#define WS_BNB_BODY(LANES, RULE, PLANT, FB) bnb_body<LANES, RULE>(WS_BNB_PASS)
 
 // ---------------------------------------------------------------------------------------------
 // K2 + K4: retain / shift identifiers / shift duals / re-evaluate the bounds / plant update
@@ -760,12 +734,12 @@ __global__ void fallback_step_kernel(DevProblem P, int n_inst, FallbackView fb, 
 // model plus an additive error; the kernels without it carry no code of the plant and never read `pv`.
 // FB: the fallback policy (wshmpc_closed_loop_fallback, `fv`): after K3 the plant and K2 + K4 read the applied pair
 // fv.app_cost / fv.app_primal instead of the incumbent; the kernels without it never read `fv`.
-template <int LANES, int RULE, bool PLANT, bool FB = false>
+template <int LANES, int RULE, bool PLANT, bool FB>
 __device__ __forceinline__ void
 closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf, double *scratch, const LoopView &L, int n_slots, int n_inst,
                    const TreeView &t0, const TreeView &t1, double tol, int max_solves,
                    double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *status_out,
-                   unsigned long long *totals, const PlantView &pv, const FallbackView &fv = FallbackView())
+                   unsigned long long *totals, const PlantView &pv, const FallbackView &fv)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ int s_inst_[WS_MAXL];
@@ -967,85 +941,10 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
 
 #define WS_LOOP_ARGS DevProblem P, double *slot_d, int *slot_i, double *ybuf, double *scratch, LoopView L, int n_slots, int n_inst, \
     TreeView t0, TreeView t1, double tol, int max_solves, double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, \
-    int *status_out, unsigned long long *totals
+    int *status_out, unsigned long long *totals, PlantView pv, FallbackView fv
 #define WS_LOOP_PASS P, slot_d, slot_i, ybuf, scratch, L, n_slots, n_inst, t0, t1, tol, max_solves, inc_cost, inc_node, inc_primal, \
-    n_solves, status_out, totals
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_kernel_1(WS_LOOP_ARGS)
-#if WS_TU_HAS(5)
-{ closed_loop_body<1, 0, false>(WS_LOOP_PASS, PlantView()); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_kernel_m(WS_LOOP_ARGS)
-#if WS_TU_HAS(6)
-{ closed_loop_body<WS_MAXL, 0, false>(WS_LOOP_PASS, PlantView()); }
-#else
-;
-#endif
-// the fused loop of the conventional MIQP comparator (node rule 1 or 2; cold trees only)
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_kernel_1(WS_LOOP_ARGS)
-#if WS_TU_HAS(9)
-{ closed_loop_body<1, BNB_RULE_MIQP, false>(WS_LOOP_PASS, PlantView()); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_kernel_m(WS_LOOP_ARGS)
-#if WS_TU_HAS(10)
-{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP, false>(WS_LOOP_PASS, PlantView()); }
-#else
-;
-#endif
-// the fused loop against the nonlinear plant (wshmpc_closed_loop_plant): node rule 0 (warm or cold) and the comparator
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_plant_kernel_1(WS_LOOP_ARGS, PlantView pv)
-#if WS_TU_HAS(11)
-{ closed_loop_body<1, 0, true>(WS_LOOP_PASS, pv); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_plant_kernel_m(WS_LOOP_ARGS, PlantView pv)
-#if WS_TU_HAS(12)
-{ closed_loop_body<WS_MAXL, 0, true>(WS_LOOP_PASS, pv); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_miqp_plant_kernel_1(WS_LOOP_ARGS, PlantView pv)
-#if WS_TU_HAS(13)
-{ closed_loop_body<1, BNB_RULE_MIQP, true>(WS_LOOP_PASS, pv); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_miqp_plant_kernel_m(WS_LOOP_ARGS, PlantView pv)
-#if WS_TU_HAS(14)
-{ closed_loop_body<WS_MAXL, BNB_RULE_MIQP, true>(WS_LOOP_PASS, pv); }
-#else
-;
-#endif
-// the fused loop under the fallback policy (wshmpc_closed_loop_fallback; node rule 0, warm or cold): linear plant ...
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_fb_kernel_1(WS_LOOP_ARGS, FallbackView fv)
-#if WS_TU_HAS(15)
-{ closed_loop_body<1, 0, false, true>(WS_LOOP_PASS, PlantView(), fv); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_fb_kernel_m(WS_LOOP_ARGS, FallbackView fv)
-#if WS_TU_HAS(16)
-{ closed_loop_body<WS_MAXL, 0, false, true>(WS_LOOP_PASS, PlantView(), fv); }
-#else
-;
-#endif
-// ... and the nonlinear plant on the device
-__global__ void __launch_bounds__(WS_NT, 1) closed_loop_plant_fb_kernel_1(WS_LOOP_ARGS, PlantView pv, FallbackView fv)
-#if WS_TU_HAS(17)
-{ closed_loop_body<1, 0, true, true>(WS_LOOP_PASS, pv, fv); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) closed_loop_plant_fb_kernel_m(WS_LOOP_ARGS, PlantView pv, FallbackView fv)
-#if WS_TU_HAS(18)
-{ closed_loop_body<WS_MAXL, 0, true, true>(WS_LOOP_PASS, pv, fv); }
-#else
-;
-#endif
+    n_solves, status_out, totals, pv, fv
+#define WS_LOOP_BODY(LANES, RULE, PLANT, FB) closed_loop_body<LANES, RULE, PLANT, FB>(WS_LOOP_PASS)
 
 #if WS_TU_HAS(0)
 // wshmpc_plant_step: one thread per state, x_out[i] = Phi(x[i], u[i][fc_index]; parameter set i or 0)

@@ -41,11 +41,10 @@
 #include <math.h>
 #include <stdint.h>
 
-// Translation units.  The eighteen large kernels (K1 / K3 / fused loop, one- and multi-lane build each, K3 / fused loop under
-// the conventional MIQP node rule, the fused loop against the nonlinear plant under either rule, and the fused loop under the
-// fallback policy with either plant) take about a minute of ptxas each; wshmpc.cu can be compiled as ONE unit (WS_TU
-// undefined: everything) or as nineteen units in parallel (-DWS_TU=0: C ABI + the small kernels, -DWS_TU=1..18: one large
-// kernel each; __graft_entry__.build()).  A unit that does not define a kernel only declares it.
+// Translation units.  The large kernels (the kernel table in wshmpc.cu: one row per kernel) take about a minute of ptxas
+// each; wshmpc.cu can be compiled as ONE unit (WS_TU undefined: everything) or as one unit per large kernel plus unit 0 in
+// parallel (-DWS_TU=0: C ABI + the small kernels, -DWS_TU=u: the kernel of row u; __graft_entry__.build()).  A unit that
+// does not define a kernel only declares it.
 #ifndef WS_TU
 #define WS_TU_HAS(id) 1
 #else
@@ -73,10 +72,9 @@
 #ifndef WS_NOINLINE
 #define WS_NOINLINE __forceinline__      // measured: out-of-line phases (__noinline__) shrink the code by a third and cost 25 % (call ABI spills)
 #endif
-// Register-budget knobs of a translation unit: the one-lane kernels (units 1, 3, 5, 7, 9, 11, 13, 15, 17) have 255 registers
-// per thread, the two-lane kernels (2, 4, 6, 8, 10, 12, 14, 16, 18; also single-unit builds) 128.  None of them changes a result.
-#if defined(WS_TU) && (WS_TU == 1 || WS_TU == 3 || WS_TU == 5 || WS_TU == 7 || WS_TU == 9 || WS_TU == 11 || WS_TU == 13 || \
-                       WS_TU == 15 || WS_TU == 17)
+// Register-budget knobs of a translation unit: the one-lane kernels (the odd units of the kernel table, which checks this)
+// have 255 registers per thread, the two-lane kernels (even units; also single-unit builds) 128.  None of them changes a result.
+#if defined(WS_TU) && WS_TU % 2 == 1
 #define WS_WIDE_REGS 1
 #else
 #define WS_WIDE_REGS 0

@@ -105,17 +105,51 @@ solve_nodes_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
     const int *__restrict__ hot, const double *__restrict__ y0, const double *__restrict__ yc0, \
     int *status, double *cost, double *dobj, int *iters, double *primal, double *dual, double *yc_out
 #define WS_K1_PASS P, slot_d, slot_i, ybuf, n_slots, n_nodes, x0, lb, ub, slot_of, hot, y0, yc0, status, cost, dobj, iters, primal, dual, yc_out
-__global__ void __launch_bounds__(WS_NT, 1) solve_nodes_kernel_1(WS_K1_ARGS)
-#if WS_TU_HAS(1)
-{ solve_nodes_body<1>(WS_K1_PASS); }
-#else
-;
-#endif
-__global__ void __launch_bounds__(WS_MAXL * WS_NT, 1) solve_nodes_kernel_m(WS_K1_ARGS)
-#if WS_TU_HAS(2)
-{ solve_nodes_body<WS_MAXL>(WS_K1_PASS); }
-#else
-;
+#define WS_K1_BODY(LANES, RULE, PLANT, FB) solve_nodes_body<LANES>(WS_K1_PASS)
+
+// ---------------------------------------------------------------------------------------------
+// The large kernels.  Row u is translation unit u (-DWS_TU=u compiles exactly that kernel; unit 0 holds the C ABI and the
+// small kernels).  Columns: unit, name, family (K1: solve_nodes_body, BNB: bnb_body, LOOP: closed_loop_body), solver lanes
+// per CTA, node rule (0 the structured search, BNB_RULE_MIQP the conventional MIQP search of wshmpc_set_node_rule 1 and 2),
+// nonlinear plant on the device (wshmpc_closed_loop_plant), fallback policy (wshmpc_closed_loop_fallback).  One lane keeps
+// 255 registers per thread for launches that cannot fill WS_MAXL lanes per SM (latency mode, large systems); WS_MAXL lanes
+// get 65536 / (WS_MAXL WS_NT) (throughput mode).  The one-lane kernels take the odd units, which set WS_WIDE_REGS
+// (qp_device.cuh).  The host sets the kernels' attributes and picks the kernel of a launch from this table (kernel_for).
+// ---------------------------------------------------------------------------------------------
+#define WS_ROW_1(X)  X(1,  solve_nodes_kernel_1,            K1,   1,       0,             0, 0)
+#define WS_ROW_2(X)  X(2,  solve_nodes_kernel_m,            K1,   WS_MAXL, 0,             0, 0)
+#define WS_ROW_3(X)  X(3,  bnb_kernel_1,                    BNB,  1,       0,             0, 0)
+#define WS_ROW_4(X)  X(4,  bnb_kernel_m,                    BNB,  WS_MAXL, 0,             0, 0)
+#define WS_ROW_5(X)  X(5,  closed_loop_kernel_1,            LOOP, 1,       0,             0, 0)
+#define WS_ROW_6(X)  X(6,  closed_loop_kernel_m,            LOOP, WS_MAXL, 0,             0, 0)
+#define WS_ROW_7(X)  X(7,  bnb_miqp_kernel_1,               BNB,  1,       BNB_RULE_MIQP, 0, 0)
+#define WS_ROW_8(X)  X(8,  bnb_miqp_kernel_m,               BNB,  WS_MAXL, BNB_RULE_MIQP, 0, 0)
+#define WS_ROW_9(X)  X(9,  closed_loop_miqp_kernel_1,       LOOP, 1,       BNB_RULE_MIQP, 0, 0)
+#define WS_ROW_10(X) X(10, closed_loop_miqp_kernel_m,       LOOP, WS_MAXL, BNB_RULE_MIQP, 0, 0)
+#define WS_ROW_11(X) X(11, closed_loop_plant_kernel_1,      LOOP, 1,       0,             1, 0)
+#define WS_ROW_12(X) X(12, closed_loop_plant_kernel_m,      LOOP, WS_MAXL, 0,             1, 0)
+#define WS_ROW_13(X) X(13, closed_loop_miqp_plant_kernel_1, LOOP, 1,       BNB_RULE_MIQP, 1, 0)
+#define WS_ROW_14(X) X(14, closed_loop_miqp_plant_kernel_m, LOOP, WS_MAXL, BNB_RULE_MIQP, 1, 0)
+#define WS_ROW_15(X) X(15, closed_loop_fb_kernel_1,         LOOP, 1,       0,             0, 1)
+#define WS_ROW_16(X) X(16, closed_loop_fb_kernel_m,         LOOP, WS_MAXL, 0,             0, 1)
+#define WS_ROW_17(X) X(17, closed_loop_plant_fb_kernel_1,   LOOP, 1,       0,             1, 1)
+#define WS_ROW_18(X) X(18, closed_loop_plant_fb_kernel_m,   LOOP, WS_MAXL, 0,             1, 1)
+#define WS_KERNELS(X) WS_ROW_1(X) WS_ROW_2(X) WS_ROW_3(X) WS_ROW_4(X) WS_ROW_5(X) WS_ROW_6(X) WS_ROW_7(X) WS_ROW_8(X) \
+    WS_ROW_9(X) WS_ROW_10(X) WS_ROW_11(X) WS_ROW_12(X) WS_ROW_13(X) WS_ROW_14(X) WS_ROW_15(X) WS_ROW_16(X) WS_ROW_17(X) WS_ROW_18(X)
+
+#define WS_KERNEL_SIG(name, fam, lanes) __global__ void __launch_bounds__((lanes) * WS_NT, 1) name(WS_##fam##_ARGS)
+#define WS_DECLARE(u, name, fam, lanes, rule, plant, fb) WS_KERNEL_SIG(name, fam, lanes);
+#define WS_DEFINE(u, name, fam, lanes, rule, plant, fb) WS_KERNEL_SIG(name, fam, lanes) { WS_##fam##_BODY(lanes, rule, plant, fb); }
+WS_KERNELS(WS_DECLARE)
+#ifndef WS_TU
+WS_KERNELS(WS_DEFINE)
+#elif WS_TU > 0
+#define WS_DEFINE_UNIT(u, name, fam, lanes, rule, plant, fb) \
+    static_assert(((lanes) == 1) == (WS_WIDE_REGS == 1), #name ": one-lane kernels take the odd units, the others the even ones"); \
+    WS_DEFINE(u, name, fam, lanes, rule, plant, fb)
+#define WS_CAT_(a, b) a##b
+#define WS_CAT(a, b) WS_CAT_(a, b)
+WS_CAT(WS_ROW_, WS_TU)(WS_DEFINE_UNIT)
 #endif
 
 #if WS_TU_HAS(0)          // the C ABI (host code) lives in unit 0
@@ -138,6 +172,31 @@ static std::vector<double> transpose(const double *a, int rows, int cols) {
     std::vector<double> t((size_t)rows * cols);
     for (int i = 0; i < rows; ++i) for (int j = 0; j < cols; ++j) t[(size_t)j * rows + i] = a[(size_t)i * cols + j];
     return t;
+}
+
+enum KernelFamily { FAMILY_K1, FAMILY_BNB, FAMILY_LOOP };
+struct KernelRow { void *fn; KernelFamily family; int lanes; bool miqp, plant, fb; };
+#define WS_KERNEL_ROW(u, name, fam, lanes, rule, plant, fb) {(void *)name, FAMILY_##fam, lanes, (rule) != 0, (plant) != 0, (fb) != 0},
+static const KernelRow g_kernels[] = {WS_KERNELS(WS_KERNEL_ROW)};
+
+// the kernel of `family` compiled for (lanes, node rule != 0, plant, fb); a combination without a row fails with a message
+template <class F>
+static int kernel_for(KernelFamily family, int lanes, bool miqp, bool plant, bool fb, F *out)
+{
+    for (const KernelRow &r : g_kernels)
+        if (r.family == family && r.lanes == lanes && r.miqp == miqp && r.plant == plant && r.fb == fb) { *out = (F)r.fn; return 0; }
+    WS_FAIL(-1, "no kernel of family %d for %d lanes, node rule %s, plant %d, fallback %d", (int)family, lanes, miqp ? "!= 0" : "0",
+            (int)plant, (int)fb);
+}
+
+// launch shape of a large kernel over `slots` solver states: one lane per CTA (P1) when the states cannot fill P.lanes lanes
+// on every SM or the handle has one lane, P.lanes lanes per CTA (P) otherwise.  `lanes` is what the kernel is compiled for.
+struct LaunchShape { int lanes; const DevProblem *P; dim3 grid, block; size_t smem; };
+static LaunchShape launch_shape(const wshmpc_handle *h, int slots)
+{
+    const bool one = slots <= h->n_sm || h->P.lanes == 1;
+    const DevProblem &P = one ? h->P1 : h->P;
+    return {one ? 1 : WS_MAXL, &P, dim3((slots + P.lanes - 1) / P.lanes), dim3(P.lanes * WS_NT), (size_t)P.so.total_bytes};
 }
 
 extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, void *stream, wshmpc_handle **out)
@@ -294,30 +353,13 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
         lay(h->P1, 1);
         h->smem = (size_t)(P.so.total_bytes > h->P1.so.total_bytes ? P.so.total_bytes : h->P1.so.total_bytes);
     }
-    WS_CUDA(cudaFuncSetAttribute(solve_nodes_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(solve_nodes_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    for (const KernelRow &r : g_kernels) WS_CUDA(cudaFuncSetAttribute(r.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     // slot memory
     void *d = nullptr;
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * slot_doubles(n, P.ld) * sizeof(double))); h->allocs.push_back(d); h->slot_d = (double *)d;
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * slot_ints(n) * sizeof(int))); h->allocs.push_back(d); h->slot_i = (int *)d;
     WS_CUDA(cudaMemset(h->slot_i, 0, (size_t)n_slots * slot_ints(n) * sizeof(int)));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * m * sizeof(double))); h->allocs.push_back(d); h->ybuf = (double *)d;
-    WS_CUDA(cudaFuncSetAttribute(bnb_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(bnb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(bnb_miqp_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(bnb_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_miqp_plant_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_fb_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_fb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_fb_kernel_1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
-    WS_CUDA(cudaFuncSetAttribute(closed_loop_plant_fb_kernel_m, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * bnb_scratch_doubles(p->nb, L.primal) * sizeof(double))); h->allocs.push_back(d); h->scratch = (double *)d;
     WS_CUDA(cudaMalloc(&d, 64)); h->allocs.push_back(d); h->work_counter = (int *)d;
     h->shift_smem = shift_smem_bytes(P, optin, &h->shift_stage);
@@ -404,14 +446,11 @@ extern "C" int wshmpc_solve_nodes(wshmpc_handle *h, int n_nodes, const double *d
     if (!h) WS_FAIL(-1, "null handle");
     if (n_nodes <= 0) return 0;
     WS_CUDA(cudaSetDevice(h->device));
-    if (h->n_slots <= h->n_sm || h->P.lanes == 1)
-        solve_nodes_kernel_1<<<h->n_slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
-            h->P1, h->slot_d, h->slot_i, h->ybuf, h->n_slots, n_nodes, d_x0, d_lb, d_ub, d_slot, d_hot, d_y0, d_yc0,
-            d_status, d_cost, d_dobj, d_iters, d_primal, d_dual, d_yc);
-    else
-    solve_nodes_kernel_m<<<(h->n_slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
-        h->P, h->slot_d, h->slot_i, h->ybuf, h->n_slots, n_nodes, d_x0, d_lb, d_ub, d_slot, d_hot, d_y0, d_yc0,
-        d_status, d_cost, d_dobj, d_iters, d_primal, d_dual, d_yc);
+    const LaunchShape s = launch_shape(h, h->n_slots);
+    void (*k)(WS_K1_ARGS);
+    int rc = kernel_for(FAMILY_K1, s.lanes, false, false, false, &k); if (rc) return rc;
+    k<<<s.grid, s.block, s.smem, h->stream>>>(*s.P, h->slot_d, h->slot_i, h->ybuf, h->n_slots, n_nodes, d_x0, d_lb, d_ub, d_slot, d_hot,
+                                              d_y0, d_yc0, d_status, d_cost, d_dobj, d_iters, d_primal, d_dual, d_yc);
     WS_CUDA(cudaGetLastError());
     return 0;
 }
@@ -468,18 +507,13 @@ extern "C" int wshmpc_bnb_solve(wshmpc_handle *h, int n_inst, const double *d_x0
     WS_CUDA(cudaSetDevice(h->device));
     WS_CUDA(cudaMemsetAsync(h->work_counter, 0, sizeof(int), h->stream));
     const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
-    const bool one = slots <= h->n_sm || h->P.lanes == 1, miqp = h->P.node_rule != 0;
+    const LaunchShape s = launch_shape(h, slots);
     // the node rule picks the kernel: the structured search's kernels carry no code of the conventional rule
-    auto *k1 = miqp ? bnb_miqp_kernel_1 : bnb_kernel_1;
-    auto *km = miqp ? bnb_miqp_kernel_m : bnb_kernel_m;
-    if (one)
-        k1<<<slots, WS_NT, h->P1.so.total_bytes, h->stream>>>(
-            h->P1, h->slot_d, h->slot_i, h->ybuf, h->scratch, h->work_counter, slots, n_inst, d_x0, d_active, tv, tol, max_solves,
-            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_trace, d_totals);
-    else
-    km<<<(slots + h->P.lanes - 1) / h->P.lanes, h->P.lanes * WS_NT, h->P.so.total_bytes, h->stream>>>(
-        h->P, h->slot_d, h->slot_i, h->ybuf, h->scratch, h->work_counter, slots, n_inst, d_x0, d_active, tv, tol, max_solves,
-        d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_trace, d_totals);
+    void (*k)(WS_BNB_ARGS);
+    rc = kernel_for(FAMILY_BNB, s.lanes, h->P.node_rule != 0, false, false, &k); if (rc) return rc;
+    k<<<s.grid, s.block, s.smem, h->stream>>>(*s.P, h->slot_d, h->slot_i, h->ybuf, h->scratch, h->work_counter, slots, n_inst, d_x0,
+                                              d_active, tv, tol, max_solves, d_inc_cost, d_inc_node, d_inc_primal, d_n_solves,
+                                              d_status, d_trace, d_totals);
     WS_CUDA(cudaGetLastError());
     return 0;
 }
@@ -620,35 +654,15 @@ static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *l
         L.mb_stage = (double *)mb->priv;
         L.mb_timeout_ns = (unsigned long long)(mb->timeout_ms > 0 ? mb->timeout_ms : 5000) * 1000000ull;
     }
+    const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
+    const LaunchShape s = launch_shape(h, slots);
+    void (*k)(WS_LOOP_ARGS);
+    rc = kernel_for(FAMILY_LOOP, s.lanes, h->P.node_rule != 0, plant != nullptr, fb != nullptr, &k); if (rc) return rc;
     const int n_items = n_inst * (loop->n_steps + 1);
     loop_init_kernel<<<(n_items + 255) / 256, 256, 0, h->stream>>>(n_inst, n_items, L);
     WS_CUDA(cudaGetLastError());
-    const int slots = n_inst < h->n_slots ? n_inst : h->n_slots;
-    const bool miqp = h->P.node_rule != 0, one = slots <= h->n_sm || h->P.lanes == 1;
-    const DevProblem &P = one ? h->P1 : h->P;
-    const dim3 grid(one ? slots : (slots + h->P.lanes - 1) / h->P.lanes), block(one ? WS_NT : h->P.lanes * WS_NT);
-    if (fb && plant) {
-        auto *k = one ? closed_loop_plant_fb_kernel_1 : closed_loop_plant_fb_kernel_m;
-        k<<<grid, block, P.so.total_bytes, h->stream>>>(
-            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
-            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, pv, fv);
-    } else if (fb) {
-        auto *k = one ? closed_loop_fb_kernel_1 : closed_loop_fb_kernel_m;
-        k<<<grid, block, P.so.total_bytes, h->stream>>>(
-            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
-            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, fv);
-    } else if (plant) {
-        auto *k = one ? (miqp ? closed_loop_miqp_plant_kernel_1 : closed_loop_plant_kernel_1)
-                      : (miqp ? closed_loop_miqp_plant_kernel_m : closed_loop_plant_kernel_m);
-        k<<<grid, block, P.so.total_bytes, h->stream>>>(
-            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
-            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, pv);
-    } else {
-        auto *k = one ? (miqp ? closed_loop_miqp_kernel_1 : closed_loop_kernel_1) : (miqp ? closed_loop_miqp_kernel_m : closed_loop_kernel_m);
-        k<<<grid, block, P.so.total_bytes, h->stream>>>(
-            P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
-            d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals);
-    }
+    k<<<s.grid, s.block, s.smem, h->stream>>>(*s.P, h->slot_d, h->slot_i, h->ybuf, h->scratch, L, slots, n_inst, v0, v1, tol, max_solves,
+                                              d_inc_cost, d_inc_node, d_inc_primal, d_n_solves, d_status, d_totals, pv, fv);
     WS_CUDA(cudaGetLastError());
     return 0;
 }
