@@ -311,10 +311,15 @@ int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *lo
  *   incumbent                                 plan <- incumbent, age <- 0; the applied pair is the incumbent;       hold 0
  *   status 1 (infeasible), age + 1 <= max_hold  age <- age + 1; applied u_0 = u_age of the plan,
  *                                             x_1|t = A x_t + B u_0; the instance stays live;                      hold age
- *   otherwise (no plan, plan used up, status 2 or 3, instance off)   the instance is switched off as without a fallback; hold -1
+ *   status 1, otherwise (no plan or plan used up), law_n + 1 <= max_law
+ *                                             law_n <- law_n + 1; applied u_0 = K x_t (the terminal law),
+ *                                             x_1|t = A x_t + B u_0; age kept; the instance stays live;              hold -2
+ *   otherwise (law used up, status 2 or 3, instance off)   the instance is switched off as without a fallback;      hold -1
+ * An incumbent also resets law_n to 0.  The terminal law is the linear feedback of the terminal set (e.g. the LQR gain it was
+ * built with), without offset or saturation; K is [nu][nx], row-major, shared by all instances.
  * A status-1 step ran its search to the end: its leaves are a complete cover (Farkas proofs and bounds) and K2 + K4 shift them
- * with the applied input like a solved tree.  The logs of a fallback step keep cost +inf and status 1; u0 is the applied
- * input.  All buffers are device memory owned by the caller, so plans survive launches.
+ * with the applied input like a solved tree, for any input.  The logs of a fallback step keep cost +inf and status 1; u0 is
+ * the applied input.  All buffers are device memory owned by the caller, so plans survive launches.
  *   d_plan       [n_inst][layout.primal]
  *   d_age        [n_inst] in/out (fill with -1 to start without plans)
  *   d_app_cost   [n_inst] applied pair, what K2 + K4 and the plant read in place of the incumbent: the incumbent's cost, 0 on a
@@ -322,8 +327,10 @@ int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *lo
  *   d_app_primal [n_inst][layout.primal] the incumbent's record; on a fallback step only x_0, x_1 and u_0 are defined.
  *                Must not overlap d_plan.
  *   d_hold       [n_steps][n_inst] (wshmpc_closed_loop_fallback) or [n_inst] (wshmpc_fallback_step): 0 the incumbent,
- *                a > 0 input u_a of the plan, -1 the instance left the loop (or was off)
- * max_hold = 0 is the behaviour without a fallback, bit for bit. */
+ *                a > 0 input u_a of the plan, -2 the terminal law, -1 the instance left the loop (or was off)
+ *   d_law_K      [nu][nx] the terminal law's gain (read when max_law > 0)
+ *   d_law_n      [n_inst] in/out, law steps since the last incumbent (fill with 0 to start; read when max_law > 0)
+ * max_hold = max_law = 0 is the behaviour without a fallback, bit for bit; max_law = 0 is the policy without the law. */
 typedef struct {
     int max_hold;          /* H, 0 <= H <= T - 1 */
     double *d_plan;
@@ -331,11 +338,15 @@ typedef struct {
     double *d_app_cost;
     double *d_app_primal;
     int *d_hold;
+    int max_law;           /* L >= 0 */
+    const double *d_law_K;
+    int *d_law_n;
 } wshmpc_fallback;
 
 /* wshmpc_closed_loop (plant = NULL: the linear plant x <- x_1|t + e_t) or wshmpc_closed_loop_plant under the fallback policy:
  * the plant and the warm start of every step use the applied pair.  Fails under node rules 1 and 2 (the comparator), with a
- * mailbox, for max_hold outside 0 .. T - 1, null buffers, or d_plan overlapping d_app_primal. */
+ * mailbox, for max_hold outside 0 .. T - 1, null buffers, d_plan overlapping d_app_primal, max_law < 0, or max_law > 0 with a
+ * null d_law_K or d_law_n. */
 int wshmpc_closed_loop_fallback(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
                                 const wshmpc_fallback *fb, const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol,
                                 int max_solves, double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,

@@ -107,16 +107,21 @@ def _plant_struct(plant, log_x=None):
 
 class _Fallback(C.Structure):
     _fields_ = [('max_hold', C.c_int), ('d_plan', C.c_void_p), ('d_age', C.c_void_p), ('d_app_cost', C.c_void_p),
-                ('d_app_primal', C.c_void_p), ('d_hold', C.c_void_p)]
+                ('d_app_primal', C.c_void_p), ('d_hold', C.c_void_p), ('max_law', C.c_int), ('d_law_K', C.c_void_p),
+                ('d_law_n', C.c_void_p)]
 
 
 def _fallback_struct(fb, hold):
-    """wshmpc_fallback of a dict(max_hold, plan, age, app_cost, app_primal) of CUDA tensors, with the hold log `hold`"""
+    """wshmpc_fallback of a dict(max_hold, plan, age, app_cost, app_primal) of CUDA tensors, with the hold log `hold`; the
+    terminal law comes from the optional keys max_law, law_K and law_n (without them: max_law = 0 and null pointers)"""
     c = _Fallback()
     c.max_hold = int(fb['max_hold'])
     for k in ('plan', 'age', 'app_cost', 'app_primal'):
         setattr(c, 'd_' + k, fb[k].data_ptr() if fb[k] is not None else None)
     c.d_hold = hold.data_ptr() if hold is not None else None
+    c.max_law = int(fb.get('max_law', 0))
+    for k in ('law_K', 'law_n'):
+        setattr(c, 'd_' + k, fb[k].data_ptr() if fb.get(k) is not None else None)
     return c
 
 
@@ -312,16 +317,23 @@ class Handle(object):
                                           C.c_void_p(out.data_ptr())))
         return out
 
-    def new_fallback(self, n_inst, max_hold):
+    def new_fallback(self, n_inst, max_hold, max_law=0, K=None):
         """Caller-owned buffers of the fallback policy (wshmpc_fallback) for n_inst instances, without plans (age -1):
-        dict(max_hold, plan, age, app_cost, app_primal, hold [n_inst]) of CUDA tensors."""
+        dict(max_hold, plan, age, app_cost, app_primal, hold [n_inst]) of CUDA tensors.  With max_law > 0 also the terminal
+        law: dict(max_law, law_K = a device copy of the gain K [nu, nx], law_n [n_inst] = 0)."""
         import torch
         f64 = dict(dtype=torch.float64, device=self.torch_device)
         i32 = dict(dtype=torch.int32, device=self.torch_device)
-        P = self.layout.primal
-        return dict(max_hold=int(max_hold), plan=torch.zeros((n_inst, P), **f64), age=torch.full((n_inst,), -1, **i32),
-                    app_cost=torch.zeros(n_inst, **f64), app_primal=torch.zeros((n_inst, P), **f64),
-                    hold=torch.zeros(n_inst, **i32))
+        P, nx, nu = self.layout.primal, self.pd.nx, self.pd.nu
+        fb = dict(max_hold=int(max_hold), plan=torch.zeros((n_inst, P), **f64), age=torch.full((n_inst,), -1, **i32),
+                  app_cost=torch.zeros(n_inst, **f64), app_primal=torch.zeros((n_inst, P), **f64),
+                  hold=torch.zeros(n_inst, **i32), max_law=int(max_law))
+        if max_law:
+            K = np.asarray(K, dtype=float)
+            if K.shape != (nu, nx):
+                raise ValueError('terminal law gain of shape %s: [nu, nx] = [%d, %d]' % (K.shape, nu, nx))
+            fb.update(law_K=torch.as_tensor(np.ascontiguousarray(K), **f64), law_n=torch.zeros(n_inst, **i32))
+        return fb
 
     def fallback_step(self, fb, x, active, out):
         """wshmpc_fallback_step: the fallback policy after a lock-step branch and bound (`out` of bnb_solve) at states
@@ -340,7 +352,7 @@ class Handle(object):
         plant: a plants.DevicePlant -- the nonlinear plant advances the state on the device (wshmpc_closed_loop_plant), e is
         an additive disturbance on its output, and the logs gain 'x' [n_steps, n_inst, nx], the state after every step.
         fallback: buffers of new_fallback -- the loop runs under the fallback policy (wshmpc_closed_loop_fallback, also with
-        max_hold = 0) and the logs gain 'hold' [n_steps, n_inst].
+        max_hold = 0, and with the terminal law when the buffers have one) and the logs gain 'hold' [n_steps, n_inst].
         Returns the dict of per-step logs (CUDA tensors)."""
         import torch
         dev = self.torch_device

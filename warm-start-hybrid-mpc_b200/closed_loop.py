@@ -20,7 +20,7 @@ def shard(n_total, rank, world):
 class ClosedLoop(object):
 
     def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
-                 mip_start=True, plant=None, fallback=0):
+                 mip_start=True, plant=None, fallback=0, terminal_law=0, law_gain=None):
         """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
         paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
         incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
@@ -31,7 +31,10 @@ class ClosedLoop(object):
         fallback: H, 0 <= H <= T - 1.  With H > 0 an instance whose MIQP is infeasible applies the next input of its last plan
         for up to H steps in a row instead of leaving the loop, and the shifted tree of the infeasible step warm-starts the
         next one (wshmpc_fallback in include/wshmpc.h); out['hold'] and the logs' 'hold' say where each applied input came
-        from (0 the incumbent, a > 0 input u_a of the plan, -1 none).  Not with the comparator."""
+        from (0 the incumbent, a > 0 input u_a of the plan, -2 the terminal law, -1 none).  Not with the comparator.
+        terminal_law: L >= 0.  With L > 0 an instance whose MIQP is infeasible and that has no plan step left applies the
+        terminal law u = K x for up to L steps in a row (counted since its last incumbent) instead of leaving the loop; also
+        with fallback = 0.  law_gain: K [nu, nx], default controller.terminal_law()."""
         import torch
         if comparator and warm:
             raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
@@ -39,8 +42,15 @@ class ClosedLoop(object):
             raise ValueError('the plant has %d parameter sets: 1, or one per instance (%d)' % (plant.n_sets, n_inst))
         if int(fallback) != fallback or not 0 <= fallback <= controller.T - 1:
             raise ValueError('fallback = %r: the steps an instance may hold its plan, 0 .. T - 1 = %d' % (fallback, controller.T - 1))
-        if fallback and comparator:
+        if int(terminal_law) != terminal_law or terminal_law < 0:
+            raise ValueError('terminal_law = %r: the steps an instance may run on the terminal law, >= 0' % (terminal_law,))
+        if (fallback or terminal_law) and comparator:
             raise ValueError('the fallback policy runs under the structured search only, not with the MIQP comparator')
+        if terminal_law:
+            law_gain = controller.terminal_law() if law_gain is None else np.asarray(law_gain, dtype=float)
+            if law_gain.shape != (controller.mld.nu, controller.mld.nx):
+                raise ValueError('law_gain of shape %s: the terminal law gain is [nu, nx] = [%d, %d]'
+                                 % (law_gain.shape, controller.mld.nu, controller.mld.nx))
         self.plant = plant
         if max_roots is None:
             max_roots = 2 if comparator else 512
@@ -69,7 +79,8 @@ class ClosedLoop(object):
         self.fresh = True
         self.launches = 0
         self.events = None          # list -> (start, after K3, after K2+K4) CUDA events of every step
-        self.fb = h.new_fallback(n_inst, fallback) if fallback else None     # plans, ages, applied pairs (wshmpc_fallback)
+        # plans, ages, applied pairs and the terminal law (wshmpc_fallback)
+        self.fb = h.new_fallback(n_inst, fallback, int(terminal_law), law_gain) if (fallback or terminal_law) else None
         if self.fb is not None:
             self.out['hold'] = self.fb['hold']
 
@@ -88,6 +99,8 @@ class ClosedLoop(object):
         self.active.fill_(1)
         if self.fb is not None:
             self.fb['age'].fill_(-1)
+            if self.fb.get('law_n') is not None:
+                self.fb['law_n'].zero_()
         self.totals.zero_()
         self.fresh = True
 

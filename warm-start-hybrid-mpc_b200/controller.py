@@ -159,6 +159,26 @@ class HybridModelPredictiveController(object):
             cols.append(res.x)
         return np.vstack(cols).T if cols else np.zeros((n, 0))
 
+    def terminal_law(self, inputs=None):
+        """The linear feedback u = K x of the terminal set, K [nu, nx]: the DARE (LQR) gain of the stage cost on the inputs
+        `inputs`, zero for every other input.  inputs: column indices of B (default: the columns of R that are not all
+        zero, i.e. the inputs the stage cost penalises).  K solves the DARE on (A, B[:, inputs], Q'Q, R_u'R_u) with
+        R_u = R[:, inputs]; when the terminal cost and set were built from that LQR law (a terminal cost Q_T'Q_T = P and
+        the maximal admissible set of A + B K), u = K x keeps a state of the terminal set in it."""
+        from scipy.linalg import solve_discrete_are
+        mld = self.mld
+        if inputs is None:
+            inputs = np.nonzero(np.any(self.R != 0., axis=0))[0]
+        inputs = np.asarray(inputs, dtype=int).ravel()
+        if inputs.size == 0:
+            raise ValueError('terminal_law: no inputs (R has no nonzero column)')
+        Bu, Ru = mld.B[:, inputs], self.R[:, inputs]
+        Qc, Rc = self.Q.T.dot(self.Q), Ru.T.dot(Ru)
+        P = solve_discrete_are(mld.A, Bu, Qc, Rc)
+        K = np.zeros((mld.nu, mld.nx))
+        K[inputs] = -np.linalg.inv(Bu.T.dot(P).dot(Bu) + Rc).dot(Bu.T).dot(P).dot(mld.A)
+        return K
+
     # -- device handle --------------------------------------------------------------------------
     @staticmethod
     def _require_gpu():

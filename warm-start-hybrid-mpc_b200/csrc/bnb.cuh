@@ -680,15 +680,28 @@ struct FallbackView {
     int *age;                // [n_inst] steps since that step, -1 = no plan
     double *app_cost;        // [n_inst] applied pair: +inf = the instance leaves the loop, finite otherwise
     double *app_primal;      // [n_inst][n_primal] (a fallback step defines x_0, x_1 and u_0 only)
-    int *hold;               // [n_inst] of the step: 0 the incumbent, a > 0 input u_a of the plan, -1 none
+    int *hold;               // [n_inst] of the step: 0 the incumbent, a > 0 input u_a of the plan, -2 the law, -1 none
+    int max_law;             // L: consecutive steps an instance may run on the terminal law u = K x, 0 = no law
+    const double *law_K;     // [nu][nx] the law's gain, shared by all instances (null when L = 0)
+    int *law_n;              // [n_inst] law steps since the last incumbent (null when L = 0)
 };
 
+// u_r = (K x)_r, fused multiply-adds over the columns in order (every caller and every thread gets the same bits)
+__device__ __forceinline__ double law_input(const double *__restrict__ K, const double *__restrict__ x, int r, int nx)
+{
+    double s = 0.;
+    for (int c = 0; c < nx; ++c) s = __fma_rn(K[r * nx + c], x[c], s);
+    return s;
+}
+
 // The fallback policy for instance `inst` after its branch and bound (status st; the fused loop and wshmpc_fallback_step):
-//   incumbent                            plan <- incumbent, age 0, applied pair = incumbent, hold 0;
+//   incumbent                            plan <- incumbent, age 0, law_n 0, applied pair = incumbent, hold 0;
 //   status 1, a plan with age + 1 <= H   age += 1, applied u_0 = u_age of the plan, x_1 = A x + B u_0 (fused multiply-adds
 //                                        in a fixed order, so that every caller gets the same bits), hold = age;
+//   status 1, otherwise, law_n + 1 <= L  law_n += 1, applied u_0 = K x, x_1 = A x + B u_0 (the same order), age kept, hold -2;
 //   otherwise                            applied cost +inf (K2 + K4 switch the instance off), hold -1.
-// Threads tid = 0 .. nt - 1 share the copies; `sync` is the callers' barrier (age is read by all before thread 0 writes it).
+// Threads tid = 0 .. nt - 1 share the copies; `sync` is the callers' barrier (age and law_n are read by all before thread 0
+// writes them).  With L = 0, law_n and law_K are never touched.
 template <class Sync>
 __device__ __forceinline__ void fallback_apply(const DevProblem &P, const FallbackView &fb, int inst, bool live, int st,
                                                const double *__restrict__ x, const double *__restrict__ inc_cost,
@@ -697,7 +710,9 @@ __device__ __forceinline__ void fallback_apply(const DevProblem &P, const Fallba
     const int nx = P.nx, nu = P.nu, np_ = P.n_primal;
     const size_t o = (size_t)inst * np_;
     const int a = fb.age[inst];
-    const int mode = !live ? 2 : inc_cost[inst] < INFINITY ? 0 : (st == BNB_INFEASIBLE && a >= 0 && a + 1 <= fb.max_hold) ? 1 : 2;
+    int mode = !live ? 2 : inc_cost[inst] < INFINITY ? 0 : (st == BNB_INFEASIBLE && a >= 0 && a + 1 <= fb.max_hold) ? 1 : 2;
+    const int n = fb.max_law > 0 ? fb.law_n[inst] : 0;
+    if (mode == 2 && live && st == BNB_INFEASIBLE && n + 1 <= fb.max_law) mode = 3;
     if (mode == 0) {
         for (int j = tid; j < np_; j += nt) { const double v = inc_primal[o + j]; fb.plan[o + j] = v; fb.app_primal[o + j] = v; }
     } else if (mode == 1) {
@@ -710,11 +725,22 @@ __device__ __forceinline__ void fallback_apply(const DevProblem &P, const Fallba
             ap[j] = x[j]; ap[nx + j] = s;
         }
         for (int j = tid; j < nu; j += nt) ap[(size_t)(P.T + 1) * nx + j] = u[j];
+    } else if (mode == 3) {
+        // every thread forms the inputs it needs from K x itself: no barrier between u and x_1
+        double *ap = fb.app_primal + o;
+        for (int j = tid; j < nx; j += nt) {
+            double s = 0.;
+            for (int c = 0; c < nx; ++c) s = __fma_rn(P.A[j * nx + c], x[c], s);
+            for (int c = 0; c < nu; ++c) s = __fma_rn(P.B[j * nu + c], law_input(fb.law_K, x, c, nx), s);
+            ap[j] = x[j]; ap[nx + j] = s;
+        }
+        for (int j = tid; j < nu; j += nt) ap[(size_t)(P.T + 1) * nx + j] = law_input(fb.law_K, x, j, nx);
     }
     sync();
     if (tid == 0) {
-        if (mode == 0) { fb.age[inst] = 0; fb.app_cost[inst] = inc_cost[inst]; hold[inst] = 0; }
+        if (mode == 0) { fb.age[inst] = 0; fb.app_cost[inst] = inc_cost[inst]; hold[inst] = 0; if (fb.max_law > 0) fb.law_n[inst] = 0; }
         else if (mode == 1) { fb.age[inst] = a + 1; fb.app_cost[inst] = 0.; hold[inst] = a + 1; }
+        else if (mode == 3) { fb.law_n[inst] = n + 1; fb.app_cost[inst] = 0.; hold[inst] = -2; }
         else { fb.app_cost[inst] = INFINITY; hold[inst] = -1; }
     }
 }

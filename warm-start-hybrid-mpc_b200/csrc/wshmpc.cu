@@ -575,8 +575,11 @@ static int fallback_view(const wshmpc_handle *h, const wshmpc_fallback *fb, int 
     const size_t bytes = (size_t)n * h->P.n_primal * sizeof(double);
     const char *p = (const char *)fb->d_plan, *a = (const char *)fb->d_app_primal;
     if (p < a + bytes && a < p + bytes) WS_FAIL(-1, "fallback d_plan and d_app_primal overlap");
+    if (fb->max_law < 0) WS_FAIL(-1, "fallback max_law = %d: the law steps an instance may take, >= 0", fb->max_law);
+    if (fb->max_law > 0 && (!fb->d_law_K || !fb->d_law_n)) WS_FAIL(-1, "fallback max_law = %d with a null d_law_K or d_law_n", fb->max_law);
     v->max_hold = fb->max_hold; v->plan = fb->d_plan; v->age = fb->d_age; v->app_cost = fb->d_app_cost;
     v->app_primal = fb->d_app_primal; v->hold = fb->d_hold;
+    v->max_law = fb->max_law; v->law_K = fb->max_law > 0 ? fb->d_law_K : nullptr; v->law_n = fb->max_law > 0 ? fb->d_law_n : nullptr;
     return 0;
 }
 
