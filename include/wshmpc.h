@@ -113,7 +113,10 @@ int wshmpc_set_node_rule(wshmpc_handle *h, int rule);
  *                            2: the multipliers d_y0 / proximal centre d_yc0 of this node -- what the reference hands
  *                               from a parent to its children as `active_set` (controller.py:262-264, 426)
  *   d_y0   [n_nodes][m]      (hot = 2; may be NULL otherwise) signed multipliers of the rows mu_0..mu_{T-1} | binaries:
- *                            m = layout.off_nu_lb - layout.off_mu + nb; > 0 upper side (mu, nu_ub), < 0 lower (nu_lb)
+ *                            m = layout.off_nu_lb - layout.off_mu + nb; > 0 upper side (mu, nu_ub), < 0 lower (nu_lb).
+ *                            Only finite entries that are > 0 on a row mu or != 0 on a binary enter the start; every
+ *                            other entry (negative on a row mu, which has no lower side, NaN, +-inf) is ignored, i.e.
+ *                            projected to zero, so the start stays dual feasible
  *   d_yc0  [n_nodes][n]      (hot = 2; may be NULL = 0) proximal centre, n = T * nu
  * outputs
  *   d_status [n_nodes]       2 optimal, 3 infeasible (Gurobi status codes, bounded_qp.py:212), 9 iteration limit (also: the

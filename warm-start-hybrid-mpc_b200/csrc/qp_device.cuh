@@ -1034,7 +1034,9 @@ __device__ __forceinline__ void store_slot(const DevProblem &P, const Ctx &cx, c
 // Working set from signed multipliers of the ORIGINAL rows (ysigned(r) > 0: upper side, < 0: lower side) and a
 // proximal centre: the start the reference hands from a parent to its children (`active_set`,
 // controller.py:262-264, 426) and what a shifted dual solution gives a warm-start root.  Rows keep their
-// natural order.  yc0 may be null (centre 0).
+// natural order.  yc0 may be null (centre 0).  A row enters only if its multiplier is finite and it is a bound row
+// (either side) or a stage row with y > 0: a stage row has no lower side, so every other entry is ignored (projected
+// to zero), and the start stays dual feasible whatever the caller passes.
 template <class Y>
 __device__ __forceinline__ void load_ws_from_multipliers(const DevProblem &P, const Ctx &cx, Y ysigned, const double *yc0, int &k) {
     const int lane = WS_TID & 31, w = WS_TID >> 5;
@@ -1048,7 +1050,8 @@ __device__ __forceinline__ void load_ws_from_multipliers(const DevProblem &P, co
         const int r = r0 + WS_TID;
         double yv = 0.;
         if (r < P.m) yv = ysigned(r);
-        const int keep = yv != 0. && base < P.n && !(r >= P.mc && r - P.mc < d);   // eliminated rows carry no working-set entry
+        const bool entry = isfinite(yv) && (r < P.mc ? yv > 0. : yv != 0.);
+        const int keep = entry && base < P.n && !(r >= P.mc && r - P.mc < d);   // eliminated rows carry no working-set entry
         const unsigned bal = __ballot_sync(0xffffffffu, keep);
         WS_SYNC();
         if (lane == 0) wsum[w] = __popc(bal);

@@ -356,7 +356,10 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     for (const KernelRow &r : g_kernels) WS_CUDA(cudaFuncSetAttribute(r.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
     // slot memory
     void *d = nullptr;
+    // both cleared: a slot that never stored a state starts from the empty working set AND the centre 0 (hot = 1 on a fresh
+    // slot equals hot = 0), whatever an earlier allocation left in the pages
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * slot_doubles(n, P.ld) * sizeof(double))); h->allocs.push_back(d); h->slot_d = (double *)d;
+    WS_CUDA(cudaMemset(h->slot_d, 0, (size_t)n_slots * slot_doubles(n, P.ld) * sizeof(double)));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * slot_ints(n) * sizeof(int))); h->allocs.push_back(d); h->slot_i = (int *)d;
     WS_CUDA(cudaMemset(h->slot_i, 0, (size_t)n_slots * slot_ints(n) * sizeof(int)));
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * m * sizeof(double))); h->allocs.push_back(d); h->ybuf = (double *)d;
