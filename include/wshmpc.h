@@ -54,10 +54,12 @@ typedef struct {
     int primal;                  /* (T+1)*nx + T*nu : x_0..x_T, u_0..u_{T-1}  (subproblem_solution.py:86-91) */
     int dual;                    /* lam | mu | nu_lb | nu_ub | rho | sigma     (subproblem_solution.py:137-166) */
     int off_lam, off_mu, off_nu_lb, off_nu_ub, off_rho, off_sigma;
-    int rec_stride;              /* doubles per dual record INSIDE a wshmpc_tree: dual + n.  The n extra doubles hold the
-                                    proximal centre (orthonormal coordinates) of the solve the record came from, i.e. the
-                                    `active_set` payload the reference hands from a parent to its children
-                                    (subproblem_solution.py:10, controller.py:426) */
+    int rec_stride;              /* doubles per dual record INSIDE a wshmpc_tree: dual + n, rounded up to even; the padding
+                                    double is zero.  The n doubles behind the duals hold the proximal centre (orthonormal
+                                    coordinates) of the solve the record came from, i.e. the `active_set` payload the
+                                    reference hands from a parent to its children (subproblem_solution.py:10,
+                                    controller.py:426).  The even stride keeps every record of a 16-byte aligned tree
+                                    16-byte aligned, which the tree shift's bulk copies of records need */
 } wshmpc_layout;
 
 const char *wshmpc_last_error(void);

@@ -16,31 +16,10 @@ import pytest
 import torch
 
 from oracle.models import load_model, GOLDEN, MODELS
-from oracle.qp_c import CoreC
-from oracle.bnb_ref import OracleController
-from tests.util import make_controller
+from tests.util import make_controller, oracle_loop
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-6
-
-
-def _oracle_loop(model, x0, e, warm=True):
-    """statistical_analysis.py:93-196 for one instance on the oracle: list of per-step dicts (ends when infeasible)."""
-    ctl = OracleController(model, CoreC(model, variant=1), hot_start='record')
-    x = np.array(x0, dtype=float); ws = None; log = []
-    for t in range(len(e)):
-        try:
-            inc, leaves, solves = ctl.feedforward(x, warm_start=ws if warm else None)
-        except RuntimeError:
-            log.append(dict(failed=True)); break
-        if inc is None:
-            log.append(dict(cost=np.inf, solves=solves)); break
-        u0 = inc.primal['u'][0]
-        ws = ctl.construct_warm_start(leaves, x, u0[:ctl.nuc], u0[ctl.nuc:], e[t])
-        log.append(dict(cost=inc.primal['objective'], solves=solves, u0=u0.copy(), ub=inc.primal['u'][:, ctl.nuc:].copy(),
-                        cover=len(ws), x=x.copy()))
-        x = inc.primal['x'][1] + e[t]
-    return log
 
 
 def _ub_of(ctl, primal_row):
@@ -108,7 +87,7 @@ def test_multi_instance_noisy_closed_loop_matches_oracle():
     assert np.all(status <= 1)
     n_dead = 0; worst = 0.; dn = []
     for k in range(N):
-        ref = _oracle_loop(model, x0[k], e[:, k])
+        ref = oracle_loop(model, x0[k], e[:, k])
         assert not any('failed' in r for r in ref)
         for t, r in enumerate(ref):
             if np.isinf(r['cost']):
@@ -141,7 +120,7 @@ def test_cp40_warm_start_matches_oracle():
     e = 0.003 * rng.standard_normal((S, 4)) * model['x_max']
     L = ClosedLoop(ctl, 1, warm=True, max_solves=4096, max_roots=1024, n_slots=1)
     L.reset(model['x0_nominal'][None])
-    ref = _oracle_loop(model, model['x0_nominal'], e)
+    ref = oracle_loop(model, model['x0_nominal'], e)
     assert len(ref) == S and all(np.isfinite(r['cost']) for r in ref)
     for t in range(S):
         out = L.step(e=torch.as_tensor(e[t][None], device='cuda'))
@@ -166,7 +145,7 @@ def test_syn30_bnb_and_shift_match_oracle():
     x0 = 0.3 * model['x0_nominal']           # at the full x0_nominal the MIQP needs > 10^4 nodes (best-first stalls at depth 40)
     rng = np.random.default_rng(30)
     e = 0.003 * rng.standard_normal((2, x0.size)) * model['x_max']
-    ref = _oracle_loop(model, x0, e)
+    ref = oracle_loop(model, x0, e)
     assert len(ref) == 2 and all(np.isfinite(r['cost']) for r in ref)
     L = ClosedLoop(ctl, 1, warm=True, max_solves=4096, max_roots=2048, n_slots=1)
     L.reset(x0[None])

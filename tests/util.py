@@ -222,3 +222,24 @@ def oracle_launch(model, pd, variant=1):
         return dict(status=out['status'], cost=out['cost'], dobj=dobj, iters=out['iters'], primal=primal, dual=dual,
                     yc=np.array(yc), runtime=0.)
     return launch
+
+
+def oracle_loop(model, x0, e, warm=True):
+    """statistical_analysis.py:93-196 for one instance on the oracle: list of per-step dicts (ends when infeasible)."""
+    from oracle.qp_c import CoreC
+    from oracle.bnb_ref import OracleController
+    ctl = OracleController(model, CoreC(model, variant=1), hot_start='record')
+    x = np.array(x0, dtype=float); ws = None; log = []
+    for t in range(len(e)):
+        try:
+            inc, leaves, solves = ctl.feedforward(x, warm_start=ws if warm else None)
+        except RuntimeError:
+            log.append(dict(failed=True)); break
+        if inc is None:
+            log.append(dict(cost=np.inf, solves=solves)); break
+        u0 = inc.primal['u'][0]
+        ws = ctl.construct_warm_start(leaves, x, u0[:ctl.nuc], u0[ctl.nuc:], e[t])
+        log.append(dict(cost=inc.primal['objective'], solves=solves, u0=u0.copy(), ub=inc.primal['u'][:, ctl.nuc:].copy(),
+                        cover=len(ws), x=x.copy()))
+        x = inc.primal['x'][1] + e[t]
+    return log

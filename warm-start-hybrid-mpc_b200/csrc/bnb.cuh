@@ -150,7 +150,7 @@ __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, 
         if (qs == WS_ITER_LIMIT) { st = BNB_QP_LIMIT; break; }
         double *dual = rdual + (size_t)nr * P.n_rec;
         build_records(P, qs, SMV(yc), y, xi, lbv, ubv, prim, dual, cost_s, dobj_s, SMV(part), SMV(red));
-        for (int j = WS_TID; j < P.n; j += WS_NT) dual[P.n_dual + j] = qs == WS_OPTIMAL ? SMV(yc)[j] : 0.;
+        for (int j = WS_TID; j < P.n_rec - P.n_dual; j += WS_NT) dual[P.n_dual + j] = qs == WS_OPTIMAL && j < P.n ? SMV(yc)[j] : 0.;
         prof_mark(17);
         const double cost = *cost_s;
         if (WS_TID == 0) {
@@ -412,11 +412,14 @@ __device__ __forceinline__ int shift_instance(const DevProblem &P, double *shm, 
 #if defined(WS_NO_STAGE)
     stage_avail = 0;
 #endif
-    const bool staged = (P.n_dual & 1) == 0 && stage_avail > 0 && (size_t)stage_avail >= (size_t)(w + 1) * sbuf;
+    // has_buf: the warp owns a staging buffer.  A leaf is staged only if its record starts 16-byte aligned, as cp.async.bulk
+    // requires: the even record stride keeps every record of an aligned tree aligned, and the check per leaf covers trees on
+    // any caller pointer.  Other leaves are read in place.
+    const bool has_buf = (P.n_dual & 1) == 0 && stage_avail > 0 && (size_t)stage_avail >= (size_t)(w + 1) * sbuf;
     double *stage = shm + scr + (size_t)w * sbuf;
     uint64_t *bar = reinterpret_cast<uint64_t *>(shm + scr - (NT / 32 + 1)) + w;
     uint32_t par = 0;
-    if (staged) {
+    if (has_buf) {
         if (lane == 0) { mbar_init(bar, 1); fence_async_smem(); }
         __syncwarp();
     }
@@ -446,6 +449,7 @@ __device__ __forceinline__ int shift_instance(const DevProblem &P, double *shm, 
             continue;
         }
         const double *Dg = ot.rec_dual + ((size_t)inst * ot.cap_recs + ro) * P.n_rec;
+        const bool staged = has_buf && ((uintptr_t)Dg & 15) == 0;
         if (staged) {
             __syncwarp();                                  // every lane is done with the previous leaf's copy
             if (lane == 0) {
@@ -545,7 +549,7 @@ __device__ __forceinline__ int shift_instance(const DevProblem &P, double *shm, 
             nt.lb[on_ + idx] = lbn; nt.rec[on_ + idx] = rn; nt.rec_dobj[(size_t)inst * nt.cap_recs + idx] = obj;
         }
     }
-    if (staged) {
+    if (has_buf) {
         // the barrier's memory goes back to the solver (LANE) / is initialised again for the next instance: invalidate it
         __syncwarp();
         if (lane == 0) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" :: "r"(smem_u32(bar)) : "memory");

@@ -140,7 +140,7 @@ struct DevProblem {
     SmemOff so;
     // record layout
     int n_primal, n_dual, off_lam, off_mu, off_nulb, off_nuub, off_rho, off_sigma;
-    int n_rec;               // stride of a dual record in a tree: n_dual + n (the proximal centre of the solve follows the duals)
+    int n_rec;               // stride of a dual record in a tree: n_dual + n rounded up to even (the proximal centre of the solve follows the duals)
     int node_rule;           // node rule of the device B&B (wshmpc_set_node_rule): 0 structured, 1 conventional MIQP, 2 = 1 + MIP start
 };
 

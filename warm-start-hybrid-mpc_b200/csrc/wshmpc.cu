@@ -199,6 +199,15 @@ static LaunchShape launch_shape(const wshmpc_handle *h, int slots)
     return {one ? 1 : WS_MAXL, &P, dim3((slots + P.lanes - 1) / P.lanes), dim3(P.lanes * WS_NT), (size_t)P.so.total_bytes};
 }
 
+// dynamic shared memory a launch of `fn` may use: the device's opt-in budget less the kernel's static shared memory
+static cudaError_t raise_smem_limit(const void *fn, size_t optin)
+{
+    cudaFuncAttributes fa;
+    const cudaError_t e = cudaFuncGetAttributes(&fa, fn);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(optin - fa.sharedSizeBytes));
+}
+
 extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, void *stream, wshmpc_handle **out)
 {
     if (!p || !out) WS_FAIL(-1, "null argument");
@@ -276,7 +285,7 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     L.off_rho = L.off_nu_ub + p->nb;
     L.off_sigma = L.off_rho + p->T * p->nq + p->nqT;
     L.dual = L.off_sigma + p->T * p->nr;
-    L.rec_stride = L.dual + n;
+    L.rec_stride = (L.dual + n + 1) & ~1;          // even: every record of a tree allocation starts 16-byte aligned
     P.n_primal = L.primal; P.n_dual = L.dual; P.n_rec = L.rec_stride; P.off_lam = L.off_lam; P.off_mu = L.off_mu; P.off_nulb = L.off_nu_lb;
     P.off_nuub = L.off_nu_ub; P.off_rho = L.off_rho; P.off_sigma = L.off_sigma;
     // shared memory budget: one CTA per SM holding `lanes` solver lanes; the lanes share the read-only tables, each lane has
@@ -338,11 +347,13 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
         P.lanes = lanes;
         g_lanes_last = lanes;
         h->n_sm = prop.multiProcessorCount;
-        const size_t pool_max = (size_t)n * P.ld + tri_off(n) + 2;          // the whole factor of the largest node
+        // the whole factor of the largest node, and at least the scratch of the fused loop's tree shift (few inputs, many states)
+        size_t pool_max = (size_t)n * P.ld + tri_off(n) + 2;
+        if (pool_max < need_shift) pool_max = need_shift;
         auto lay = [&](DevProblem &D, int L) {
             size_t pool = (avail - so.tab_doubles) / L - fixed;
-            pool &= ~(size_t)1;
             if (pool > pool_max) pool = pool_max;
+            pool &= ~(size_t)1;                         // even (pool_max is odd when n = 1, 2 mod 4): lane 1 starts 16-byte aligned
             D.lanes = L;
             D.so.pool = fixed; D.so.pool_sz = (int)pool;
             D.so.lane_doubles = fixed + (int)pool;
@@ -353,7 +364,9 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
         lay(h->P1, 1);
         h->smem = (size_t)(P.so.total_bytes > h->P1.so.total_bytes ? P.so.total_bytes : h->P1.so.total_bytes);
     }
-    for (const KernelRow &r : g_kernels) WS_CUDA(cudaFuncSetAttribute(r.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem));
+    // the limit is an attribute of the kernel, not of the handle: raise it to what the device allows, so that a handle created
+    // later for a smaller problem cannot lower it below what this handle launches with
+    for (const KernelRow &r : g_kernels) WS_CUDA(raise_smem_limit(r.fn, optin));
     // slot memory
     void *d = nullptr;
     // both cleared: a slot that never stored a state starts from the empty working set AND the centre 0 (hot = 1 on a fresh
@@ -366,8 +379,7 @@ extern "C" int wshmpc_create(const wshmpc_problem *p, int device, int n_slots, v
     WS_CUDA(cudaMalloc(&d, (size_t)n_slots * bnb_scratch_doubles(p->nb, L.primal) * sizeof(double))); h->allocs.push_back(d); h->scratch = (double *)d;
     WS_CUDA(cudaMalloc(&d, 64)); h->allocs.push_back(d); h->work_counter = (int *)d;
     h->shift_smem = shift_smem_bytes(P, optin, &h->shift_stage);
-    if (h->shift_smem > 48 * 1024)
-        WS_CUDA(cudaFuncSetAttribute(shift_tree_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->shift_smem));
+    WS_CUDA(raise_smem_limit((const void *)shift_tree_kernel, optin));
     {
         // best effort: persisting L2 lines for the shared operators (1.2 MB on the T = 20 cart-pole; the trees are GBs)
         h->l2_window = 0;

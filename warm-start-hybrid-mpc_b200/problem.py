@@ -30,6 +30,8 @@ class RecordLayout(object):
         self.off_rho = self.off_nu_ub + T * nub
         self.off_sigma = self.off_rho + T * nq + nqT
         self.dual = self.off_sigma + T * nr
+        # a tree's dual record: the duals, the proximal centre (T nu doubles), and one zero double if that sum is odd
+        self.rec_stride = (self.dual + T * nu + 1) & ~1
 
 
 class ProblemData(object):
