@@ -1,5 +1,5 @@
-"""Problem shapes at the branch conditions of the kernels, shared by tests/test_shape_grid_cpu.py and
-tests/test_gpu_shapes.py.
+"""Problem shapes at the branch conditions of the kernels, shared by tests/test_shape_grid_cpu.py,
+tests/test_gpu_shapes.py and tests/test_gpu_shape_search.py.
 
 The shipped models (CP20, CP40, CP1W40, SYN30) are even in every dimension the kernels branch on.  Each entry below is a
 deterministic generator call (oracle.models.build_synthetic, or CP20 at another horizon, the way CP40 is made) and the
@@ -118,6 +118,17 @@ def conditions(shape):
         c.add('n (n + 1) / 2 odd')                          # the factor's triangle: an odd whole-factor pool of a lane
     if d['T'] in (1, 2):
         c.add('T == %d' % d['T'])
+    if d['T'] == 2 and shape.tier == ALL:
+        c.add('H = T - 1 == 1')                             # the longest plan hold of the fallback is one step
+    if d['nu'] - d['nub'] > 1:
+        c.add('nuc > 1')                                    # binaries start nuc entries into an input, not at 1
+    if d['nu'] & 1:
+        c.add('nu odd')
+    words, tail = (d['nb'] + 31) // 32, d['nb'] % 32
+    if words > 1 and tail:
+        c.add('words > 1 with a partial last word')
+    if words == 1 and tail == 0:
+        c.add('one full identifier word')
     if d['T'] & 1 and d['nh1'] != d['nh'] and shape.tier == ALL:
         c.add('odd T with a terminal set')
     if shape.tier != REFUSED:
@@ -137,7 +148,8 @@ COVERAGE = ['n odd', 'n even', 'ns odd', 'ns even', 'm odd', 'm even', 'dual odd
             'dual + n even', 'shift stages records that dual + n would misalign', 'shift reads every record in place',
             'nb % 32 == 0', 'nub == 1', 'nub == 32 through the shift', 'nub > 32', 'nx == 32', 'nx > 32', 'T == 1', 'T == 2',
             'odd T with a terminal set', 'n (n + 1) / 2 odd', 'gp == 0', 'gp > 0', 'n == 512', 'n > 512 refused', 'n_elim == 0',
-            '0 < n_elim < nb, odd', 'n_elim == nb']
+            '0 < n_elim < nb, odd', 'n_elim == nb', 'nuc > 1', 'nu odd', 'words > 1 with a partial last word',
+            'one full identifier word', 'H = T - 1 == 1']
 
 
 def problem(shape, n_elim=None):

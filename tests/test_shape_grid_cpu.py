@@ -22,7 +22,8 @@ def test_grid_reaches_every_listed_condition():
 
 def test_conditions_name_what_an_edited_grid_loses():
     """The coverage check fails, and names the condition, when the only shape that reaches it leaves the grid."""
-    for name, cond in (('n513', 'n > 512 refused'), ('nx33', 'nx > 32'), ('odd_rec', 'shift stages records that dual + n would misalign')):
+    for name, cond in (('n513', 'n > 512 refused'), ('nx33', 'nx > 32'), ('odd_rec', 'shift stages records that dual + n would misalign'),
+                       ('nub32', 'H = T - 1 == 1')):
         rest = [s for s in sg.GRID if s.name != name]
         reached = set().union(*(sg.conditions(s) for s in rest))
         assert cond not in reached, (name, cond)

@@ -25,6 +25,36 @@ def policy_law(live, has_inc, status, age, law_n, H, L):
     return source, hold, (source >= 0).astype(int), new_age, new_n
 
 
+def fallback_reference(A, B, K, T, H, L, live, status, cost, age, law_n, x, plan, inc):
+    """What wshmpc_fallback_step writes for one step of n instances (include/wshmpc.h, wshmpc_fallback), with the arithmetic in
+    np.longdouble: the policy of policy_law, then per instance the applied cost, the new plan and, on plan and law steps,
+    u_0 (u_a of the plan, or K x) and x_1 = A x + B u_0.  x [n, nx], plan and inc [n, primal] (records x_0..x_T, u_0..u_T-1).
+    Returns a dict: source, hold, active, age, law_n, app_cost, plan, u [n, nu] and x1 [n, nx] (long double; NaN where the
+    step applies neither), u_terms and x1_terms (sums of the magnitudes of the products each entry is summed from)."""
+    source, hold, active, new_age, new_n = policy_law(live, np.isfinite(cost), status, age, law_n, H, L)
+    ld = np.longdouble
+    nx, nu = B.shape
+    U = (T + 1) * nx
+    A_, B_, K_ = (np.asarray(M, dtype=ld) for M in (A, B, K))
+    u = np.full((len(source), nu), np.nan, dtype=ld); u_terms = np.zeros((len(source), nu))
+    x1 = np.full((len(source), nx), np.nan, dtype=ld); x1_terms = np.zeros((len(source), nx))
+    for i in np.nonzero(source > 0)[0]:
+        xi = np.asarray(x[i], dtype=ld)
+        if source[i] == 1:
+            u[i] = plan[i, U + hold[i] * nu:U + (hold[i] + 1) * nu]
+            u_err = np.zeros(nu)
+        else:
+            u[i] = K_.dot(xi)
+            u_terms[i] = u_err = np.abs(K).dot(np.abs(x[i]))
+        x1[i] = A_.dot(xi) + B_.dot(u[i])
+        # the device forms u in double first: its rounding reaches x_1 through B
+        x1_terms[i] = np.abs(A).dot(np.abs(x[i])) + np.abs(B).dot(np.abs(u[i].astype(float)) + u_err)
+    app_cost = np.where(source == 0, cost, np.where(source > 0, 0., np.inf))
+    new_plan = np.where((source == 0)[:, None], inc, plan)
+    return dict(source=source, hold=hold, active=active, age=new_age, law_n=new_n, app_cost=app_cost, plan=new_plan, u=u,
+                x1=x1, u_terms=u_terms, x1_terms=x1_terms)
+
+
 def replay_law(status, cost, H, L, active0=None):
     """hold [n_steps, n_inst] the policy gives to the logs of a loop (status, cost [n_steps, n_inst]) started without plans"""
     S, N = status.shape
@@ -87,6 +117,61 @@ def test_replay_runs_of_law_steps():
     cost = np.where(st == 0, 1., inf)
     assert replay_law(st, cost, 0, 2)[:, 0].tolist() == [-2, -2, 0, -2, -2, -1, -1]
     assert replay_law(st, cost, 1, 2)[:, 0].tolist() == [-2, -2, 0, 1, -2, -2, 0]
+
+
+def test_fallback_reference_reproduces_the_policy_table():
+    """The numpy reference of wshmpc_fallback_step on the hand-built grid of test_gpu_fallback.py's policy-table test (CP20,
+    H = 3, without the law), held to what that test asserts of the kernel, then with a law (L = 2) and on values worked out
+    by hand."""
+    from oracle.models import load_model
+    from tests.test_fallback_cpu import policy
+    model = load_model('cp20')
+    A, B = model['A'], model['B']
+    T, nx, nu, H = int(model['T']), A.shape[0], B.shape[1], 3
+    P, U = (T + 1) * nx + T * nu, (T + 1) * nx
+    grid = [(lv, hi, st, a) for lv in (0, 1) for hi in (0, 1) for st in (0, 1, 2, 3) for a in (-1, 0, 1, 2, 3)
+            if not (hi and st == 1)]
+    N = len(grid)
+    lv, hi, st, age = (np.array(c) for c in zip(*grid))
+    rng = np.random.default_rng(0)
+    x = rng.standard_normal((N, nx))
+    plan = rng.standard_normal((N, P)); inc = rng.standard_normal((N, P))
+    cost = np.where(hi == 1, rng.uniform(1., 2., N), np.inf)
+    K = rng.standard_normal((nu, nx))
+    ref = fallback_reference(A, B, K, T, H, 0, lv, st, cost, age, np.zeros(N, int), x, plan, inc)
+    src, hold, act, new_age = policy(lv, hi, st, age, H)
+    assert np.array_equal(ref['hold'], hold) and np.array_equal(ref['age'], new_age)
+    assert np.array_equal(np.isfinite(ref['app_cost']), act == 1) and np.array_equal(ref['source'], src)
+    for i in range(N):
+        if src[i] == 0:
+            assert ref['app_cost'][i] == cost[i] and np.array_equal(ref['plan'][i], inc[i])
+        else:
+            assert np.array_equal(ref['plan'][i], plan[i])
+        if src[i] == 1:
+            u = plan[i, U + hold[i] * nu:U + (hold[i] + 1) * nu]
+            assert np.array_equal(ref['u'][i].astype(float), u)
+            assert np.allclose(ref['x1'][i].astype(float), A.dot(x[i]) + B.dot(u), rtol=1e-13, atol=1e-14)
+        else:
+            assert np.isnan(ref['u'][i].astype(float)).all() and np.isnan(ref['x1'][i].astype(float)).all()
+    # with the law: the plan first, then K x
+    n = np.array([0, 1, 2] * (N // 3 + 1))[:N]
+    law = fallback_reference(A, B, K, T, H, 2, lv, st, cost, age, n, x, plan, inc)
+    s2, h2, _, a2, n2 = policy_law(lv, hi, st, age, n, H, 2)
+    assert np.array_equal(law['hold'], h2) and np.array_equal(law['age'], a2) and np.array_equal(law['law_n'], n2)
+    assert (s2 == 2).any()
+    for i in np.nonzero(s2 == 2)[0]:
+        assert law['app_cost'][i] == 0.
+        assert np.allclose(law['u'][i].astype(float), K.dot(x[i]), rtol=1e-13, atol=1e-14)
+        assert np.allclose(law['x1'][i].astype(float), A.dot(x[i]) + B.dot(K.dot(x[i])), rtol=1e-13, atol=1e-13)
+    # by hand: nx = 2, nu = 1, T = 2; the record is x_0 x_1 x_2 | u_0 u_1
+    A2, B2, K2 = np.array([[1., 2.], [0., 1.]]), np.array([[0.], [3.]]), np.array([[-1., 0.5]])
+    plan2 = np.array([[0., 0., 0., 0., 0., 0., 10., 20.]] * 3)
+    r = fallback_reference(A2, B2, K2, 2, 1, 1, [1, 1, 1], [1, 1, 0], [np.inf, np.inf, 7.], [0, 1, 0], [0, 0, 0],
+                           np.array([[1., 1.]] * 3), plan2, np.full((3, 8), 4.))
+    assert r['hold'].tolist() == [1, LAW, 0] and r['app_cost'].tolist() == [0., 0., 7.]
+    assert r['u'][0, 0] == 20. and r['x1'][0].astype(float).tolist() == [3., 61.]           # u_1 of the plan
+    assert r['u'][1, 0] == -0.5 and r['x1'][1].astype(float).tolist() == [3., -0.5]         # K x, then A x + B K x
+    assert r['plan'][2].tolist() == [4.] * 8 and r['plan'][0].tolist() == plan2[0].tolist()
 
 
 @pytest.fixture(scope='module', params=['cp20', 'cp40'])
