@@ -317,11 +317,15 @@ int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *lo
  *   status 1 (infeasible), age + 1 <= max_hold  age <- age + 1; applied u_0 = u_age of the plan,
  *                                             x_1|t = A x_t + B u_0; the instance stays live;                      hold age
  *   status 1, otherwise (no plan or plan used up), law_n + 1 <= max_law
- *                                             law_n <- law_n + 1; applied u_0 = K x_t (the terminal law),
+ *                                             law_n <- law_n + 1; applied u_0 = the terminal law's input (below),
  *                                             x_1|t = A x_t + B u_0; age kept; the instance stays live;              hold -2
  *   otherwise (law used up, status 2 or 3, instance off)   the instance is switched off as without a fallback;      hold -1
- * An incumbent also resets law_n to 0.  The terminal law is the linear feedback of the terminal set (e.g. the LQR gain it was
- * built with), without offset or saturation; K is [nu][nx], row-major, shared by all instances.
+ * An incumbent also resets law_n to 0.  The terminal law of instance i is
+ *     u_0 = sat_[lo, hi](K_i x_t + k_i),   sat clamping each component: u_r < lo_r ? lo_r : (u_r > hi_r ? hi_r : u_r)
+ * with K_i, k_i set i of the gain and offset (set 0 when there is one), e.g. the LQR gain the terminal set was built with and
+ * the bounds of the input box (a bound of +-inf leaves its component free; NaN passes through).  x_1|t, the logs, the plant
+ * and K2 + K4 all use the clamped input.  A zero-initialised tail (law_sets = 0, d_law_k = d_law_lo = d_law_hi = NULL) is
+ * the linear law u_0 = K x_t of one shared gain, without offset or saturation.
  * A status-1 step ran its search to the end: its leaves are a complete cover (Farkas proofs and bounds) and K2 + K4 shift them
  * with the applied input like a solved tree, for any input.  The logs of a fallback step keep cost +inf and status 1; u0 is
  * the applied input.  All buffers are device memory owned by the caller, so plans survive launches.
@@ -333,8 +337,13 @@ int wshmpc_closed_loop_plant(wshmpc_handle *h, int n_inst, const wshmpc_loop *lo
  *                Must not overlap d_plan.
  *   d_hold       [n_steps][n_inst] (wshmpc_closed_loop_fallback) or [n_inst] (wshmpc_fallback_step): 0 the incumbent,
  *                a > 0 input u_a of the plan, -2 the terminal law, -1 the instance left the loop (or was off)
- *   d_law_K      [nu][nx] the terminal law's gain (read when max_law > 0)
+ *   d_law_K      [law_sets][nu][nx] the terminal law's gain, row-major (read when max_law > 0)
  *   d_law_n      [n_inst] in/out, law steps since the last incumbent (fill with 0 to start; read when max_law > 0)
+ *   law_sets     0 or 1: one gain (and offset) for all instances; n_inst: set i for instance i
+ *   d_law_k      [law_sets][nu] the law's offset, or NULL (no offset)
+ *   d_law_lo, d_law_hi  [nu] the bounds of the law's input, both or neither (NULL: no saturation); lo <= hi, no NaN (not
+ *                checked here: the bounds are not read back)
+ * law_sets, d_law_k, d_law_lo and d_law_hi must stay 0 / NULL when max_law = 0.
  * max_hold = max_law = 0 is the behaviour without a fallback, bit for bit; max_law = 0 is the policy without the law. */
 typedef struct {
     int max_hold;          /* H, 0 <= H <= T - 1 */
@@ -346,12 +355,17 @@ typedef struct {
     int max_law;           /* L >= 0 */
     const double *d_law_K;
     int *d_law_n;
+    int law_sets;          /* 0, 1 or n_inst */
+    const double *d_law_k;
+    const double *d_law_lo;
+    const double *d_law_hi;
 } wshmpc_fallback;
 
 /* wshmpc_closed_loop (plant = NULL: the linear plant x <- x_1|t + e_t) or wshmpc_closed_loop_plant under the fallback policy:
  * the plant and the warm start of every step use the applied pair.  Fails under node rules 1 and 2 (the comparator), with a
- * mailbox, for max_hold outside 0 .. T - 1, null buffers, d_plan overlapping d_app_primal, max_law < 0, or max_law > 0 with a
- * null d_law_K or d_law_n. */
+ * mailbox, for max_hold outside 0 .. T - 1, null buffers, d_plan overlapping d_app_primal, max_law < 0, max_law > 0 with a
+ * null d_law_K or d_law_n, law_sets outside {0, 1, n_inst}, exactly one of d_law_lo and d_law_hi null, or max_law = 0 with
+ * law_sets, d_law_k, d_law_lo or d_law_hi set. */
 int wshmpc_closed_loop_fallback(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop, const wshmpc_plant *plant,
                                 const wshmpc_fallback *fb, const wshmpc_tree *tree0, const wshmpc_tree *tree1, double tol,
                                 int max_solves, double *d_inc_cost, int *d_inc_node, double *d_inc_primal, int *d_n_solves,

@@ -108,21 +108,49 @@ def _plant_struct(plant, log_x=None):
 class _Fallback(C.Structure):
     _fields_ = [('max_hold', C.c_int), ('d_plan', C.c_void_p), ('d_age', C.c_void_p), ('d_app_cost', C.c_void_p),
                 ('d_app_primal', C.c_void_p), ('d_hold', C.c_void_p), ('max_law', C.c_int), ('d_law_K', C.c_void_p),
-                ('d_law_n', C.c_void_p)]
+                ('d_law_n', C.c_void_p), ('law_sets', C.c_int), ('d_law_k', C.c_void_p), ('d_law_lo', C.c_void_p),
+                ('d_law_hi', C.c_void_p)]
 
 
 def _fallback_struct(fb, hold):
     """wshmpc_fallback of a dict(max_hold, plan, age, app_cost, app_primal) of CUDA tensors, with the hold log `hold`; the
-    terminal law comes from the optional keys max_law, law_K and law_n (without them: max_law = 0 and null pointers)"""
+    terminal law comes from the optional keys max_law, law_K and law_n (without them: max_law = 0 and null pointers), and its
+    sets, offset and bounds from the optional keys law_sets, law_k, law_lo and law_hi (without them: 0 and null pointers,
+    the linear law of one shared gain)"""
     c = _Fallback()
     c.max_hold = int(fb['max_hold'])
     for k in ('plan', 'age', 'app_cost', 'app_primal'):
         setattr(c, 'd_' + k, fb[k].data_ptr() if fb[k] is not None else None)
     c.d_hold = hold.data_ptr() if hold is not None else None
     c.max_law = int(fb.get('max_law', 0))
-    for k in ('law_K', 'law_n'):
+    for k in ('law_K', 'law_n', 'law_k', 'law_lo', 'law_hi'):
         setattr(c, 'd_' + k, fb[k].data_ptr() if fb.get(k) is not None else None)
+    c.law_sets = int(fb.get('law_sets', 0))
     return c
+
+
+def check_terminal_law(n_inst, nu, nx, K, k=None, lo=None, hi=None, names=('terminal law gain', 'terminal law offset',
+                                                                         'terminal law bounds')):
+    """(K, k, lo, hi) of a terminal law u = sat_[lo, hi](K_i x + k_i) as float arrays, checked on the host: K [nu, nx] or
+    [n_inst, nu, nx], k None, [nu] or [n_inst, nu], lo and hi both None or both [nu] with lo <= hi and no NaN.  A
+    ValueError names the argument (`names`: of K, k and the bounds)."""
+    K = np.asarray(K, dtype=float)
+    if K.shape not in ((nu, nx), (n_inst, nu, nx)):
+        raise ValueError('%s of shape %s: [nu, nx] = [%d, %d] or [n_inst, nu, nx] = [%d, %d, %d]'
+                         % (names[0], K.shape, nu, nx, n_inst, nu, nx))
+    if k is not None:
+        k = np.asarray(k, dtype=float)
+        if k.shape not in ((nu,), (n_inst, nu)):
+            raise ValueError('%s of shape %s: [nu] = [%d] or [n_inst, nu] = [%d, %d]' % (names[1], k.shape, nu, n_inst, nu))
+    if (lo is None) != (hi is None):
+        raise ValueError('%s: both lo and hi, or neither' % names[2])
+    if lo is not None:
+        lo, hi = np.asarray(lo, dtype=float), np.asarray(hi, dtype=float)
+        if lo.shape != (nu,) or hi.shape != (nu,):
+            raise ValueError('%s of shapes %s, %s: lo and hi are [nu] = [%d]' % (names[2], lo.shape, hi.shape, nu))
+        if np.isnan(lo).any() or np.isnan(hi).any() or not np.all(lo <= hi):
+            raise ValueError('%s: lo <= hi and no NaN' % names[2])
+    return K, k, lo, hi
 
 
 class _Tree(C.Structure):
@@ -317,10 +345,14 @@ class Handle(object):
                                           C.c_void_p(out.data_ptr())))
         return out
 
-    def new_fallback(self, n_inst, max_hold, max_law=0, K=None):
+    def new_fallback(self, n_inst, max_hold, max_law=0, K=None, k=None, lo=None, hi=None):
         """Caller-owned buffers of the fallback policy (wshmpc_fallback) for n_inst instances, without plans (age -1):
         dict(max_hold, plan, age, app_cost, app_primal, hold [n_inst]) of CUDA tensors.  With max_law > 0 also the terminal
-        law: dict(max_law, law_K = a device copy of the gain K [nu, nx], law_n [n_inst] = 0)."""
+        law u = sat_[lo, hi](K_i x + k_i): dict(max_law, law_K = a device copy of the gain, law_n [n_inst] = 0).
+        K: [nu, nx], or [n_inst, nu, nx] (one gain per instance).  k: the offset, None, [nu] or [n_inst, nu].  lo, hi: the
+        bounds of the input [nu] (+-inf: free), both or neither, lo <= hi and no NaN.  A per-instance gain or offset makes
+        both per instance (law_sets = n_inst, law_K [n_inst, nu, nx], law_k [n_inst, nu]); an offset adds law_k, bounds add
+        law_lo and law_hi.  Without k, lo and hi and with K [nu, nx] the dict has none of these keys."""
         import torch
         f64 = dict(dtype=torch.float64, device=self.torch_device)
         i32 = dict(dtype=torch.int32, device=self.torch_device)
@@ -328,11 +360,20 @@ class Handle(object):
         fb = dict(max_hold=int(max_hold), plan=torch.zeros((n_inst, P), **f64), age=torch.full((n_inst,), -1, **i32),
                   app_cost=torch.zeros(n_inst, **f64), app_primal=torch.zeros((n_inst, P), **f64),
                   hold=torch.zeros(n_inst, **i32), max_law=int(max_law))
-        if max_law:
-            K = np.asarray(K, dtype=float)
-            if K.shape != (nu, nx):
-                raise ValueError('terminal law gain of shape %s: [nu, nx] = [%d, %d]' % (K.shape, nu, nx))
-            fb.update(law_K=torch.as_tensor(np.ascontiguousarray(K), **f64), law_n=torch.zeros(n_inst, **i32))
+        if not max_law:
+            return fb
+        K, k, lo, hi = check_terminal_law(n_inst, nu, nx, K, k, lo, hi)
+        per = K.ndim == 3 or (k is not None and k.ndim == 2)
+        if per:
+            K = np.broadcast_to(K, (n_inst, nu, nx))
+            k = np.broadcast_to(k, (n_inst, nu)) if k is not None else None
+            fb['law_sets'] = int(n_inst)
+        dev = lambda a: torch.as_tensor(np.array(a, dtype=float, order='C'), **f64)
+        fb.update(law_K=dev(K), law_n=torch.zeros(n_inst, **i32))
+        if k is not None:
+            fb['law_k'] = dev(k)
+        if lo is not None:
+            fb.update(law_lo=dev(lo), law_hi=dev(hi))
         return fb
 
     def fallback_step(self, fb, x, active, out):

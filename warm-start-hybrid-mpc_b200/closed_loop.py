@@ -20,7 +20,7 @@ def shard(n_total, rank, world):
 class ClosedLoop(object):
 
     def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
-                 mip_start=True, plant=None, fallback=0, terminal_law=0, law_gain=None):
+                 mip_start=True, plant=None, fallback=0, terminal_law=0, law_gain=None, law_offset=None, law_bounds=None):
         """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
         paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
         incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
@@ -34,7 +34,13 @@ class ClosedLoop(object):
         from (0 the incumbent, a > 0 input u_a of the plan, -2 the terminal law, -1 none).  Not with the comparator.
         terminal_law: L >= 0.  With L > 0 an instance whose MIQP is infeasible and that has no plan step left applies the
         terminal law u = K x for up to L steps in a row (counted since its last incumbent) instead of leaving the loop; also
-        with fallback = 0.  law_gain: K [nu, nx], default controller.terminal_law()."""
+        with fallback = 0.  The law of instance i is u = sat_[lo, hi](K_i x + k_i), each component clamped to its bounds;
+        x_1|t, the logs, the plant and the warm start use the clamped input.
+        law_gain: K [nu, nx] shared by all instances, or [n_inst, nu, nx] one per instance (e.g.
+        [controller.terminal_law(A=..., B=...) for every plant]); default controller.terminal_law().
+        law_offset: k, None (no offset), [nu] or [n_inst, nu].
+        law_bounds: None (no saturation), (lo, hi) of shape [nu] each (+-inf leaves a component free), or 'model' for
+        controller.input_box(), the bounds the stage rows put on single inputs."""
         import torch
         if comparator and warm:
             raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
@@ -46,11 +52,22 @@ class ClosedLoop(object):
             raise ValueError('terminal_law = %r: the steps an instance may run on the terminal law, >= 0' % (terminal_law,))
         if (fallback or terminal_law) and comparator:
             raise ValueError('the fallback policy runs under the structured search only, not with the MIQP comparator')
+        lo = hi = None
         if terminal_law:
-            law_gain = controller.terminal_law() if law_gain is None else np.asarray(law_gain, dtype=float)
-            if law_gain.shape != (controller.mld.nu, controller.mld.nx):
-                raise ValueError('law_gain of shape %s: the terminal law gain is [nu, nx] = [%d, %d]'
-                                 % (law_gain.shape, controller.mld.nu, controller.mld.nx))
+            from .capi import check_terminal_law
+            if isinstance(law_bounds, str):
+                if law_bounds != 'model':
+                    raise ValueError("law_bounds = %r: None, (lo, hi) or 'model'" % (law_bounds,))
+                lo, hi = controller.input_box()
+            elif law_bounds is not None:
+                if not isinstance(law_bounds, (tuple, list)) or len(law_bounds) != 2:
+                    raise ValueError("law_bounds: None, (lo, hi) or 'model'")
+                lo, hi = law_bounds
+            law_gain, law_offset, lo, hi = check_terminal_law(
+                n_inst, controller.mld.nu, controller.mld.nx, controller.terminal_law() if law_gain is None else law_gain,
+                law_offset, lo, hi, names=('law_gain', 'law_offset', 'law_bounds'))
+        elif law_offset is not None or law_bounds is not None:
+            raise ValueError('law_offset and law_bounds shape the terminal law: they need terminal_law > 0')
         self.plant = plant
         if max_roots is None:
             max_roots = 2 if comparator else 512
@@ -80,7 +97,8 @@ class ClosedLoop(object):
         self.launches = 0
         self.events = None          # list -> (start, after K3, after K2+K4) CUDA events of every step
         # plans, ages, applied pairs and the terminal law (wshmpc_fallback)
-        self.fb = h.new_fallback(n_inst, fallback, int(terminal_law), law_gain) if (fallback or terminal_law) else None
+        self.fb = (h.new_fallback(n_inst, fallback, int(terminal_law), law_gain, law_offset, lo, hi)
+                   if (fallback or terminal_law) else None)
         if self.fb is not None:
             self.out['hold'] = self.fb['hold']
 

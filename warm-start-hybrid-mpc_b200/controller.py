@@ -159,25 +159,49 @@ class HybridModelPredictiveController(object):
             cols.append(res.x)
         return np.vstack(cols).T if cols else np.zeros((n, 0))
 
-    def terminal_law(self, inputs=None):
+    def terminal_law(self, inputs=None, A=None, B=None):
         """The linear feedback u = K x of the terminal set, K [nu, nx]: the DARE (LQR) gain of the stage cost on the inputs
         `inputs`, zero for every other input.  inputs: column indices of B (default: the columns of R that are not all
         zero, i.e. the inputs the stage cost penalises).  K solves the DARE on (A, B[:, inputs], Q'Q, R_u'R_u) with
         R_u = R[:, inputs]; when the terminal cost and set were built from that LQR law (a terminal cost Q_T'Q_T = P and
-        the maximal admissible set of A + B K), u = K x keeps a state of the terminal set in it."""
+        the maximal admissible set of A + B K), u = K x keeps a state of the terminal set in it.
+        A [nx, nx], B [nx, nu]: the model the gain is designed on (default: the controller's own, mld.A and mld.B), e.g.
+        the model of one plant of a mismatch sweep (plants.CartPoleWithWalls.discrete_model)."""
         from scipy.linalg import solve_discrete_are
         mld = self.mld
+        A = mld.A if A is None else np.asarray(A, dtype=float)
+        B = mld.B if B is None else np.asarray(B, dtype=float)
+        if A.shape != (mld.nx, mld.nx) or B.shape != (mld.nx, mld.nu):
+            raise ValueError('terminal_law: A of shape %s, B of shape %s: [nx, nx] = [%d, %d] and [nx, nu] = [%d, %d]'
+                             % (A.shape, B.shape, mld.nx, mld.nx, mld.nx, mld.nu))
         if inputs is None:
             inputs = np.nonzero(np.any(self.R != 0., axis=0))[0]
         inputs = np.asarray(inputs, dtype=int).ravel()
         if inputs.size == 0:
             raise ValueError('terminal_law: no inputs (R has no nonzero column)')
-        Bu, Ru = mld.B[:, inputs], self.R[:, inputs]
+        Bu, Ru = B[:, inputs], self.R[:, inputs]
         Qc, Rc = self.Q.T.dot(self.Q), Ru.T.dot(Ru)
-        P = solve_discrete_are(mld.A, Bu, Qc, Rc)
+        P = solve_discrete_are(A, Bu, Qc, Rc)
         K = np.zeros((mld.nu, mld.nx))
-        K[inputs] = -np.linalg.inv(Bu.T.dot(P).dot(Bu) + Rc).dot(Bu.T).dot(P).dot(mld.A)
+        K[inputs] = -np.linalg.inv(Bu.T.dot(P).dot(Bu) + Rc).dot(Bu.T).dot(P).dot(A)
         return K
+
+    def input_box(self):
+        """(lo, hi) [nu]: the bounds the stage rows F x + G u <= h put on single inputs.  A row with F zero and one nonzero
+        entry g = G[i, r] bounds u_r by h_i / g (from above when g > 0, from below when g < 0); the tightest such bound of
+        each input is kept, and an input without one gets -inf / +inf.  The bounds a saturated terminal law
+        (ClosedLoop(..., law_bounds='model')) clamps its input to."""
+        mld = self.mld
+        lo, hi = np.full(mld.nu, -np.inf), np.full(mld.nu, np.inf)
+        rows = np.nonzero(np.all(mld.F == 0., axis=1) & (np.count_nonzero(mld.G, axis=1) == 1))[0]
+        for i in rows:
+            r = int(np.flatnonzero(mld.G[i])[0])
+            b = mld.h[i] / mld.G[i, r]
+            if mld.G[i, r] > 0.:
+                hi[r] = min(hi[r], b)
+            else:
+                lo[r] = max(lo[r], b)
+        return lo, hi
 
     # -- device handle --------------------------------------------------------------------------
     @staticmethod

@@ -685,16 +685,30 @@ struct FallbackView {
     double *app_cost;        // [n_inst] applied pair: +inf = the instance leaves the loop, finite otherwise
     double *app_primal;      // [n_inst][n_primal] (a fallback step defines x_0, x_1 and u_0 only)
     int *hold;               // [n_inst] of the step: 0 the incumbent, a > 0 input u_a of the plan, -2 the law, -1 none
-    int max_law;             // L: consecutive steps an instance may run on the terminal law u = K x, 0 = no law
-    const double *law_K;     // [nu][nx] the law's gain, shared by all instances (null when L = 0)
+    int max_law;             // L: consecutive steps an instance may run on the terminal law, 0 = no law
+    const double *law_K;     // [law_sets][nu][nx] the law's gain (null when L = 0)
     int *law_n;              // [n_inst] law steps since the last incumbent (null when L = 0)
+    int law_sets;            // 0 or 1: one gain (and offset) for all instances; n_inst: set i for instance i
+    const double *law_k;     // [law_sets][nu] the law's offset, or null (no offset)
+    const double *law_lo;    // [nu] lower and upper bounds of the law's input, or both null (no saturation)
+    const double *law_hi;
 };
 
-// u_r = (K x)_r, fused multiply-adds over the columns in order (every caller and every thread gets the same bits)
-__device__ __forceinline__ double law_input(const double *__restrict__ K, const double *__restrict__ x, int r, int nx)
+// u_r = sat_[lo_r, hi_r]((K_i x)_r + k_ir), K_i and k_i set i = inst of the law (set 0 when there is one): fused
+// multiply-adds over the columns in order, then the offset, then the clamp (every caller and every thread gets the same
+// bits).  The offset is added only when there is one (adding +0. would turn a -0. into +0.); the clamp leaves NaN and a
+// component with infinite bounds as they are.
+__device__ __forceinline__ double law_input(const FallbackView &fb, int inst, const double *__restrict__ x, int r, int nx, int nu)
 {
+    const size_t set = fb.law_sets > 1 ? (size_t)inst : 0;
+    const double *__restrict__ K = fb.law_K + set * nu * nx;
     double s = 0.;
     for (int c = 0; c < nx; ++c) s = __fma_rn(K[r * nx + c], x[c], s);
+    if (fb.law_k) s = __dadd_rn(s, fb.law_k[set * nu + r]);
+    if (fb.law_lo) {
+        const double lo = fb.law_lo[r], hi = fb.law_hi[r];
+        s = s < lo ? lo : (s > hi ? hi : s);
+    }
     return s;
 }
 
@@ -702,10 +716,11 @@ __device__ __forceinline__ double law_input(const double *__restrict__ K, const 
 //   incumbent                            plan <- incumbent, age 0, law_n 0, applied pair = incumbent, hold 0;
 //   status 1, a plan with age + 1 <= H   age += 1, applied u_0 = u_age of the plan, x_1 = A x + B u_0 (fused multiply-adds
 //                                        in a fixed order, so that every caller gets the same bits), hold = age;
-//   status 1, otherwise, law_n + 1 <= L  law_n += 1, applied u_0 = K x, x_1 = A x + B u_0 (the same order), age kept, hold -2;
+//   status 1, otherwise, law_n + 1 <= L  law_n += 1, applied u_0 = the law's input (law_input), x_1 = A x + B u_0 (the same
+//                                        order), age kept, hold -2;
 //   otherwise                            applied cost +inf (K2 + K4 switch the instance off), hold -1.
 // Threads tid = 0 .. nt - 1 share the copies; `sync` is the callers' barrier (age and law_n are read by all before thread 0
-// writes them).  With L = 0, law_n and law_K are never touched.
+// writes them).  With L = 0, law_n and the law's gain, offset and bounds are never touched.
 template <class Sync>
 __device__ __forceinline__ void fallback_apply(const DevProblem &P, const FallbackView &fb, int inst, bool live, int st,
                                                const double *__restrict__ x, const double *__restrict__ inc_cost,
@@ -735,10 +750,10 @@ __device__ __forceinline__ void fallback_apply(const DevProblem &P, const Fallba
         for (int j = tid; j < nx; j += nt) {
             double s = 0.;
             for (int c = 0; c < nx; ++c) s = __fma_rn(P.A[j * nx + c], x[c], s);
-            for (int c = 0; c < nu; ++c) s = __fma_rn(P.B[j * nu + c], law_input(fb.law_K, x, c, nx), s);
+            for (int c = 0; c < nu; ++c) s = __fma_rn(P.B[j * nu + c], law_input(fb, inst, x, c, nx, nu), s);
             ap[j] = x[j]; ap[nx + j] = s;
         }
-        for (int j = tid; j < nu; j += nt) ap[(size_t)(P.T + 1) * nx + j] = law_input(fb.law_K, x, j, nx);
+        for (int j = tid; j < nu; j += nt) ap[(size_t)(P.T + 1) * nx + j] = law_input(fb, inst, x, j, nx, nu);
     }
     sync();
     if (tid == 0) {

@@ -592,9 +592,15 @@ static int fallback_view(const wshmpc_handle *h, const wshmpc_fallback *fb, int 
     if (p < a + bytes && a < p + bytes) WS_FAIL(-1, "fallback d_plan and d_app_primal overlap");
     if (fb->max_law < 0) WS_FAIL(-1, "fallback max_law = %d: the law steps an instance may take, >= 0", fb->max_law);
     if (fb->max_law > 0 && (!fb->d_law_K || !fb->d_law_n)) WS_FAIL(-1, "fallback max_law = %d with a null d_law_K or d_law_n", fb->max_law);
+    if (fb->max_law == 0 && (fb->law_sets != 0 || fb->d_law_k || fb->d_law_lo || fb->d_law_hi))
+        WS_FAIL(-1, "fallback law_sets, d_law_k, d_law_lo or d_law_hi set with max_law = 0");
+    if (fb->law_sets != 0 && fb->law_sets != 1 && fb->law_sets != n)
+        WS_FAIL(-1, "fallback law_sets = %d: 0 or 1 (one set) or one per instance (%d)", fb->law_sets, n);
+    if (!fb->d_law_lo != !fb->d_law_hi) WS_FAIL(-1, "fallback d_law_lo and d_law_hi: both or neither");
     v->max_hold = fb->max_hold; v->plan = fb->d_plan; v->age = fb->d_age; v->app_cost = fb->d_app_cost;
     v->app_primal = fb->d_app_primal; v->hold = fb->d_hold;
     v->max_law = fb->max_law; v->law_K = fb->max_law > 0 ? fb->d_law_K : nullptr; v->law_n = fb->max_law > 0 ? fb->d_law_n : nullptr;
+    v->law_sets = fb->law_sets; v->law_k = fb->d_law_k; v->law_lo = fb->d_law_lo; v->law_hi = fb->d_law_hi;
     return 0;
 }
 

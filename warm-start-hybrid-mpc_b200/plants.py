@@ -78,6 +78,20 @@ class CartPoleWithWalls(object):
         B[2:, 0] = Minv.dot([1., 0.]); B[2:, 1] = Minv.dot([1., -l]); B[2:, 2] = Minv.dot([-1., l])
         return A, B
 
+    def discrete_model(self, dt, nu=3):
+        """(A, B) of this plant in the coordinates of the MLD model: the linearisation at the upright equilibrium
+        discretised as the shipped cart-pole models were, by explicit Euler with step dt (A = I + dt A_c, B = dt B_c).
+        B has nu >= 3 columns: (fc, fl, fr), then zero columns for the model's binary inputs.  With the nominal parameters
+        and dt = 0.05 it is the model's (A, B) of CP20 / CP40; controller.terminal_law(A=A, B=B) designs this plant's law."""
+        if int(nu) != nu or nu < 3:
+            raise ValueError('discrete_model: nu = %r, the model has the inputs (fc, fl, fr) first, nu >= 3' % (nu,))
+        if not dt > 0.:
+            raise ValueError('discrete_model: dt must be positive, got %r' % (dt,))
+        Ac, Bc = self.linearization()
+        B = np.zeros((4, int(nu)))
+        B[:, :3] = dt * Bc
+        return np.eye(4) + dt * Ac, B
+
 
 class DevicePlant(object):
     """The cart-pole between soft walls integrated on the device (wshmpc_plant in include/wshmpc.h): what
