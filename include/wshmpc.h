@@ -273,6 +273,15 @@ typedef struct {
     int *d_log_status;                /* [n_steps][n_inst] status of wshmpc_bnb_solve */
     const wshmpc_mailbox *mailbox;    /* NULL: the plant x <- x_1|t + e_t is advanced on the device (d_e); else the host is
                                        * in the loop every step (d_e unused) and the call returns while the kernel runs */
+    /* per-step statistics of the warm start and the search, each NULL = not written (the loop computes nothing for it) */
+    int *d_log_cover;                 /* [n_steps][n_inst] warm-start roots handed to step t + 1: the leaves the tree shift of
+                                       * step t retained (the reference's len(warm_start)); 0 once the instance is off or
+                                       * when the shift overflowed the new tree.  In mailbox mode the shift of step t runs
+                                       * after the host's answer to it, and its numbers still go to row t */
+    int *d_log_lapsed;                /* [n_steps][n_inst] of those roots, the ones whose Farkas proof did not survive the
+                                       * shift (the reference's dual = None, controller.py:555-558; wshmpc_tree rec <= -2) */
+    int *d_log_iters;                 /* [n_steps][n_inst] active-set iterations summed over the node QPs of step t's branch
+                                       * and bound (what the step adds to d_totals[1]; 0 for an instance that is off) */
 } wshmpc_loop;
 
 int wshmpc_closed_loop(wshmpc_handle *h, int n_inst, const wshmpc_loop *loop,

@@ -88,7 +88,8 @@ class Mailbox(object):
 class _Loop(C.Structure):
     _fields_ = ([(k, C.c_int) for k in ('n_steps', 'warm', 'fresh', 'par')]
                 + [(k, C.c_void_p) for k in ('d_queue', 'd_step_of', 'd_x', 'd_e', 'd_active', 'd_log_cost', 'd_log_u0',
-                                             'd_log_solves', 'd_log_status', 'mailbox')])
+                                             'd_log_solves', 'd_log_status', 'mailbox', 'd_log_cover', 'd_log_lapsed',
+                                             'd_log_iters')])
 
 
 class _Plant(C.Structure):
@@ -386,9 +387,12 @@ class Handle(object):
                                              V(out['primal'])))
 
     def closed_loop(self, n_steps, warm, fresh, par, xbuf, e, active, trees, out, tol=0., max_solves=1024, totals=None, logs=None,
-                    mailbox=None, plant=None, fallback=None):
+                    mailbox=None, plant=None, fallback=None, stats=False):
         """Fused closed loop (wshmpc_closed_loop): `n_steps` receding-horizon steps of every instance in one
         launch.  xbuf [2, n_inst, nx]; e [n_steps, n_inst, nx] or None; trees = (tree0, tree1).  Asynchronous.
+        stats: the logs gain 'cover', 'lapsed' and 'iters' [n_steps, n_inst] (int32): the warm-start roots each step hands
+        to the next, how many of them lost their Farkas proof in the shift, and the active-set iterations of each step's
+        branch and bound (wshmpc_loop d_log_cover, d_log_lapsed, d_log_iters).
         mailbox: a Mailbox -- the host is in the loop every step (the caller must answer it while the kernel runs).
         plant: a plants.DevicePlant -- the nonlinear plant advances the state on the device (wshmpc_closed_loop_plant), e is
         an additive disturbance on its output, and the logs gain 'x' [n_steps, n_inst, nx], the state after every step.
@@ -418,6 +422,12 @@ class Handle(object):
         L.d_queue, L.d_step_of, L.d_x, L.d_e, L.d_active = P(self._queue), P(self._step_of), P(xbuf), P(e), P(active)
         L.d_log_cost, L.d_log_u0, L.d_log_solves, L.d_log_status = P(logs['cost']), P(logs['u0']), P(logs['n_solves']), P(logs['status'])
         L.mailbox = C.addressof(mailbox.c) if mailbox is not None else None
+        if stats:
+            for k in ('cover', 'lapsed', 'iters'):
+                if k not in logs:
+                    logs[k] = torch.empty((n_steps, N), dtype=torch.int32, device=dev)
+                assert logs[k].is_contiguous() and logs[k].dtype == torch.int32 and tuple(logs[k].shape) == (n_steps, N)
+            L.d_log_cover, L.d_log_lapsed, L.d_log_iters = P(logs['cover']), P(logs['lapsed']), P(logs['iters'])
         V = lambda a: C.c_void_p(a.data_ptr()) if a is not None else None
         tail = (C.byref(trees[0].c), C.byref(trees[1].c), C.c_double(tol), int(max_solves), V(out['cost']), V(out['node']),
                 V(out['primal']), V(out['n_solves']), V(out['status']), V(totals))

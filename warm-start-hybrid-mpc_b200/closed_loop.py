@@ -20,7 +20,8 @@ def shard(n_total, rank, world):
 class ClosedLoop(object):
 
     def __init__(self, controller, n_inst, warm=True, tol=0., max_solves=1024, max_roots=None, n_slots=None, comparator=False,
-                 mip_start=True, plant=None, fallback=0, terminal_law=0, law_gain=None, law_offset=None, law_bounds=None):
+                 mip_start=True, plant=None, fallback=0, terminal_law=0, law_gain=None, law_offset=None, law_bounds=None,
+                 stats=False):
         """comparator=True runs the conventional MIQP branch and bound of `feedforward_miqp` (controller.py:530-582, the
         paper's third curve) instead of the structured search, cold-started every step; with mip_start the previous step's
         incumbent binaries, shifted by one step, are the MIP start (shift_binary_solution).  max_roots: initial leaves a
@@ -40,8 +41,16 @@ class ClosedLoop(object):
         [controller.terminal_law(A=..., B=...) for every plant]); default controller.terminal_law().
         law_offset: k, None (no offset), [nu] or [n_inst, nu].
         law_bounds: None (no saturation), (lo, hi) of shape [nu] each (+-inf leaves a component free), or 'model' for
-        controller.input_box(), the bounds the stage rows put on single inputs."""
+        controller.input_box(), the bounds the stage rows put on single inputs.
+        stats: True adds per step and instance how good the warm start was and what the search cost: the logs of run() and
+        run_mailbox() gain 'cover', 'lapsed' and 'iters' [n_steps, n_inst], and step() / step_with_plant() fill out['cover'],
+        out['lapsed'] and out['iters'] [n_inst] (int32).  cover: the warm-start roots the step hands to the next one (the
+        reference's len(warm_start); 0 once an instance is off); lapsed: of those, the roots whose Farkas proof did not
+        survive the shift (dual = None); iters: active-set iterations summed over the step's node QPs.  False (default)
+        leaves the logs and the loop's work exactly as they are without it."""
         import torch
+        if not isinstance(stats, (bool, np.bool_)):
+            raise ValueError('stats = %r: True or False' % (stats,))
         if comparator and warm:
             raise ValueError('the MIQP comparator runs cold trees only: use ClosedLoop(..., warm=False, comparator=True)')
         if plant is not None and plant.n_sets not in (1, n_inst):
@@ -71,7 +80,7 @@ class ClosedLoop(object):
         self.plant = plant
         if max_roots is None:
             max_roots = 2 if comparator else 512
-        self.comparator, self.mip_start = comparator, mip_start
+        self.comparator, self.mip_start, self.stats = comparator, mip_start, bool(stats)
         self.node_rule = (2 if mip_start else 1) if comparator else 0
         self.ctl, self.n_inst, self.warm, self.tol = controller, n_inst, warm, tol
         self.max_solves, self.max_roots = max_solves, max_roots
@@ -156,11 +165,26 @@ class ClosedLoop(object):
             h.set_node_rule(self.node_rule)
         try:
             h.bnb_solve(self.x, tree, tol=self.tol, max_solves=self.max_solves, active=self.active, out=self.out,
-                        totals=self.totals)
+                        totals=self.totals, trace=self.stats)
         finally:
             if self.node_rule:
                 h.set_node_rule(0)
         self.launches += 1
+        if self.stats:
+            # iterations of the step: the sum over its solves' trace entries (node, iterations)
+            import torch
+            it = self.out.pop('trace')[:, 1::2]
+            done = torch.arange(it.shape[1], device=it.device)[None, :] < self.out['n_solves'][:, None]
+            self.out['iters'] = torch.where(done, it, 0).sum(1).to(torch.int32)
+
+    def _shift_stats(self, new):
+        """out['cover'] and out['lapsed'] of the tree the step's shift built (what the fused loop logs)"""
+        if self.stats:
+            import torch
+            nn = new.n_nodes
+            root = torch.arange(new.cap_nodes, device=nn.device)[None, :] < nn[:, None]
+            self.out['cover'] = nn.clone()
+            self.out['lapsed'] = ((new.rec <= -2) & root).sum(1).to(torch.int32)
 
     def _closed_loop(self, n_steps, par, e, logs, mailbox=None):
         h = self.h
@@ -170,7 +194,7 @@ class ClosedLoop(object):
         try:
             return h.closed_loop(n_steps, self.warm, fresh, par, self.xbuf, e, self.active, self.trees, self.out,
                                  tol=self.tol, max_solves=self.max_solves, totals=self.totals, logs=logs, mailbox=mailbox,
-                                 plant=self.plant, fallback=self.fb)
+                                 plant=self.plant, fallback=self.fb, stats=self.stats)
         finally:
             if self.node_rule:
                 h.set_node_rule(0)
@@ -210,6 +234,7 @@ class ClosedLoop(object):
             x_meas, e = self._device_plant(e, cost, prim)
         h.shift_tree(self.x, e, tree, cost, prim, new, active=self.active,
                      x_next=self.xbuf[1 - self.xpar], u0=self.u0)
+        self._shift_stats(new)
         if x_meas is not None:
             self.xbuf[1 - self.xpar].copy_(x_meas)
         self.cur = 1 - self.cur
@@ -260,6 +285,7 @@ class ClosedLoop(object):
         new = self.trees[1 - self.cur]
         h.shift_tree(self.x, ed, tree, cost_d, prim_d, new, active=self.active,
                      x_next=self.xbuf[1 - self.xpar], u0=self.u0)
+        self._shift_stats(new)
         if live.any():
             # the next step starts from the MEASURED state itself (x_1|t + (x_measured - x_1|t) is one rounding away from it)
             lv = torch.as_tensor(live, device=self.x.device)
@@ -274,7 +300,8 @@ class ClosedLoop(object):
         form of calling step() n_steps times, without a barrier between the steps of different instances.
         e: [n_steps, n_inst, nx] CUDA tensor of model errors or None (with a device plant: of disturbances on the plant's
         output).  Returns per-step logs (cost, u0, n_solves, status), each [n_steps, n_inst, ...], with a device plant
-        also x, the state after every step, and with a fallback also hold; self.x holds the final states."""
+        also x, the state after every step, with a fallback also hold, and with stats also cover, lapsed and iters;
+        self.x holds the final states."""
         par = self.cur
         # states and trees flip together: make the state parity equal to the tree parity
         if self.xpar != par:

@@ -50,11 +50,12 @@ __global__ void init_root_kernel(int n_inst, TreeView tr)
 // branch and bound of ONE instance by the calling CTA (all threads).  Returns the status.
 // RULE: 0 the structured search, 1 the conventional MIQP rule (BNB_RULE_MIQP; the branching binary is chosen AFTER the
 // node's solve, from its relaxation) -- a template parameter, so that the default kernels carry none of the rule-1 code.
+// n_iters (null: not wanted): every thread gets the active-set iterations of the search, the sum it adds to totals[1].
 template <int RULE>
 __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, const SlotPtrs &sp, double *y, double *sc, int *iters_s,
                                    int inst, const double *xi, const TreeView &tr, double tol, int max_solves,
                                    double *inc_cost, int *inc_node, double *inc_primal, int *n_solves, int *trace,
-                                   unsigned long long *totals)
+                                   unsigned long long *totals, int *n_iters = nullptr)
 {
     const int nb = P.nb;
     double *lbv = sc, *ubv = sc + nb, *prim = sc + 2 * nb, *cost_s = prim + P.n_primal, *dobj_s = cost_s + 1;
@@ -219,6 +220,7 @@ __device__ __forceinline__ int bnb_instance(const DevProblem &P, const Ctx &cx, 
             atomicAdd(totals + 4, (unsigned long long)dsum); atomicAdd(totals + 5, (unsigned long long)k0sum);
         }
     }
+    if (n_iters) *n_iters = (int)iters;
     WS_SYNC();
     return st;
 }
@@ -609,6 +611,9 @@ struct LoopView {
     double *log_u0;         // [n_steps][n_inst][nu]
     int *log_solves;        // [n_steps][n_inst]
     int *log_status;        // [n_steps][n_inst]
+    int *log_cover;         // [n_steps][n_inst] or null: roots of the tree the shift of the step built
+    int *log_lapsed;        // [n_steps][n_inst] or null: of those, roots whose Farkas proof lapsed in the shift (rec <= -2)
+    int *log_iters;         // [n_steps][n_inst] or null: active-set iterations of the step's branch and bound
     // host mailbox (wshmpc_mailbox; all null = the plant is advanced on the device).  mb_* point into pinned, mapped HOST
     // memory and are read / written with system-scope ordering; mb_stage is device scratch [n_inst][nx].
     volatile int *mb_in_step, *mb_out_step, *mb_stop;
@@ -775,6 +780,25 @@ __global__ void fallback_step_kernel(DevProblem P, int n_inst, FallbackView fb, 
 }
 #endif
 
+// The cover and lapsed logs of row `lo` (wshmpc_loop d_log_cover, d_log_lapsed), right after a shift_instance of the lane
+// built `nt`: its roots, and how many of them carry a Farkas proof the shift let lapse.  Writes nothing when neither log
+// is wanted.
+__device__ __forceinline__ void log_shifted_tree(const DevProblem &P, const Ctx &cx, const LoopView &L, const TreeView &nt,
+                                                 int inst, size_t lo)
+{
+    if (!L.log_cover && !L.log_lapsed) return;
+    WS_SYNC();                                         // n_nodes (thread 0) and rec (every warp) of the new tree
+    const int nn = nt.n_nodes[inst];
+    if (WS_TID == 0 && L.log_cover) L.log_cover[lo] = nn;
+    if (L.log_lapsed) {
+        const int *rec = nt.rec + (size_t)inst * nt.cap_nodes;
+        double c = 0.;
+        for (int j = WS_TID; j < nn; j += WS_NT) c += rec[j] <= -2 ? 1. : 0.;
+        c = block_sum(c, SMV(red));
+        if (WS_TID == 0) L.log_lapsed[lo] = (int)c;
+    }
+}
+
 // PLANT: the state advances through the nonlinear plant on the device (wshmpc_closed_loop_plant, `pv`) instead of the linear
 // model plus an additive error; the kernels without it carry no code of the plant and never read `pv`.
 // FB: the fallback policy (wshmpc_closed_loop_fallback, `fv`): after K3 the plant and K2 + K4 read the applied pair
@@ -885,6 +909,7 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
             const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, L.mb_stage, cur, inc_cost, inc_primal,
                                                   L.active, nxt, nullptr, L.log_u0 + (size_t)ts * n_inst * P.nu);
             if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)ts * n_inst + inst] = BNB_CAPACITY; }
+            log_shifted_tree(P, cx, L, nxt, inst, (size_t)ts * n_inst + inst);
             prof_mark(19);
             WS_SYNC();
         }
@@ -907,19 +932,20 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                 }
                 WS_SYNC();
             }
-            int st;
+            int st, it = 0;
             if (!L.active[inst]) {
                 if (WS_TID == 0) { inc_cost[inst] = INFINITY; inc_node[inst] = -1; n_solves[inst] = 0; }
                 st = BNB_INFEASIBLE;
                 WS_SYNC();
             } else {
                 st = bnb_instance<RULE>(P, cx, sp, y, sc, iters_s, inst, xc + (size_t)inst * P.nx, cur, tol, max_solves,
-                                  inc_cost, inc_node, inc_primal, n_solves, nullptr, totals);
+                                  inc_cost, inc_node, inc_primal, n_solves, nullptr, totals, &it);
             }
             if (WS_TID == 0) {
                 status_out[inst] = st;
                 const size_t lo = (size_t)t * n_inst + inst;
                 L.log_cost[lo] = inc_cost[inst]; L.log_solves[lo] = n_solves[inst]; L.log_status[lo] = st;
+                if (L.log_iters) L.log_iters[lo] = it;
             }
             WS_SYNC();
             // the pair the plant and K2 + K4 apply: the incumbent, or under FB the policy's choice
@@ -954,11 +980,13 @@ closed_loop_body(const DevProblem &P, double *slot_d, int *slot_i, double *ybuf,
                 const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, pv.stage,
                                                       cur, a_cost, a_primal, L.active, nxt, nullptr, L.log_u0 + (size_t)t * n_inst * P.nu);
                 if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
+                log_shifted_tree(P, cx, L, nxt, inst, (size_t)t * n_inst + inst);
                 prof_mark(19);
             } else if (!mbx) {
                 const int ovf = shift_instance<WS_NT, true>(P, SMV(pool), P.so.pool_sz - (int)shift_smem_doubles(P, WS_NT), SMI(ired), SMI(ired) + 16, inst, xc, L.e ? L.e + (size_t)t * xs : nullptr,
                                                       cur, a_cost, a_primal, L.active, nxt, xn, L.log_u0 + (size_t)t * n_inst * P.nu);
                 if (ovf && WS_TID == 0) { status_out[inst] = BNB_CAPACITY; L.log_status[(size_t)t * n_inst + inst] = BNB_CAPACITY; }
+                log_shifted_tree(P, cx, L, nxt, inst, (size_t)t * n_inst + inst);
                 prof_mark(19);
             } else {
                 // publish step t: applied input, predicted next state, cost, status -- then the step counter

@@ -661,6 +661,7 @@ static int closed_loop_launch(wshmpc_handle *h, int n_inst, const wshmpc_loop *l
     L.n_steps = loop->n_steps; L.warm = loop->warm; L.fresh = loop->fresh; L.par = loop->par & 1;
     L.q = loop->d_queue; L.step_of = loop->d_step_of; L.x = loop->d_x; L.e = loop->d_e; L.active = loop->d_active;
     L.log_cost = loop->d_log_cost; L.log_u0 = loop->d_log_u0; L.log_solves = loop->d_log_solves; L.log_status = loop->d_log_status;
+    L.log_cover = loop->d_log_cover; L.log_lapsed = loop->d_log_lapsed; L.log_iters = loop->d_log_iters;
     WS_CUDA(cudaSetDevice(h->device));
     L.mb_in_step = L.mb_out_step = L.mb_stop = nullptr; L.mb_in_x = L.mb_in_e = nullptr;
     L.mb_out_u0 = L.mb_out_x1 = L.mb_out_cost = nullptr; L.mb_out_status = nullptr; L.mb_stage = nullptr; L.mb_timeout_ns = 0;
